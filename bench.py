@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — BEAST tokenizer hot path on B200: trajectories/s, encode + decode.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload = BASELINE.json configs[1]: bimanual tokenizer (num_dof=14, num_basis=10, seq_len=50,
 vocab 256, grippers [6, 13] zero-order, llm_vocab_size=32000), batch 65 536 per GPU, synthetic
@@ -17,6 +17,8 @@ trajectories.  One step = encode (K1) of one batch + reconstruct_traj (K3) of on
   cpu_baseline  the oracle's literal port of the reference algorithm on the host cores (rank 0, N=1).
 
 `--impl reference` times that CPU port alone (rank 0 only under torchrun).
+`--dump-outputs DIR` writes what the last timed step computed to DIR/<name>.npy (rank 0), so that two builds can be
+compared output for output: the inputs depend only on the arguments.
 """
 import argparse
 import json
@@ -710,6 +712,24 @@ def synth_bins_sample(tok, dev):
     return tok.encode(synth_device(BPE_CPU_SAMPLE, T, D, 1000, dev), respect_llm_vocab_size=False)[0]
 
 
+DUMP_ROWS = 8192          # 8 192 x 4 480 B = 37 MB of .npy files whatever the batch
+
+
+def dump_outputs(out_dir, tokens, params, trajectories):
+    """What one timed step hands back — encode's tokens and coefficients, decode's trajectories — as
+    out_dir/<name>.npy: the same seeded sample of rows (all rows of a batch up to DUMP_ROWS), tokens as
+    float64 (exact), the rest float32."""
+    import numpy as np
+    import torch
+    n = tokens.shape[0]
+    rows = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_ROWS), replace=False))
+    idx = torch.from_numpy(rows).to(tokens.device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t, dtype in (("encode_tokens", tokens, np.float64), ("encode_params", params, np.float32),
+                           ("decode_trajectories", trajectories, np.float32)):
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.index_select(0, idx).cpu().numpy().astype(dtype))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -721,7 +741,14 @@ def main():
     ap.add_argument("--no-bpe", action="store_true", help="skip the BPE-train / BPE-apply legs")
     ap.add_argument("--no-bpe-cpu-full", action="store_true",
                     help="skip the reference BPE trainer on the full 1.6 M-sequence corpus (about a minute of host time)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the tokens, coefficients and trajectories of the last one to "
+                         f"DIR/<name>.npy (a fixed sample of {DUMP_ROWS} rows of the batch)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the B200 path; it does not apply to --impl reference")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -867,6 +894,9 @@ def main():
     if world > 1:
         dist.barrier()
     ms_total = t_start.elapsed_time(t_end)
+    if args.dump_outputs and rank == 0:
+        last = K - 1                        # step(K - 1): encode of buffer set last % R, decode of set (last + 2) % R
+        dump_outputs(args.dump_outputs, toks[last % R], pars[last % R], outs[(last + 2) % R])
 
     # ---- end-to-end leg: public API, pinned host input, results back on the host.  The step is the same
     # 65 536-trajectory batch, fed as 8 chunks over 3 streams so that the H2D copy of one chunk, the

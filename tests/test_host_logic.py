@@ -215,6 +215,40 @@ def test_bench_reference_arm_contract():
     assert "workload" in line["config"]
 
 
+def test_bench_dump_outputs_writes_a_fixed_sample(tmp_path):
+    """`bench.py --dump-outputs DIR`: float32 / float64 .npy files of at most 64 MB in all, the same seeded rows of
+    every output on every run, every row of a small batch; out-of-range --steps and the reference arm are refused."""
+    import importlib.util
+    import subprocess
+    import sys
+    spec = importlib.util.spec_from_file_location("bench_under_test", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    names = {"encode_tokens.npy", "encode_params.npy", "decode_trajectories.npy"}
+
+    def dump(n, d):
+        row = torch.arange(n, dtype=torch.int64)                   # every value of a row holds the row index
+        bench.dump_outputs(str(d), row[:, None].repeat(1, 140) + 31744, row[:, None].repeat(1, 140).float(),
+                           row[:, None, None].repeat(1, 50, 14).float())
+        assert set(os.listdir(d)) == names
+        out = {f[:-4]: np.load(d / f) for f in names}
+        assert all(a.dtype in (np.float32, np.float64) for a in out.values())
+        assert sum(os.path.getsize(d / f) for f in names) <= 64 << 20
+        rows = out["encode_tokens"][:, 0] - 31744
+        assert np.array_equal(out["encode_params"][:, 0], rows) and np.array_equal(out["decode_trajectories"][:, 0, 0], rows)
+        return rows
+
+    n = bench.DUMP_ROWS + 4099
+    a, b = dump(n, tmp_path / "a"), dump(n, tmp_path / "b")
+    assert a.shape == (bench.DUMP_ROWS,) and np.array_equal(a, b) and np.all(np.diff(a) > 0) and a[-1] < n
+    assert np.array_equal(dump(300, tmp_path / "small"), np.arange(300))
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path / "ref")]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *extra], capture_output=True, text=True,
+                             timeout=120, cwd=ROOT)
+        assert out.returncode == 2 and "error" in out.stderr, out.stderr[-2000:]
+    assert not os.path.exists(tmp_path / "ref")
+
+
 def test_fit_parameters_gathers_small_batches():
     """fit_parameters fits the loader's small batches ~4 096 trajectories at a time (host logic only: the fit and
     the quantile select are stubbed)."""
