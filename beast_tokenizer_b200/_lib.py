@@ -50,6 +50,9 @@ _SIGNATURES = {
     "beast_version": (C.c_char_p, []),
     "beast_launch_count": (C.c_int64, []),
     "beast_debug_disable_fast": (C.c_int, [C.c_int32]),
+    "beast_overlap_count": (C.c_int64, []),
+    "beast_debug_force_wait": (C.c_int, [C.c_int32]),
+    "beast_debug_ranges_conflict": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32]),
     "beast_encode_f32": (C.c_int, [C.c_void_p, c_f32p, C.c_int64, c_f32p, c_f32p, C.c_int64, c_f32p, c_i64p, C.c_void_p]),
     "beast_quantize_f32": (C.c_int, [C.c_void_p, c_f32p, C.c_int64, c_f32p, c_f32p, C.c_int64, c_i64p, C.c_void_p]),
     "beast_normalize_f32": (C.c_int, [C.c_void_p, c_f32p, C.c_int64, c_f32p, c_f32p, c_f32p, C.c_void_p]),
@@ -165,3 +168,7 @@ def stream_ptr(device):
 
 def launch_count():
     return int(load().beast_launch_count())
+
+
+def overlap_count():
+    return int(load().beast_overlap_count())

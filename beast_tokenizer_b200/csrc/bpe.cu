@@ -81,13 +81,10 @@ __device__ __forceinline__ unsigned long long global_ns() {
     asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
     return t;
 }
-constexpr unsigned long long kPeerWaitNs = 5000000000ull;
-// Programmatic dependent launch: the three kernels of a merge iteration are launched with
-// cudaLaunchAttributeProgrammaticStreamSerialization, so the blocks of the next kernel are scheduled while the
-// previous one drains; pdl_wait() blocks until the previous grid has completed and its writes are visible,
-// pdl_launch() lets the next grid start being scheduled.
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_launch() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }     // a peer that stays silent for 5 s is reported, not waited for
+constexpr unsigned long long kPeerWaitNs = 5000000000ull;     // a peer that stays silent for 5 s is reported, not waited for
+// Programmatic dependent launch (pdl_wait / pdl_launch, common.cuh): the three kernels of a merge iteration are
+// launched with cudaLaunchAttributeProgrammaticStreamSerialization, so the blocks of the next kernel are scheduled
+// while the previous one drains.
 
 
 // GPT-2 pre-tokeniser character classes for codepoints 0..255 (SURVEY.md Appendix A.2)

@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <cstdlib>
+#include <utility>
 #include "beast_b200.h"
 
 #ifndef __CUDA_ARCH__
@@ -61,6 +62,60 @@ int launch_decode_tiled(const Plan* p, const long long* tokens, const float* par
 
 extern long long g_launch_count;
 inline void count_launch(int n = 1) { g_launch_count += n; }
+
+// ---------------------------------------------------------------- launch-boundary overlap of K1 / K3 (csrc/plan.cu)
+// A bulk-copy K1 / K3 launch may start streaming while the launch before it drains (it skips griddepcontrol.wait)
+// only when that launch provably is the previous bulk-copy K1 / K3 launch of this library and the two touch disjoint
+// memory.  Adjacency can only be proven inside a stream capture: the dependency set the next captured node gets must
+// be exactly the node recorded right after that launch.  Eager launches never overlap (the library cannot see
+// foreign work enqueued between two of its calls).  Every CTA issues griddepcontrol.launch_dependents only after its
+// own griddepcontrol.wait has returned, so a successor starts only once its predecessor's predecessor has completed:
+// checking against the immediate predecessor is enough.
+struct MemRange {
+    uintptr_t lo, hi;      // bytes [lo, hi)
+    int write;             // 0 = read, 1 = written (or read and written)
+};
+struct LaunchRanges {
+    static constexpr int kMax = 8;
+    MemRange r[kMax];
+    int n = 0;
+    void add(const void* p, size_t bytes, bool write) {
+        if (p && bytes && n < kMax) r[n++] = MemRange{(uintptr_t)p, (uintptr_t)p + bytes, write ? 1 : 0};
+    }
+};
+// read-after-write, write-after-read or write-after-write between two launches; touching and empty ranges never conflict
+bool ranges_conflict(const LaunchRanges& prev, const LaunchRanges& next);
+// Before a bulk-copy K1 / K3 launch on `st`: true when it may overlap its predecessor (launch it with the programmatic
+// stream serialization attribute and wait_first = 0).
+bool overlap_begin(cudaStream_t st, const LaunchRanges& mine);
+// Right after it: records the launch's capture node and ranges for the next launch on `st` (or forgets the stream's
+// record when the launch was eager or failed) and counts overlapped launches.
+void overlap_end(cudaStream_t st, const LaunchRanges& mine, bool overlapped, cudaError_t launch_error);
+// 1 = every bulk-copy K1 / K3 launch waits for its predecessor (beast_debug_force_wait): the A/B measurement and the
+// overlap tests compare against it
+extern int g_force_wait;
+
+template <typename... P, typename... A>
+static inline cudaError_t launch_maybe_overlapped(void (*kernel)(P...), int grid, int block, size_t smem,
+                                                  cudaStream_t st, bool overlap, A&&... args) {
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(grid);
+    cfg.blockDim = dim3(block);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = st;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = overlap ? 1 : 0;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    return cudaLaunchKernelEx(&cfg, kernel, std::forward<A>(args)...);
+}
+
+// Programmatic dependent launch: pdl_wait() blocks until the previous grid has completed and its writes are visible
+// (a no-op when the launch did not allow programmatic serialization); pdl_launch() lets the next grid start being
+// scheduled once every CTA of this one has issued it or exited.
+__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+__device__ __forceinline__ void pdl_launch() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 // 1 = take the one-thread-per-column reference kernels only (beast_debug_disable_fast, or BEAST_B200_DISABLE_FAST=1
 // read once at the first call): the parity tests compare them with the tiled / bulk-copy kernels bit for bit.
 extern int g_disable_fast;

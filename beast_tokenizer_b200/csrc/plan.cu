@@ -1,13 +1,79 @@
 // Plan: immutable per-tokenizer constants (geometry, projector / basis tables) on host and device.
 #include <cstdlib>
 #include <cstring>
+#include <map>
+#include <mutex>
 #include <new>
 #include "common.cuh"
 
 namespace beast {
 long long g_launch_count = 0;
 int g_disable_fast = -1;
+int g_force_wait = 0;
+
+bool ranges_conflict(const LaunchRanges& prev, const LaunchRanges& next) {
+    for (int i = 0; i < prev.n; ++i)
+        for (int j = 0; j < next.n; ++j) {
+            const MemRange &p = prev.r[i], &q = next.r[j];
+            if ((p.write || q.write) && p.lo < q.hi && q.lo < p.hi && p.lo < p.hi && q.lo < q.hi) return true;
+        }
+    return false;
 }
+
+namespace {
+// The last bulk-copy K1 / K3 launch captured on a (device, stream): its capture sequence, its node and its ranges.
+struct LaunchRecord {
+    unsigned long long capture_id;
+    cudaGraphNode_t node;
+    LaunchRanges ranges;
+};
+std::mutex g_record_mutex;
+std::map<std::pair<int, cudaStream_t>, LaunchRecord> g_records;
+long long g_overlap_count = 0;
+
+// The dependency set the next node captured on `st` gets, when it is exactly one node over a plain edge.
+bool single_capture_dependency(cudaStream_t st, unsigned long long* id, cudaGraphNode_t* node) {
+    cudaStreamCaptureStatus status = cudaStreamCaptureStatusNone;
+    const cudaGraphNode_t* deps = nullptr;
+    const cudaGraphEdgeData* edges = nullptr;
+    size_t n = 0;
+    if (cudaStreamGetCaptureInfo_v3(st, &status, id, nullptr, &deps, &edges, &n) != cudaSuccess) {
+        cudaGetLastError();                      // the launch that follows reports any real stream error itself
+        return false;
+    }
+    if (status != cudaStreamCaptureStatusActive || n != 1) return false;
+    if (edges && (edges[0].type != cudaGraphDependencyTypeDefault || edges[0].from_port != 0 || edges[0].to_port != 0))
+        return false;
+    *node = deps[0];
+    return true;
+}
+}  // namespace
+
+bool overlap_begin(cudaStream_t st, const LaunchRanges& mine) {
+    if (g_force_wait) return false;
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess) return false;
+    unsigned long long id = 0;
+    cudaGraphNode_t dep = nullptr;
+    if (!single_capture_dependency(st, &id, &dep)) return false;
+    std::lock_guard<std::mutex> lock(g_record_mutex);
+    auto it = g_records.find({dev, st});
+    return it != g_records.end() && it->second.capture_id == id && it->second.node == dep &&
+           !ranges_conflict(it->second.ranges, mine);
+}
+
+void overlap_end(cudaStream_t st, const LaunchRanges& mine, bool overlapped, cudaError_t launch_error) {
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess) return;
+    unsigned long long id = 0;
+    cudaGraphNode_t node = nullptr;
+    const bool captured = launch_error == cudaSuccess && single_capture_dependency(st, &id, &node);
+    std::lock_guard<std::mutex> lock(g_record_mutex);
+    if (captured) g_records[{dev, st}] = LaunchRecord{id, node, mine};
+    else g_records.erase({dev, st});
+    if (overlapped && launch_error == cudaSuccess) ++g_overlap_count;
+}
+}  // namespace beast
 using beast::Plan;
 
 static float* dup_h(const float* src, size_t n) {
@@ -23,6 +89,23 @@ extern "C" int beast_debug_disable_fast(int32_t flag) {
     const int prev = beast::g_disable_fast == 1 ? 1 : 0;
     beast::g_disable_fast = flag ? 1 : 0;
     return prev;
+}
+extern "C" int64_t beast_overlap_count(void) {
+    std::lock_guard<std::mutex> lock(beast::g_record_mutex);
+    return beast::g_overlap_count;
+}
+extern "C" int beast_debug_force_wait(int32_t flag) {
+    const int prev = beast::g_force_wait;
+    beast::g_force_wait = flag ? 1 : 0;
+    return prev;
+}
+extern "C" int beast_debug_ranges_conflict(const int64_t* prev, int32_t n_prev, const int64_t* next, int32_t n_next) {
+    if (n_prev < 0 || n_next < 0 || n_prev > beast::LaunchRanges::kMax || n_next > beast::LaunchRanges::kMax) return BEAST_E_SHAPE;
+    if ((n_prev && !prev) || (n_next && !next)) return BEAST_E_NULL;
+    beast::LaunchRanges a, b;
+    for (int i = 0; i < n_prev; ++i) a.r[a.n++] = beast::MemRange{(uintptr_t)prev[3 * i], (uintptr_t)prev[3 * i + 1], prev[3 * i + 2] ? 1 : 0};
+    for (int i = 0; i < n_next; ++i) b.r[b.n++] = beast::MemRange{(uintptr_t)next[3 * i], (uintptr_t)next[3 * i + 1], next[3 * i + 2] ? 1 : 0};
+    return beast::ranges_conflict(a, b) ? 1 : 0;
 }
 
 extern "C" int beast_plan_create(const beast_plan_desc_t* d, beast_plan_t** out) {

@@ -22,7 +22,9 @@ namespace beast {
 constexpr int kDecGroupWarps = 7;
 constexpr int kDecGroups = 2;
 constexpr int kDecStages = 5;
-constexpr int kDecThreads = (kDecGroups * kDecGroupWarps + 1) * 32;
+constexpr int kDecCopyWarp = kDecGroups * kDecGroupWarps;
+constexpr int kDecPdlWarp = kDecCopyWarp + 1;          // griddepcontrol only (as in K1)
+constexpr int kDecThreads = (kDecPdlWarp + 1) * 32;
 constexpr int kDecColumns = kDecGroupWarps * 32;
 constexpr int kMaxEvalKnots = 320;       // generic path: num_basis + degree_p <= 319
 
@@ -43,6 +45,7 @@ struct DecArgs {
     long long offset;
     float vm1;
     int D, n_joint, S, n_tiles;
+    int wait_first;        // 0 = may stream while the previous launch drains (disjoint buffers, common.cuh)
     int slot_to_dof[BEAST_MAX_SLOTS];
 };
 
@@ -71,10 +74,11 @@ __device__ __forceinline__ void eval_grip(const DecTables<T, NB>& tab, const flo
 
 // Persistent CTA, one per SM; same stage life cycle as K1 (spline_encode.cu): bulk load of the token
 // tile (+ init_p) -> one 7-warp group pulls its tokens into registers and evaluates -> [t][dof] rows
-// staged over the tile -> bulk store -> reload.
+// staged over the tile -> bulk store -> reload.  Warp 15 and wait_first as in K1.
 template <int T, int NB, int DT>
 __global__ void __launch_bounds__(kDecThreads, 1)
 decode_fast_kernel(const __grid_constant__ DecTables<T, NB> tab, const __grid_constant__ DecArgs a) {
+    if (a.wait_first) pdl_wait();
     extern __shared__ __align__(128) unsigned char smem[];
     __shared__ __align__(8) uint64_t full_bar[kDecStages];
     __shared__ __align__(8) uint64_t out_full_bar[kDecStages];
@@ -97,7 +101,12 @@ decode_fast_kernel(const __grid_constant__ DecTables<T, NB> tab, const __grid_co
     }
     __syncthreads();
 
-    if (warp == kDecGroups * kDecGroupWarps) {
+    if (warp == kDecPdlWarp) {
+        pdl_wait();
+        pdl_launch();
+        return;
+    }
+    if (warp == kDecCopyWarp) {
         if (lane == 0) {
             auto load = [&](int j) {
                 const int s = j % kDecStages;
@@ -317,7 +326,17 @@ static int launch_dec_fast(const Plan* p, const long long* tokens, long long n_t
     static size_t granted[kMaxDevices] = {};
     if (int rc = opt_in_smem(decode_fast_kernel<T, NB, DT>, smem, granted)) return rc;
     const int grid = (int)(n_tiles < p->num_sms ? n_tiles : p->num_sms);
-    decode_fast_kernel<T, NB, DT><<<grid, kDecThreads, smem, st>>>(tab, a);
+    LaunchRanges rg;
+    const size_t n_traj = (size_t)n_tiles * S, n_col = (size_t)p->D * NB;
+    rg.add(tokens, n_traj * n_col * sizeof(long long), false);
+    rg.add(init_p, n_traj * p->D * sizeof(float), false);
+    rg.add(w_min, n_col * sizeof(float), false);
+    rg.add(w_max, n_col * sizeof(float), false);
+    rg.add(out, n_traj * T * p->D * sizeof(float), true);
+    const bool overlap = overlap_begin(st, rg);
+    a.wait_first = overlap ? 0 : 1;
+    const cudaError_t e = launch_maybe_overlapped(decode_fast_kernel<T, NB, DT>, grid, kDecThreads, smem, st, overlap, tab, a);
+    overlap_end(st, rg, overlap, e);
     count_launch();
     BEAST_CHECK_LAUNCH();
     return BEAST_OK;

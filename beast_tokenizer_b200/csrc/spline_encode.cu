@@ -28,7 +28,9 @@ namespace beast {
 constexpr int kEncGroupWarps = 7;                       // 224 columns per tile
 constexpr int kEncGroups = 2;                           // tiles computed concurrently per SM
 constexpr int kEncStages = 5;                           // 5 x 44.8 KB of the 227 KB shared memory
-constexpr int kEncThreads = (kEncGroups * kEncGroupWarps + 1) * 32;
+constexpr int kEncCopyWarp = kEncGroups * kEncGroupWarps;
+constexpr int kEncPdlWarp = kEncCopyWarp + 1;          // griddepcontrol only: no copies, no compute
+constexpr int kEncThreads = (kEncPdlWarp + 1) * 32;
 constexpr int kEncColumns = kEncGroupWarps * 32;
 
 __device__ __forceinline__ void group_barrier(int group) {
@@ -56,6 +58,7 @@ struct EncArgs {
     float* bmax;
     float* mm_ws;          // workspace of the single-launch reduction: [grid][2][D*NB] per-CTA partials + ticket; NULL = atomics
     int mm_accumulate;     // fold the existing contents of bmin / bmax into the result
+    int wait_first;        // 0 = may stream while the previous launch drains (disjoint buffers, common.cuh)
     long long offset;
     float vm1;
     int D, n_joint, S, n_tiles;
@@ -100,9 +103,12 @@ __device__ __forceinline__ void fit_grip(const EncTables<T, NB>& tab, const floa
 //   bulk load in flight -> computed by one 7-warp group -> outputs staged over the tile -> bulk store -> reload.
 // Two groups compute two different tiles at once; the copy thread (warp 14, lane 0) issues every
 // bulk copy.  full[s] (tx-count) hands a stage to its group, out_full[s] (7 warp arrivals) hands it back.
+// Warp 15 waits for the previous grid and only then lets the next one launch (common.cuh: overlap_begin); with
+// wait_first every thread waits before its first global access instead.
 template <int T, int NB, int DT>
 __global__ void __launch_bounds__(kEncThreads, 1)
 encode_fast_kernel(const __grid_constant__ EncTables<T, NB> tab, const __grid_constant__ EncArgs a) {
+    if (a.wait_first) pdl_wait();
     extern __shared__ __align__(128) unsigned char smem[];
     __shared__ __align__(8) uint64_t full_bar[kEncStages];
     __shared__ __align__(8) uint64_t out_full_bar[kEncStages];
@@ -132,7 +138,12 @@ encode_fast_kernel(const __grid_constant__ EncTables<T, NB> tab, const __grid_co
     }
     __syncthreads();
 
-    if (warp == kEncGroups * kEncGroupWarps) {
+    if (warp == kEncPdlWarp) {
+        pdl_wait();
+        pdl_launch();
+        return;
+    }
+    if (warp == kEncCopyWarp) {
         // ---------------- copy thread ----------------
         if (lane == 0) {
             auto load = [&](int j) {
@@ -357,6 +368,7 @@ template <int T, int NB, int DT>
 static int launch_fast(const Plan* p, const float* traj, long long n_tiles, int S, const float* w_min,
                        const float* w_max, long long offset, float* params_out, long long* tokens_out,
                        float* bmin, float* bmax, float* mm_ws, int mm_accumulate, cudaStream_t st) {
+    const int D = p->D;
     EncTables<T, NB> tab;
     constexpr int NBP = EncTables<T, NB>::NBP;
     for (int t = 0; t < T; ++t)
@@ -380,7 +392,19 @@ static int launch_fast(const Plan* p, const float* traj, long long n_tiles, int 
     static size_t granted[kMaxDevices] = {};
     if (int rc = opt_in_smem(encode_fast_kernel<T, NB, DT>, smem, granted)) return rc;
     const int grid = (int)(n_tiles < p->num_sms ? n_tiles : p->num_sms);
-    encode_fast_kernel<T, NB, DT><<<grid, kEncThreads, smem, st>>>(tab, a);
+    LaunchRanges rg;
+    const size_t n_traj = (size_t)n_tiles * S, n_col = (size_t)D * NB;
+    rg.add(traj, n_traj * T * D * sizeof(float), false);
+    if (tokens_out) { rg.add(w_min, n_col * sizeof(float), false); rg.add(w_max, n_col * sizeof(float), false); }
+    rg.add(params_out, n_traj * n_col * sizeof(float), true);
+    rg.add(tokens_out, n_traj * n_col * sizeof(long long), true);
+    rg.add(bmin, n_col * sizeof(float), true);
+    rg.add(bmax, n_col * sizeof(float), true);
+    rg.add(mm_ws, (size_t)beast_fit_minmax_workspace_bytes((const beast_plan_t*)p), true);   // partials + ticket
+    const bool overlap = overlap_begin(st, rg);
+    a.wait_first = overlap ? 0 : 1;
+    const cudaError_t e = launch_maybe_overlapped(encode_fast_kernel<T, NB, DT>, grid, kEncThreads, smem, st, overlap, tab, a);
+    overlap_end(st, rg, overlap, e);
     count_launch();
     BEAST_CHECK_LAUNCH();
     return BEAST_OK;

@@ -85,6 +85,17 @@ int64_t beast_launch_count(void);
  * BEAST_B200_DISABLE_FAST=1 does from the environment); returns the previous setting.  The parity tests compare the
  * tiled / bulk-copy kernels with them bit for bit. */
 int beast_debug_disable_fast(int32_t flag);
+/* Number of bulk-copy K1 / K3 launches made so far that may overlap the launch before them (they stream while it
+ * drains).  Only launches captured into a CUDA graph overlap, and only directly after the previous bulk-copy K1 / K3
+ * launch of this library on the same stream when the two touch disjoint memory. */
+int64_t beast_overlap_count(void);
+/* Test hook: flag != 0 makes every bulk-copy K1 / K3 launch wait for the launch before it (no overlap); returns the
+ * previous setting. */
+int beast_debug_force_wait(int32_t flag);
+/* Test hook: the hazard predicate of the overlap.  prev / next hold n_prev / n_next triples (first byte, end byte,
+ * written != 0) of two launches; returns 1 on a read-after-write, write-after-read or write-after-write conflict,
+ * 0 otherwise (touching and empty ranges never conflict). */
+int beast_debug_ranges_conflict(const int64_t* prev, int32_t n_prev, const int64_t* next, int32_t n_next);
 
 /* ---- K1: fused fit + quantise.  Replaces BEASTBsplineTokenizer.encode
  * (beast/beast_bspline_tokenizer.py:399-428) and compute_weights (:344-360):
