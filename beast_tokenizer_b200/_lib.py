@@ -35,6 +35,14 @@ class PlanDesc(C.Structure):
     ]
 
 
+class GridDesc(C.Structure):
+    """beast_grid_desc_t: one shared time grid and its basis rows of orders 0..max_order (host pointers)."""
+    _fields_ = [
+        ("n_times", C.c_int32), ("max_order", C.c_int32), ("times_h", C.POINTER(C.c_float)),
+        ("rows_joint_h", C.POINTER(C.c_float)), ("rows_grip_h", C.POINTER(C.c_float)),
+    ]
+
+
 BPE_MAX_PEERS = 16
 
 
@@ -63,7 +71,13 @@ _SIGNATURES = {
     "beast_eval_f32": (C.c_int, [C.c_void_p, c_f32p, C.c_int64, c_f32p, c_f32p, C.c_int32, c_f32p, C.c_void_p]),
     "beast_reconstruct_bc_f32": (C.c_int, [C.c_void_p, c_i64p, c_f32p, C.c_int64, c_f32p, c_f32p, C.c_int64, c_f32p, c_f32p,
                                            C.c_int32, c_f32p, c_f32p, c_f32p, C.c_void_p]),
-    "beast_fit_minmax_f32": (C.c_int, [C.c_void_p, c_f32p, C.c_int64, c_f32p, c_f32p, C.c_int32, C.c_void_p]),
+    "beast_grid_create": (C.c_int, [C.c_void_p, C.POINTER(GridDesc), C.POINTER(C.c_void_p)]),
+    "beast_grid_destroy": (C.c_int, [C.c_void_p]),
+    "beast_decode_grid_f32": (C.c_int, [C.c_void_p, C.c_void_p, c_i64p, c_f32p, C.c_int64, c_f32p, c_f32p, C.c_int64,
+                                        c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, C.c_void_p]),
+    "beast_decode_deriv_times_f32": (C.c_int, [C.c_void_p, c_i64p, c_f32p, C.c_int64, c_f32p, c_f32p, C.c_int64, c_f32p,
+                                               c_f32p, C.c_int32, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, C.c_void_p]),
+    "beast_fit_minmax_f32":(C.c_int, [C.c_void_p, c_f32p, C.c_int64, c_f32p, c_f32p, C.c_int32, C.c_void_p]),
     "beast_fit_minmax_workspace_bytes": (C.c_int64, [C.c_void_p]),
     "beast_fit_minmax_ws_f32": (C.c_int, [C.c_void_p, c_f32p, C.c_int64, c_f32p, c_f32p, C.c_int32, C.c_void_p, C.c_int64,
                                           C.c_void_p]),

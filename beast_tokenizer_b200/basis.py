@@ -68,6 +68,100 @@ def bspline_basis(times: torch.Tensor, tau: float, num_basis: int, degree_p: int
     return torch.stack(level[:num_basis], dim=-1).contiguous()
 
 
+def check_orders(orders):
+    """`orders` of the derivative API: a non-empty tuple / list of distinct ints from {0, 1, 2}."""
+    if not isinstance(orders, (tuple, list)) or len(orders) == 0:
+        raise ValueError(f"orders must be a non-empty tuple of distinct values from (0, 1, 2), got {orders!r}")
+    for o in orders:
+        if isinstance(o, bool) or not isinstance(o, int) or o not in (0, 1, 2):
+            raise ValueError(f"orders must hold values from (0, 1, 2), got {orders!r}")
+    if len(set(orders)) != len(orders):
+        raise ValueError(f"orders must be distinct, got {orders!r}")
+    return tuple(int(o) for o in orders)
+
+
+def _deriv_step(level, kn, q, n_out):
+    """d/du of the degree-q basis from the degree-(q-1) rows `level`: N'_i = q * (N_i / (k_{i+q} - k_i) -
+    N_{i+1} / (k_{i+q+1} - k_{i+1})), terms with a zero denominator dropped.  One fp32 rounding per operation, in
+    the order csrc/spline_deriv.cu (deboor_deriv) evaluates them."""
+    out = []
+    for i in range(n_out):
+        d1 = kn[i + q] - kn[i]
+        d2 = kn[i + q + 1] - kn[i + 1]
+        a = None if d1 == 0 else level[i] / d1
+        b = None if d2 == 0 else level[i + 1] / d2
+        if a is None and b is None:
+            v = torch.zeros_like(level[i])
+        elif b is None:
+            v = a
+        elif a is None:
+            v = -b
+        else:
+            v = a - b
+        out.append(v * float(q))
+    return out
+
+
+def bspline_basis_derivatives(times: torch.Tensor, tau: float, num_basis: int, degree_p: int,
+                              max_order: int) -> torch.Tensor:
+    """[max_order + 1, T, num_basis] fp32: row o holds d^o/dt^o of the basis at `times` (o <= 2).
+
+    Order 0 is `bspline_basis` bit for bit (same recursion, same operations).  Orders 1 / 2 are the derivative form
+    of the same triangular recursion on the levels below the top one (`_deriv_step`), divided by tau once per order
+    (t = u * tau).  Intervals are those of the basis: half-open, the last one closed, so an interior knot yields the
+    right-hand derivative and t = 0 / t = tau the one-sided derivative from inside.  Outside [0, tau] the phase is
+    clamped: the position is held and orders 1 / 2 are exactly 0.  csrc/spline_deriv.cu evaluates the same fp32
+    operation sequence in-kernel, so these host rows and the device recursion agree bit for bit."""
+    if isinstance(max_order, bool) or not isinstance(max_order, int) or max_order not in (0, 1, 2):
+        raise ValueError(f"max_order must be 0, 1 or 2, got {max_order!r}")
+    t = times.to(torch.float32)
+    u = linear_phase(t, tau)
+    tau_t = torch.tensor(tau, dtype=torch.float32)
+    raw = (t - torch.tensor(0.0, dtype=torch.float32)) / tau_t
+    outside = (raw < 0) | (raw > 1)
+    kn = knot_vector(num_basis, degree_p)
+    p = degree_p
+    n0 = num_basis + p
+    level = []
+    for i in range(n0):
+        if i == num_basis - 1:
+            inside = (u >= kn[i]) & (u <= kn[i + 1])
+        else:
+            inside = (u >= kn[i]) & (u < kn[i + 1])
+        level.append(inside.to(torch.float32))
+    zero = torch.zeros_like(u)
+    d1 = [zero] * num_basis
+    d2 = [zero] * num_basis
+    for q in range(1, p + 1):
+        if q == p - 1 and max_order >= 2:            # level p-2 -> d/du of level p-1 -> d2/du2 of level p
+            d2 = _deriv_step(_deriv_step(level, kn, p - 1, n0 - (p - 1)), kn, p, num_basis)
+        if q == p and max_order >= 1:                # level p-1 -> d/du of level p
+            d1 = _deriv_step(level, kn, p, num_basis)
+        nxt = []
+        for i in range(n0 - q):
+            e1 = kn[i + q] - kn[i]
+            e2 = kn[i + q + 1] - kn[i + 1]
+            t1 = None if e1 == 0 else (u - kn[i]) / e1 * level[i]
+            t2 = None if e2 == 0 else (kn[i + q + 1] - u) / e2 * level[i + 1]
+            if t1 is None and t2 is None:
+                nxt.append(torch.zeros_like(u))
+            elif t1 is None:
+                nxt.append(t2)
+            elif t2 is None:
+                nxt.append(t1)
+            else:
+                nxt.append(t1 + t2)
+        level = nxt
+    # degree 0: orders 1 / 2 stay exactly 0; degree 1: order 2 does
+    rows = [torch.stack(level[:num_basis], dim=-1)]
+    out = outside.unsqueeze(-1)
+    if max_order >= 1:
+        rows.append(torch.where(out, 0.0, torch.stack(d1, dim=-1) / tau_t))
+    if max_order >= 2:
+        rows.append(torch.where(out, 0.0, torch.stack(d2, dim=-1) / tau_t / tau_t))
+    return torch.stack(rows).contiguous()
+
+
 def ridge_projector(phi: torch.Tensor, reg: float = 1e-9) -> torch.Tensor:
     """P [nb, T] = (Phi^T Phi + reg I)^-1 Phi^T — the closed form of
     `solve(Phi_m^T Phi_m + 1e-9 I, Phi_m^T y)` (uni_bspline.py:564-586) for one DoF block, in fp64,

@@ -17,6 +17,7 @@ from typing import Iterable, List, Optional, Sequence, Union
 import numpy as np
 import torch
 
+from .basis import check_orders
 from .beast_bspline_tokenizer import CONFIG_FILENAME, BEASTBsplineTokenizer
 from .bpe_model import B200ByteLevelBPE
 
@@ -337,6 +338,13 @@ class BEASTBsplineBPETokenizer(BEASTBsplineTokenizer):
         # the reference reaches its overridden decode() (respect_llm_vocab_size=False) through the base method
         discrete = self._bpe_to_discrete(tokens)
         return self._reconstruct_from_mp_tokens(discrete, 0, times, **kwargs)
+
+    def reconstruct_traj_derivatives(self, tokens: Iterable[TokenLike], times: Optional[torch.Tensor] = None,
+                                     orders=(0, 1, 2), **kwargs) -> tuple:
+        # ids -> bins exactly as reconstruct_traj above (offset 0)
+        orders = check_orders(orders)
+        discrete = self._bpe_to_discrete(tokens)
+        return self._derivatives_from_mp_tokens(discrete, 0, times, orders, **kwargs)
 
     def reconstruct_traj_csr(self, flat: torch.Tensor, offsets: torch.Tensor, times=None, **kwargs) -> torch.Tensor:
         return self._reconstruct_from_mp_tokens(self._bpe_csr_to_discrete(flat, offsets), 0, times, **kwargs)

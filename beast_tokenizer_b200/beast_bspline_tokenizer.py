@@ -12,6 +12,7 @@ drop a NaN where torch.min / torch.clamp would propagate it.  Entry points:
 
     encode / compute_weights / encode_continuous  -> beast_encode_f32 (+ quantize / normalize)
     decode / reconstruct_traj(_continuous)        -> beast_decode_f32 / _times / dequantize / eval
+    reconstruct_traj(_continuous)_derivatives     -> beast_decode_grid_f32 / beast_decode_deriv_times_f32
     update_weights_bounds(_per_batch)             -> beast_minmax_f32 + beast_bounds_expand_f32
     fit_parameters                                -> beast_encode_f32 + beast_colselect_f32
 
@@ -28,7 +29,7 @@ import torch
 
 from . import _dist, _lib
 from .base_tokenizer import TokenizerBase
-from .basis import SplineConstants, build_constants, make_times
+from .basis import SplineConstants, bspline_basis_derivatives, build_constants, check_orders, make_times
 
 CONFIG_FILENAME = "beast_tokenizer_config.json"
 
@@ -75,6 +76,39 @@ class _Plan:
         try:
             if getattr(self, "handle", None):
                 self._lib.beast_plan_destroy(self.handle)
+                self.handle = None
+        except Exception:
+            pass
+
+
+class _Grid:
+    """Owns one beast_grid_t: the basis rows of orders 0..max_order on one time grid shared by every trajectory
+    (basis.bspline_basis_derivatives), for the plan it was built for (kept alive with it)."""
+
+    def __init__(self, plan: _Plan, times: torch.Tensor, max_order: int):
+        c = plan.consts
+        nc = c.num_basis + c.init_order + c.end_order
+        times = times.to("cpu", torch.float32).contiguous()
+        rows_j = bspline_basis_derivatives(times, c.tau, nc, c.degree_p, max_order)
+        rows_g = bspline_basis_derivatives(times, c.tau, c.num_basis, 0, max_order) if c.gripper_indices else None
+
+        def fptr(t):
+            return None if t is None else t.numpy().ctypes.data_as(C.POINTER(C.c_float))
+
+        self._keep = [times, rows_j, rows_g]
+        desc = _lib.GridDesc(n_times=int(times.numel()), max_order=int(max_order), times_h=fptr(times),
+                             rows_joint_h=fptr(rows_j), rows_grip_h=fptr(rows_g))
+        handle = C.c_void_p()
+        with torch.cuda.device(plan.device):
+            _lib.check(plan._lib.beast_grid_create(plan.handle, C.byref(desc), C.byref(handle)), "beast_grid_create")
+        self.handle = handle
+        self.plan = plan
+        self.n_times = int(times.numel())
+
+    def __del__(self):
+        try:
+            if getattr(self, "handle", None):
+                self.plan._lib.beast_grid_destroy(self.handle)
                 self.handle = None
         except Exception:
             pass
@@ -176,6 +210,22 @@ class BEASTBsplineTokenizer(TokenizerBase):
                                      self.init_cond_order, self.end_cond_order)
             self._plan_cache = (key, _Plan(consts, self.vocab_size, dev), self.times)
         return self._plan_cache[1]
+
+    _GRID_CACHE_SIZE = 8
+
+    def _grid(self, plan: _Plan, times: torch.Tensor, max_order: int) -> _Grid:
+        """The grid of `times` [Tq] (CPU fp32) for `plan`, cached per (device, plan key, grid bytes, max order)."""
+        plan_key = self._plan_cache[0]
+        cache = self.__dict__.setdefault("_grid_cache", {})
+        key = (plan_key, times.numpy().tobytes(), int(max_order))
+        grid = cache.get(key)
+        if grid is None:
+            for k in [k for k in cache if k[0] != plan_key]:       # grids of a replaced plan
+                del cache[k]
+            while len(cache) >= self._GRID_CACHE_SIZE:
+                cache.pop(next(iter(cache)))
+            grid = cache[key] = _Grid(plan, times, max_order)
+        return grid
 
     def _bounds(self, dev):
         return (self.w_min.to(dev, torch.float32).contiguous(), self.w_max.to(dev, torch.float32).contiguous())
@@ -688,19 +738,10 @@ class BEASTBsplineTokenizer(TokenizerBase):
     def reconstruct_traj_continuous(self, params, times=None, **kwargs):
         """Normalised '(t d)' coefficients -> trajectories (reference :538-582).  Upstream this
         method raises TypeError (beast/utils.py:42 clamps a Python float); here it works."""
-        from .utils import denormalize_tensor
         plan = self._plan()
         dev = plan.device
-        params = params.to(dev)
-        if len(params.shape) == 3:
-            params = params.reshape(params.shape[0], -1)
-        if params.shape[-1] != self.num_basis * self.num_dof:
-            raise ValueError(
-                f"Token dimension {params.shape[-1]} does not match expected {self.num_basis * self.num_dof}.")
+        params = self._denormalize_continuous(params, dev)
         B = params.shape[0]
-        params = params.reshape(B, self.num_basis, self.num_dof).transpose(1, 2).reshape(B, -1)
-        lo, hi = self._bounds(dev)
-        params = denormalize_tensor(params.to(torch.float32), w_min=lo, w_max=hi).contiguous()
         init_p = self._init_p(kwargs, dev, B)
         tq = 0
         if times is not None:
@@ -719,6 +760,80 @@ class BEASTBsplineTokenizer(TokenizerBase):
                                                     _lib.ptr(times), tq, _lib.ptr(out), _lib.stream_ptr(dev)),
                            "beast_eval_f32")
         return out
+
+    def _denormalize_continuous(self, params, dev):
+        """Normalised '(t d)' coefficients -> de-normalised '(d t)' coefficients [B, D*nb] on `dev`."""
+        from .utils import denormalize_tensor
+        params = params.to(dev)
+        if len(params.shape) == 3:
+            params = params.reshape(params.shape[0], -1)
+        if params.shape[-1] != self.num_basis * self.num_dof:
+            raise ValueError(
+                f"Token dimension {params.shape[-1]} does not match expected {self.num_basis * self.num_dof}.")
+        B = params.shape[0]
+        params = params.reshape(B, self.num_basis, self.num_dof).transpose(1, 2).reshape(B, -1)
+        lo, hi = self._bounds(dev)
+        return denormalize_tensor(params.to(torch.float32), w_min=lo, w_max=hi).contiguous()
+
+    # ------------------------------------------------------------------ derivatives
+    @torch.no_grad()
+    def reconstruct_traj_derivatives(self, tokens, times=None, orders=(0, 1, 2), **kwargs):
+        """tokens -> (d^o/dt^o of the decoded trajectory for o in `orders`), each fp32 [B, Tq, num_dof].
+
+        Order 0 is reconstruct_traj's position bit for bit, orders 1 / 2 velocity and acceleration in the units of
+        `times` (exact spline derivatives; one-sided at t = 0 and t = duration, right-hand at an interior knot,
+        exactly 0 outside [0, duration] and for gripper slots).  `times`: None (the tokenizer's own times), one grid
+        [Tq] shared by every trajectory, or [B, Tq] per trajectory.  Tokens, the LLM offset, init_p and the
+        condition-order state behave as in reconstruct_traj."""
+        orders = check_orders(orders)
+        offset = self._llm_vocab_offset() if self.llm_vocab_size is not None else 0   # as reconstruct_traj
+        return self._derivatives_from_mp_tokens(tokens, offset, times, orders, **kwargs)
+
+    @torch.no_grad()
+    def reconstruct_traj_continuous_derivatives(self, params, times=None, orders=(0, 1, 2), **kwargs):
+        """reconstruct_traj_derivatives from the normalised coefficients of encode_continuous."""
+        orders = check_orders(orders)
+        plan = self._plan()
+        params = self._denormalize_continuous(params, plan.device)
+        return self._derivatives(plan, None, params, None, None, 0, times, orders, kwargs)
+
+    def _derivatives_from_mp_tokens(self, tokens, offset, times, orders, **kwargs):
+        plan = self._plan()
+        dev = plan.device
+        tokens = self._flatten_tokens(tokens, dev)
+        lo, hi = self._bounds(dev)
+        return self._derivatives(plan, tokens, None, lo, hi, offset, times, orders, kwargs)
+
+    def _derivatives(self, plan, tokens, params, lo, hi, offset, times, orders, kwargs):
+        dev = plan.device
+        B = (tokens if tokens is not None else params).shape[0]
+        init_p = self._init_p(kwargs, dev, B)
+        bc, bias = self._pinned(B)
+        shared = times is None or torch.as_tensor(times).dim() == 1
+        if shared:                                  # one grid for every trajectory: the tiled kernel
+            grid_t = self.times if times is None else torch.as_tensor(times).detach().to("cpu", torch.float32)
+            grid_t = grid_t.contiguous()
+            tq = grid_t.numel()
+        else:
+            times = self._check_times(times, dev, B)
+            tq = times.shape[1]
+        outs = {o: torch.empty((B, tq, self.num_dof), device=dev, dtype=torch.float32) for o in orders}
+        o0, o1, o2 = (_lib.ptr(outs.get(o)) for o in range(3))
+        if B == 0 or tq == 0:
+            return tuple(outs[o] for o in orders)
+        with torch.cuda.device(dev):
+            if shared:
+                grid = self._grid(plan, grid_t, max(orders))
+                _lib.check(plan._lib.beast_decode_grid_f32(
+                    plan.handle, grid.handle, _lib.ptr(tokens), _lib.ptr(params), B, _lib.ptr(lo), _lib.ptr(hi),
+                    int(offset), _lib.ptr(init_p), _lib.ptr(bc), _lib.ptr(bias), o0, o1, o2, _lib.stream_ptr(dev)),
+                    "beast_decode_grid_f32")
+            else:
+                _lib.check(plan._lib.beast_decode_deriv_times_f32(
+                    plan.handle, _lib.ptr(tokens), _lib.ptr(params), B, _lib.ptr(lo), _lib.ptr(hi), int(offset),
+                    _lib.ptr(init_p), _lib.ptr(times), tq, _lib.ptr(bc), _lib.ptr(bias), o0, o1, o2,
+                    _lib.stream_ptr(dev)), "beast_decode_deriv_times_f32")
+        return tuple(outs[o] for o in orders)
 
     # ------------------------------------------------------------------ evaluation
     def _no_plotting(self, name):

@@ -60,6 +60,10 @@ int launch_encode_tiled(const Plan* p, const float* traj, long long B, const flo
 int launch_decode_tiled(const Plan* p, const long long* tokens, const float* params, long long B, const float* w_min,
                         const float* w_max, long long offset, const float* init_p, float* out, cudaStream_t st);
 
+// Generic kernels that evaluate the basis in-kernel (spline_decode.cu, spline_deriv.cu) keep one level of the
+// recursion per thread: num_ctrlp + degree_p <= 319.
+constexpr int kMaxEvalKnots = 320;
+
 extern long long g_launch_count;
 inline void count_launch(int n = 1) { g_launch_count += n; }
 

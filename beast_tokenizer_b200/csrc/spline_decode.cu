@@ -26,7 +26,6 @@ constexpr int kDecCopyWarp = kDecGroups * kDecGroupWarps;
 constexpr int kDecPdlWarp = kDecCopyWarp + 1;          // griddepcontrol only (as in K1)
 constexpr int kDecThreads = (kDecPdlWarp + 1) * 32;
 constexpr int kDecColumns = kDecGroupWarps * 32;
-constexpr int kMaxEvalKnots = 320;       // generic path: num_basis + degree_p <= 319
 
 template <int T, int NB>
 struct alignas(16) DecTables {

@@ -160,6 +160,53 @@ int beast_eval_f32(const beast_plan_t* plan, const float* params, int64_t B,
                    const float* init_p, const float* times, int32_t Tq,
                    float* traj_out, void* stream);
 
+/* ---- Derivatives of the decoded spline: position, velocity and acceleration (orders 0, 1, 2) on any time grid.
+ *   x^(o)(t) = (1/tau)^o * sum_k N_k^(o)(u(t)) * c_k (+ bias for order 0),  u = clip(t / tau, 0, 1),
+ * with the coefficients of beast_decode_f32 / beast_reconstruct_bc_f32 (tokens or params, init_p, pinned points).
+ * Order 0 equals beast_decode_times_f32 / beast_reconstruct_bc_f32 on the same times bit for bit.  Orders 1 / 2 are
+ * d/dt and d2/dt2 in the units of the times: bias does not contribute, intervals are half-open with the last one
+ * closed (right-hand derivative at an interior knot, one-sided at t = 0 and t = tau), and outside [0, tau] (phase
+ * clamped, position held) they are exactly 0, as are the orders 1 / 2 of degree-0 (gripper) slots.
+ *
+ * A grid: immutable device tables for one time grid [n_times] shared by every trajectory.
+ *   times_h      [n_times] fp32 (host)
+ *   rows_joint_h [max_order+1][n_times][num_ctrlp] fp32 (host): d^o/dt^o of the joint basis at the times, from
+ *                basis.py: bspline_basis_derivatives (num_ctrlp = num_basis + init_cond_order + end_cond_order)
+ *   rows_grip_h  [max_order+1][n_times][num_basis] likewise for the degree-0 gripper basis (NULL without grippers)
+ * beast_grid_create allocates and copies (it synchronises); the grid belongs to `plan` and must be destroyed before
+ * it.  Decoding with a grid reads only the tokens some row of the grid reads. */
+typedef struct beast_grid_desc {
+    int32_t n_times;
+    int32_t max_order;       /* 0, 1 or 2: the highest order the grid can decode */
+    const float* times_h;
+    const float* rows_joint_h;
+    const float* rows_grip_h;
+} beast_grid_desc_t;
+
+typedef struct beast_grid beast_grid_t;
+
+int beast_grid_create(const beast_plan_t* plan, const beast_grid_desc_t* desc, beast_grid_t** grid_out);
+int beast_grid_destroy(beast_grid_t* grid);
+
+/* Orders 0..2 on a grid: exactly one of tokens [B, nb*D] int64 '(t d)' / params [B, D*nb] fp32 '(d t)' (already
+ * de-normalised) is non-NULL; w_min / w_max / offset as beast_decode_f32 (tokens only); init_p [B, num_dof] or NULL;
+ * bc / bias as beast_reconstruct_bc_f32 (required / nullable when the plan pins control points, else ignored).
+ * outO [B, n_times, num_dof] fp32 receives order O; any of them may be NULL, at least one is set, and none above
+ * the grid's max_order.  Without pinned points one tiled kernel writes every requested order in one pass over the
+ * tokens; with pinned points (or beast_debug_disable_fast) the generic kernel evaluates the basis in-kernel. */
+int beast_decode_grid_f32(const beast_plan_t* plan, const beast_grid_t* grid, const int64_t* tokens,
+                          const float* params, int64_t B, const float* w_min, const float* w_max, int64_t offset,
+                          const float* init_p, const float* bc, const float* bias,
+                          float* out0, float* out1, float* out2, void* stream);
+
+/* Same with per-trajectory times [B, Tq]: one thread per (trajectory, sample) runs the de Boor recursion in-kernel
+ * and takes orders 1 / 2 from the levels below the top one.  BEAST_E_UNSUPPORTED when num_ctrlp + degree_p + 1 > 320.
+ * outO [B, Tq, num_dof]. */
+int beast_decode_deriv_times_f32(const beast_plan_t* plan, const int64_t* tokens, const float* params, int64_t B,
+                                 const float* w_min, const float* w_max, int64_t offset, const float* init_p,
+                                 const float* times, int32_t Tq, const float* bc, const float* bias,
+                                 float* out0, float* out1, float* out2, void* stream);
+
 /* ---- K2: bounds.
  * Column min/max of x [rows, cols] (update_weights_bounds :377-378; the reduction inside
  * update_weights_bounds_per_batch :382-383).  accumulate != 0 folds into the existing
