@@ -13,6 +13,8 @@ drop a NaN where torch.min / torch.clamp would propagate it.  Entry points:
     encode / compute_weights / encode_continuous  -> beast_encode_f32 (+ quantize / normalize)
     decode / reconstruct_traj(_continuous)        -> beast_decode_f32 / _times / dequantize / eval
     reconstruct_traj(_continuous)_derivatives     -> beast_decode_grid_f32 / beast_decode_deriv_times_f32
+    reconstruct_traj_continuous(_derivatives)
+        backward (autograd)                       -> beast_decode_grid_backward_f32 / beast_decode_deriv_times_backward_f32
     update_weights_bounds(_per_batch)             -> beast_minmax_f32 + beast_bounds_expand_f32
     fit_parameters                                -> beast_encode_f32 + beast_colselect_f32
 
@@ -26,6 +28,7 @@ from typing import Optional
 
 import numpy as np
 import torch
+from torch.autograd.function import once_differentiable
 
 from . import _dist, _lib
 from .base_tokenizer import TokenizerBase
@@ -112,6 +115,63 @@ class _Grid:
                 self.handle = None
         except Exception:
             pass
+
+
+class _Adjoint:
+    """The backward launch of one continuous decode: the gradients of its outputs (orders `orders`) -> the gradients
+    of the de-normalised '(d t)' coefficients [B, D*nb] and of init_p [B, num_dof].  A grid (shared times) takes
+    beast_decode_grid_backward_f32, per-row times [B, Tq] beast_decode_deriv_times_backward_f32."""
+
+    def __init__(self, plan: _Plan, batch: int, orders, grid: Optional[_Grid], times, tq: int, init_p_used: bool):
+        self.plan, self.batch, self.orders, self.grid = plan, batch, orders, grid
+        self.times, self.tq, self.init_p_used = times, tq, init_p_used
+
+    def __call__(self, grads, want_init_p):
+        plan, B, dev = self.plan, self.batch, self.plan.device
+        by_order = dict(zip(self.orders, grads))
+        g = [by_order.get(o) for o in range(3)]
+        if all(x is None for x in g):
+            return None, None
+        g = [None if x is None else x.to(dev, torch.float32).contiguous() for x in g]
+        c = plan.consts
+        grad_params = torch.empty((B, c.num_dof * c.num_basis), device=dev, dtype=torch.float32)
+        grad_init_p = (torch.empty((B, c.num_dof), device=dev, dtype=torch.float32)
+                       if self.init_p_used and want_init_p else None)
+        if B == 0 or self.tq == 0:      # no sample reads a coefficient
+            grad_params.zero_()
+            if grad_init_p is not None:
+                grad_init_p.zero_()
+            return grad_params, grad_init_p
+        args = (*[_lib.ptr(x) for x in g], int(self.init_p_used), _lib.ptr(grad_params), _lib.ptr(grad_init_p),
+                _lib.stream_ptr(dev))
+        with torch.cuda.device(dev):
+            if self.grid is not None:
+                _lib.check(plan._lib.beast_decode_grid_backward_f32(plan.handle, self.grid.handle, B, *args),
+                           "beast_decode_grid_backward_f32")
+            else:                       # per-row times, or an empty grid (every gradient is then 0)
+                _lib.check(plan._lib.beast_decode_deriv_times_backward_f32(plan.handle, B, _lib.ptr(self.times),
+                                                                           self.tq, *args),
+                           "beast_decode_deriv_times_backward_f32")
+        return grad_params, grad_init_p
+
+
+class _SplineDecodeFn(torch.autograd.Function):
+    """The coefficient contraction of reconstruct_traj_continuous(_derivatives) as an autograd node: forward = the
+    decode launch (`decode(params, init_p)` -> tuple of outputs), backward = its adjoint launch.  Denormalising and the
+    layout transposition stay torch ops in front of it.  Outputs the loss does not use arrive as None and are passed
+    to the kernel as NULL.  The map is linear, so the backward needs no saved tensors; it is not itself differentiable."""
+
+    @staticmethod
+    def forward(ctx, decode, adjoint, params, init_p):
+        ctx.set_materialize_grads(False)
+        ctx.adjoint = adjoint
+        return decode(params, init_p)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, *grads):
+        grad_params, grad_init_p = ctx.adjoint(grads, ctx.needs_input_grad[3])
+        return None, None, grad_params if ctx.needs_input_grad[2] else None, grad_init_p
 
 
 class BEASTBsplineTokenizer(TokenizerBase):
@@ -734,10 +794,27 @@ class BEASTBsplineTokenizer(TokenizerBase):
                                                             _lib.stream_ptr(dev)), "beast_decode_times_f32")
         return out
 
-    @torch.no_grad()
+    def _continuous_needs_grad(self, params, kwargs) -> bool:
+        """Grad mode is on and `params` or a used init_p requires grad: the continuous decode is then recorded."""
+        if not torch.is_grad_enabled():
+            return False
+        init_p = kwargs.get("init_p") if self.init_pos else None
+        return any(isinstance(t, torch.Tensor) and t.requires_grad for t in (params, init_p))
+
     def reconstruct_traj_continuous(self, params, times=None, **kwargs):
         """Normalised '(t d)' coefficients -> trajectories (reference :538-582).  Upstream this
-        method raises TypeError (beast/utils.py:42 clamps a Python float); here it works."""
+        method raises TypeError (beast/utils.py:42 clamps a Python float); here it works.
+
+        Differentiable with respect to `params` and `init_p` (when `params` or `init_p` requires grad under grad
+        mode): the backward is beast_decode_grid_backward_f32 (times None) / beast_decode_deriv_times_backward_f32
+        (times [B, T']).  `times`, the condition-order boundary state and w_min / w_max as the kernels see them are
+        constants; the clamp of the normalised coefficients passes no gradient where |params| > 1."""
+        if not self._continuous_needs_grad(params, kwargs):
+            with torch.no_grad():
+                return self._reconstruct_continuous(params, times, kwargs, False)
+        return self._reconstruct_continuous(params, times, kwargs, True)
+
+    def _reconstruct_continuous(self, params, times, kwargs, grad):
         plan = self._plan()
         dev = plan.device
         params = self._denormalize_continuous(params, dev)
@@ -747,19 +824,29 @@ class BEASTBsplineTokenizer(TokenizerBase):
         if times is not None:
             times = self._check_times(times, dev, B)
             tq = times.shape[1]
-        out = torch.empty((B, tq if times is not None else plan.consts.seq_len, self.num_dof), device=dev,
-                          dtype=torch.float32)
         bc, bias = self._pinned(B)
-        with torch.cuda.device(dev):
-            if bc is not None:
-                _lib.check(plan._lib.beast_reconstruct_bc_f32(
-                    plan.handle, None, _lib.ptr(params), B, None, None, 0, _lib.ptr(init_p), _lib.ptr(times), tq,
-                    _lib.ptr(bc), _lib.ptr(bias), _lib.ptr(out), _lib.stream_ptr(dev)), "beast_reconstruct_bc_f32")
-            else:
-                _lib.check(plan._lib.beast_eval_f32(plan.handle, _lib.ptr(params), B, _lib.ptr(init_p),
-                                                    _lib.ptr(times), tq, _lib.ptr(out), _lib.stream_ptr(dev)),
-                           "beast_eval_f32")
-        return out
+
+        def decode(params, init_p):
+            out = torch.empty((B, tq if times is not None else plan.consts.seq_len, self.num_dof), device=dev,
+                              dtype=torch.float32)
+            with torch.cuda.device(dev):
+                if bc is not None:
+                    _lib.check(plan._lib.beast_reconstruct_bc_f32(
+                        plan.handle, None, _lib.ptr(params), B, None, None, 0, _lib.ptr(init_p), _lib.ptr(times), tq,
+                        _lib.ptr(bc), _lib.ptr(bias), _lib.ptr(out), _lib.stream_ptr(dev)), "beast_reconstruct_bc_f32")
+                else:
+                    _lib.check(plan._lib.beast_eval_f32(plan.handle, _lib.ptr(params), B, _lib.ptr(init_p),
+                                                        _lib.ptr(times), tq, _lib.ptr(out), _lib.stream_ptr(dev)),
+                               "beast_eval_f32")
+            return (out,)
+
+        if not grad:
+            return decode(params, init_p)[0]
+        # the positions on the tokenizer's own times are the order-0 rows of its grid bit for bit
+        grid = self._grid(plan, self.times.contiguous(), 0) if times is None else None
+        adjoint = _Adjoint(plan, B, (0,), grid, times, tq if times is not None else plan.consts.seq_len,
+                           init_p is not None)
+        return _SplineDecodeFn.apply(decode, adjoint, params, init_p)[0]
 
     def _denormalize_continuous(self, params, dev):
         """Normalised '(t d)' coefficients -> de-normalised '(d t)' coefficients [B, D*nb] on `dev`."""
@@ -771,7 +858,8 @@ class BEASTBsplineTokenizer(TokenizerBase):
             raise ValueError(
                 f"Token dimension {params.shape[-1]} does not match expected {self.num_basis * self.num_dof}.")
         B = params.shape[0]
-        params = params.reshape(B, self.num_basis, self.num_dof).transpose(1, 2).reshape(B, -1)
+        n = self.num_basis * self.num_dof
+        params = params.reshape(B, self.num_basis, self.num_dof).transpose(1, 2).reshape(B, n)
         lo, hi = self._bounds(dev)
         return denormalize_tensor(params.to(torch.float32), w_min=lo, w_max=hi).contiguous()
 
@@ -789,13 +877,23 @@ class BEASTBsplineTokenizer(TokenizerBase):
         offset = self._llm_vocab_offset() if self.llm_vocab_size is not None else 0   # as reconstruct_traj
         return self._derivatives_from_mp_tokens(tokens, offset, times, orders, **kwargs)
 
-    @torch.no_grad()
     def reconstruct_traj_continuous_derivatives(self, params, times=None, orders=(0, 1, 2), **kwargs):
-        """reconstruct_traj_derivatives from the normalised coefficients of encode_continuous."""
+        """reconstruct_traj_derivatives from the normalised coefficients of encode_continuous.
+
+        Differentiable with respect to `params` and `init_p` (when either requires grad under grad mode), for every
+        form of `times` and any subset of `orders`: the backward is beast_decode_grid_backward_f32 on the grid the
+        forward used (times None or [Tq]) / beast_decode_deriv_times_backward_f32 (times [B, Tq]).  `times`, the
+        condition-order boundary state and w_min / w_max as the kernels see them are constants; the clamp of the
+        normalised coefficients passes no gradient where |params| > 1."""
         orders = check_orders(orders)
+        if not self._continuous_needs_grad(params, kwargs):
+            with torch.no_grad():
+                plan = self._plan()
+                params = self._denormalize_continuous(params, plan.device)
+                return self._derivatives(plan, None, params, None, None, 0, times, orders, kwargs)
         plan = self._plan()
         params = self._denormalize_continuous(params, plan.device)
-        return self._derivatives(plan, None, params, None, None, 0, times, orders, kwargs)
+        return self._derivatives(plan, None, params, None, None, 0, times, orders, kwargs, grad=True)
 
     def _derivatives_from_mp_tokens(self, tokens, offset, times, orders, **kwargs):
         plan = self._plan()
@@ -804,7 +902,7 @@ class BEASTBsplineTokenizer(TokenizerBase):
         lo, hi = self._bounds(dev)
         return self._derivatives(plan, tokens, None, lo, hi, offset, times, orders, kwargs)
 
-    def _derivatives(self, plan, tokens, params, lo, hi, offset, times, orders, kwargs):
+    def _derivatives(self, plan, tokens, params, lo, hi, offset, times, orders, kwargs, grad=False):
         dev = plan.device
         B = (tokens if tokens is not None else params).shape[0]
         init_p = self._init_p(kwargs, dev, B)
@@ -817,23 +915,30 @@ class BEASTBsplineTokenizer(TokenizerBase):
         else:
             times = self._check_times(times, dev, B)
             tq = times.shape[1]
-        outs = {o: torch.empty((B, tq, self.num_dof), device=dev, dtype=torch.float32) for o in orders}
-        o0, o1, o2 = (_lib.ptr(outs.get(o)) for o in range(3))
-        if B == 0 or tq == 0:
+        grid = self._grid(plan, grid_t, max(orders)) if shared and B > 0 and tq > 0 else None
+
+        def decode(params, init_p):
+            outs = {o: torch.empty((B, tq, self.num_dof), device=dev, dtype=torch.float32) for o in orders}
+            o0, o1, o2 = (_lib.ptr(outs.get(o)) for o in range(3))
+            if B == 0 or tq == 0:
+                return tuple(outs[o] for o in orders)
+            with torch.cuda.device(dev):
+                if shared:
+                    _lib.check(plan._lib.beast_decode_grid_f32(
+                        plan.handle, grid.handle, _lib.ptr(tokens), _lib.ptr(params), B, _lib.ptr(lo), _lib.ptr(hi),
+                        int(offset), _lib.ptr(init_p), _lib.ptr(bc), _lib.ptr(bias), o0, o1, o2,
+                        _lib.stream_ptr(dev)), "beast_decode_grid_f32")
+                else:
+                    _lib.check(plan._lib.beast_decode_deriv_times_f32(
+                        plan.handle, _lib.ptr(tokens), _lib.ptr(params), B, _lib.ptr(lo), _lib.ptr(hi), int(offset),
+                        _lib.ptr(init_p), _lib.ptr(times), tq, _lib.ptr(bc), _lib.ptr(bias), o0, o1, o2,
+                        _lib.stream_ptr(dev)), "beast_decode_deriv_times_f32")
             return tuple(outs[o] for o in orders)
-        with torch.cuda.device(dev):
-            if shared:
-                grid = self._grid(plan, grid_t, max(orders))
-                _lib.check(plan._lib.beast_decode_grid_f32(
-                    plan.handle, grid.handle, _lib.ptr(tokens), _lib.ptr(params), B, _lib.ptr(lo), _lib.ptr(hi),
-                    int(offset), _lib.ptr(init_p), _lib.ptr(bc), _lib.ptr(bias), o0, o1, o2, _lib.stream_ptr(dev)),
-                    "beast_decode_grid_f32")
-            else:
-                _lib.check(plan._lib.beast_decode_deriv_times_f32(
-                    plan.handle, _lib.ptr(tokens), _lib.ptr(params), B, _lib.ptr(lo), _lib.ptr(hi), int(offset),
-                    _lib.ptr(init_p), _lib.ptr(times), tq, _lib.ptr(bc), _lib.ptr(bias), o0, o1, o2,
-                    _lib.stream_ptr(dev)), "beast_decode_deriv_times_f32")
-        return tuple(outs[o] for o in orders)
+
+        if not grad:
+            return decode(params, init_p)
+        adjoint = _Adjoint(plan, B, orders, grid, None if shared else times, tq, init_p is not None)
+        return _SplineDecodeFn.apply(decode, adjoint, params, init_p)
 
     # ------------------------------------------------------------------ evaluation
     def _no_plotting(self, name):

@@ -17,68 +17,11 @@
 #include <cstdlib>
 #include <cstring>
 #include <new>
-#include "common.cuh"
+#include "spline_deriv.cuh"
 
 namespace beast {
 
 constexpr int kDerivThreads = 512;
-
-struct Grid {
-    const Plan* plan;
-    int Tq, max_order;
-    float* dev_block;     // times [Tq], rows_j [(max_order+1)][Tq][nc], rows_g [(max_order+1)][Tq][nb] (grippers only)
-    float* times_d;
-    float* rows_j_d;
-    float* rows_g_d;
-    int* bands_d;         // [joint | gripper][Tq][lo, hi): union over the orders of the non-zero columns of each row
-    int* list_d;          // dec_list of the grid: token positions some row reads, k | slot << 16 | gripper << 31
-    int n_dec;
-    int band_max;
-};
-
-// d/du of the degree-q basis from the degree-(q-1) values `in` (n entries out); in place when out == in.
-__device__ inline void deriv_step(const float* __restrict__ kn, int q, const float* in, float* out, int n) {
-    const float fq = (float)q;
-    for (int i = 0; i < n; ++i) {
-        const float d1 = __fsub_rn(kn[i + q], kn[i]);
-        const float d2 = __fsub_rn(kn[i + q + 1], kn[i + 1]);
-        const bool h1 = d1 != 0.0f, h2 = d2 != 0.0f;
-        const float a = h1 ? __fdiv_rn(in[i], d1) : 0.0f;
-        const float b = h2 ? __fdiv_rn(in[i + 1], d2) : 0.0f;
-        const float v = (h1 && h2) ? __fsub_rn(a, b) : (h1 ? a : (h2 ? -b : 0.0f));
-        out[i] = __fmul_rn(v, fq);
-    }
-}
-
-// Cox-de Boor exactly as deboor_basis (spline_decode.cu): N[0..nb) <- basis values at u; D1 / D2 [0..nb) <- d/du and
-// d2/du2 when max_order >= 1 / 2, taken from levels p-1 / p-2 before they are overwritten.
-__device__ inline void deboor_deriv(const float* __restrict__ kn, int nb, int p, float u, int max_order, float* N,
-                                    float* D1, float* D2) {
-    const int n0 = nb + p;
-    for (int i = 0; i < n0; ++i) {
-        const bool in = (u >= kn[i]) && (i == nb - 1 ? (u <= kn[i + 1]) : (u < kn[i + 1]));
-        N[i] = in ? 1.0f : 0.0f;
-    }
-    if (max_order >= 1 && p < 1)
-        for (int i = 0; i < nb; ++i) D1[i] = 0.0f;
-    if (max_order >= 2 && p < 2)
-        for (int i = 0; i < nb; ++i) D2[i] = 0.0f;
-    for (int k = 1; k <= p; ++k) {
-        if (k == p - 1 && max_order >= 2) {
-            deriv_step(kn, p - 1, N, D2, n0 - (p - 1));      // d/du of level p-1
-            deriv_step(kn, p, D2, D2, nb);                   // d2/du2 of level p
-        }
-        if (k == p && max_order >= 1) deriv_step(kn, p, N, D1, nb);
-        for (int i = 0; i < n0 - k; ++i) {
-            const float d1 = __fsub_rn(kn[i + k], kn[i]);
-            const float d2 = __fsub_rn(kn[i + k + 1], kn[i + 1]);
-            const bool h1 = d1 != 0.0f, h2 = d2 != 0.0f;
-            const float t1 = h1 ? __fmul_rn(__fdiv_rn(__fsub_rn(u, kn[i]), d1), N[i]) : 0.0f;
-            const float t2 = h2 ? __fmul_rn(__fdiv_rn(__fsub_rn(kn[i + k + 1], u), d2), N[i + 1]) : 0.0f;
-            N[i] = (h1 && h2) ? __fadd_rn(t1, t2) : (h1 ? t1 : t2);
-        }
-    }
-}
 
 struct DerivGenericArgs {
     const long long* tokens;
@@ -465,11 +408,13 @@ extern "C" int beast_grid_create(const beast_plan_t* plan, const beast_grid_desc
         int* bands = (int*)calloc((size_t)4 * Tq, sizeof(int));
         char* used = (char*)calloc((size_t)2 * nb, 1);
         int* list = (int*)malloc(((size_t)p->D * nb + 1) * sizeof(int));
-        if (!bands || !used || !list) {
-            free(bands); free(used); free(list);
+        int* colsup = (int*)malloc((size_t)4 * nb * sizeof(int));    // column supports of the adjoint (no row: [0, 0))
+        if (!bands || !used || !list || !colsup) {
+            free(bands); free(used); free(list); free(colsup);
             beast_grid_destroy((beast_grid_t*)g);
             return BEAST_E_NOMEM;
         }
+        for (int i = 0; i < 2 * nb; ++i) { colsup[2 * i] = Tq; colsup[2 * i + 1] = 0; }
         for (int side = 0; side < (has_grip ? 2 : 1); ++side) {
             const float* rows = side ? d->rows_grip_h : d->rows_joint_h;
             for (int t = 0; t < Tq; ++t) {
@@ -480,10 +425,17 @@ extern "C" int beast_grid_create(const beast_plan_t* plan, const beast_grid_desc
                 if (lo >= hi) lo = hi = 0;
                 bands[2 * (side * Tq + t)] = lo;
                 bands[2 * (side * Tq + t) + 1] = hi;
-                for (int k = lo; k < hi; ++k) used[side * nb + k] = 1;
+                for (int k = lo; k < hi; ++k) {
+                    used[side * nb + k] = 1;
+                    int* cs = colsup + 2 * (side * nb + k);
+                    if (t < cs[0]) cs[0] = t;
+                    cs[1] = t + 1;
+                }
                 if (hi - lo > g->band_max) g->band_max = hi - lo;
             }
         }
+        for (int i = 0; i < 2 * nb; ++i)
+            if (colsup[2 * i] >= colsup[2 * i + 1]) colsup[2 * i] = colsup[2 * i + 1] = 0;
         int n_dec = 0;
         for (int k = 0; k < nb; ++k)
             for (int slot = 0; slot < p->D; ++slot) {
@@ -495,7 +447,9 @@ extern "C" int beast_grid_create(const beast_plan_t* plan, const beast_grid_desc
         if (e == cudaSuccess) e = cudaMemcpy(g->bands_d, bands, (size_t)4 * Tq * sizeof(int), cudaMemcpyHostToDevice);
         if (e == cudaSuccess) e = cudaMalloc((void**)&g->list_d, ((size_t)n_dec + 1) * sizeof(int));
         if (e == cudaSuccess && n_dec) e = cudaMemcpy(g->list_d, list, (size_t)n_dec * sizeof(int), cudaMemcpyHostToDevice);
-        free(bands); free(used); free(list);
+        if (e == cudaSuccess) e = cudaMalloc((void**)&g->colsup_d, (size_t)4 * nb * sizeof(int));
+        if (e == cudaSuccess) e = cudaMemcpy(g->colsup_d, colsup, (size_t)4 * nb * sizeof(int), cudaMemcpyHostToDevice);
+        free(bands); free(used); free(list); free(colsup);
         if (e != cudaSuccess) { beast_grid_destroy((beast_grid_t*)g); return (int)e; }
     }
     *out = (beast_grid_t*)g;
@@ -508,6 +462,7 @@ extern "C" int beast_grid_destroy(beast_grid_t* grid) {
     if (g->dev_block) cudaFree(g->dev_block);
     if (g->bands_d) cudaFree(g->bands_d);
     if (g->list_d) cudaFree(g->list_d);
+    if (g->colsup_d) cudaFree(g->colsup_d);
     delete g;
     return BEAST_OK;
 }

@@ -207,6 +207,27 @@ int beast_decode_deriv_times_f32(const beast_plan_t* plan, const int64_t* tokens
                                  const float* times, int32_t Tq, const float* bc, const float* bias,
                                  float* out0, float* out1, float* out2, void* stream);
 
+/* ---- Adjoint of the two calls above for given coefficients (reconstruct_traj_continuous(_derivatives) backward):
+ *   grad_params[b, slot, k] = sum_t sum_o R_o[t, k] * gradO[b, t, dof(slot)]
+ * with R_o the rows the forward multiplies coefficient k of that slot with (joint basis for joint slots; the degree-0
+ * basis and order 0 only for gripper slots, whose orders 1 / 2 are 0).  gradO [B, n_times (Tq), num_dof] fp32 is the
+ * gradient of outO, NULL = zero (at least one is set, none above the grid's max_order).  grad_params [B, D*nb]
+ * '(d t)' receives the gradient of params.  Pinned control points, bias and the times are constants: with pinned
+ * points only the nb free columns exist in params.  init_p_used != 0: the forward took init_p (coefficient 0 of every
+ * joint slot := init_p[b, dof]); that entry of grad_params is then 0 and grad_init_p [B, num_dof] (nullable; NULL
+ * unless init_p_used) receives it, 0 for gripper DoFs.  Every element of grad_params / grad_init_p is written (no
+ * accumulation, no memset needed).  Deterministic, no atomics: each element is one fp32 sum over t ascending and, for
+ * each t, the orders ascending (fmaf); terms with an exactly-zero basis value may be skipped, which does not change
+ * the value for finite gradients, so the tiled and generic kernels agree.  On a grid without pinned points a tiled
+ * kernel streams the gradients through shared memory once; otherwise (and under beast_debug_disable_fast) the generic
+ * kernel evaluates the basis in-kernel.  Per-row times: BEAST_E_UNSUPPORTED when num_ctrlp + degree_p + 1 > 320. */
+int beast_decode_grid_backward_f32(const beast_plan_t* plan, const beast_grid_t* grid, int64_t B,
+                                   const float* grad0, const float* grad1, const float* grad2, int32_t init_p_used,
+                                   float* grad_params, float* grad_init_p, void* stream);
+int beast_decode_deriv_times_backward_f32(const beast_plan_t* plan, int64_t B, const float* times, int32_t Tq,
+                                          const float* grad0, const float* grad1, const float* grad2,
+                                          int32_t init_p_used, float* grad_params, float* grad_init_p, void* stream);
+
 /* ---- K2: bounds.
  * Column min/max of x [rows, cols] (update_weights_bounds :377-378; the reduction inside
  * update_weights_bounds_per_batch :382-383).  accumulate != 0 folds into the existing
