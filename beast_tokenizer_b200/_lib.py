@@ -81,6 +81,8 @@ _SIGNATURES = {
                                                  c_f32p, c_f32p, C.c_void_p]),
     "beast_decode_deriv_times_backward_f32": (C.c_int, [C.c_void_p, C.c_int64, c_f32p, C.c_int32, c_f32p, c_f32p, c_f32p,
                                                         C.c_int32, c_f32p, c_f32p, C.c_void_p]),
+    "beast_fit_backward_f32": (C.c_int, [C.c_void_p, C.c_int64, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p,
+                                         C.c_void_p]),
     "beast_fit_minmax_f32":(C.c_int, [C.c_void_p, c_f32p, C.c_int64, c_f32p, c_f32p, C.c_int32, C.c_void_p]),
     "beast_fit_minmax_workspace_bytes": (C.c_int64, [C.c_void_p]),
     "beast_fit_minmax_ws_f32": (C.c_int, [C.c_void_p, c_f32p, C.c_int64, c_f32p, c_f32p, C.c_int32, C.c_void_p, C.c_int64,

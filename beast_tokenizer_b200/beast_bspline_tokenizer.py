@@ -15,6 +15,7 @@ drop a NaN where torch.min / torch.clamp would propagate it.  Entry points:
     reconstruct_traj(_continuous)_derivatives     -> beast_decode_grid_f32 / beast_decode_deriv_times_f32
     reconstruct_traj_continuous(_derivatives)
         backward (autograd)                       -> beast_decode_grid_backward_f32 / beast_decode_deriv_times_backward_f32
+    encode_continuous backward (autograd)         -> beast_fit_backward_f32
     update_weights_bounds(_per_batch)             -> beast_minmax_f32 + beast_bounds_expand_f32
     fit_parameters                                -> beast_encode_f32 + beast_colselect_f32
 
@@ -174,6 +175,42 @@ class _SplineDecodeFn(torch.autograd.Function):
         return None, None, grad_params if ctx.needs_input_grad[2] else None, grad_init_p
 
 
+class _FitFn(torch.autograd.Function):
+    """encode_continuous's fit and normalisation as an autograd node: forward = `fit(x)` (the K1 launch, the optional
+    bounds expansion and beast_normalize_f32, unchanged) -> (normalised, params, (w_min, w_max) snapshot), backward =
+    one beast_fit_backward_f32 launch.  The unclamped params and the bounds the forward normalised with are saved; an
+    output the loss does not use arrives as None and is passed to the kernel as NULL.  Not itself differentiable."""
+
+    @staticmethod
+    def forward(ctx, fit, plan, x):
+        ctx.set_materialize_grads(False)
+        normalised, params, bounds = fit(x)
+        ctx.plan, ctx.bounds = plan, bounds
+        ctx.save_for_backward(params)
+        return normalised, params
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_norm, grad_params):
+        if grad_norm is None and grad_params is None:
+            return None, None, None
+        plan = ctx.plan
+        (params,), (lo, hi) = ctx.saved_tensors, ctx.bounds
+        dev = plan.device
+        c = plan.consts
+        grad_norm, grad_params = (None if g is None else g.to(dev, torch.float32).contiguous()
+                                  for g in (grad_norm, grad_params))
+        B = params.shape[0]
+        grad_traj = torch.empty((B, c.seq_len, c.num_dof), device=dev, dtype=torch.float32)
+        if B == 0:                      # empty tensors carry no data pointer
+            return None, None, grad_traj
+        with torch.cuda.device(dev):
+            _lib.check(plan._lib.beast_fit_backward_f32(
+                plan.handle, B, _lib.ptr(grad_norm), _lib.ptr(grad_params), _lib.ptr(params), _lib.ptr(lo),
+                _lib.ptr(hi), _lib.ptr(grad_traj), _lib.stream_ptr(dev)), "beast_fit_backward_f32")
+        return None, None, grad_traj
+
+
 class BEASTBsplineTokenizer(TokenizerBase):
 
     def __init__(self, num_dof=1, num_basis=10, duration=2 * torch.pi, seq_len=50, vocab_size=256,
@@ -331,6 +368,10 @@ class BEASTBsplineTokenizer(TokenizerBase):
         boundary samples y[0], y[1], y[-2], y[-1] only — O(B*D) elementwise work next to the fit."""
         if not self._has_conditions:
             return
+        self._boundary = self._boundary_state(x, plan)
+
+    def _boundary_state(self, x, plan):
+        """The boundary state of `x` (torch ops: attached to the graph of `x` under grad mode)."""
         io, eo, p = self.init_cond_order, self.end_cond_order, self.degree_p
         c = plan.consts
         nc = self.num_basis + io + eo
@@ -358,11 +399,12 @@ class BEASTBsplineTokenizer(TokenizerBase):
             st["end_pos"] = end_pos + y0 if io != 0 else end_pos       # returned absolute (:600)
         st["bc"] = torch.stack(parts, dim=-1).contiguous()             # [B, n_joint, io + eo]
         st["bias"] = y0.contiguous() if io != 0 else None
-        self._boundary = st
+        return st
 
-    def _params_dict(self, params):
-        # keys of UniformBSpline.learn_mp_params_from_trajs (mp/uni_bspline.py:597-602)
-        st = self._boundary if self._has_conditions else None
+    def _params_dict(self, params, st=None):
+        # keys of UniformBSpline.learn_mp_params_from_trajs (mp/uni_bspline.py:597-602); `st` overrides the kept state
+        if st is None:
+            st = self._boundary if self._has_conditions else None
         if st is None:
             return {"params": params, "init_pos": None, "init_vel": None, "end_pos": None, "end_vel": None}
         return {"params": params, "init_pos": st["init_pos"], "init_vel": st["init_vel"],
@@ -674,13 +716,36 @@ class BEASTBsplineTokenizer(TokenizerBase):
                                                     _lib.stream_ptr(dev)), "beast_quantize_f32")
         return tokens
 
-    @torch.no_grad()
     def encode_continuous(self, trajs, update_bounds=False):
-        """Normalised [-1, 1] coefficients in '(t d)' order (reference :430-450)."""
-        _, params = self._fit(trajs, want_tokens=False)
-        if update_bounds:
-            self.update_weights_bounds_per_batch(params)
-        return self._normalize(params), self._params_dict(params)
+        """Normalised [-1, 1] coefficients in '(t d)' order (reference :430-450).
+
+        Differentiable with respect to `trajs` when `trajs` requires grad under grad mode: the backward of `normalised`
+        and `params_dict['params']` is beast_fit_backward_f32 (the adjoint of the fit; the normaliser's clamp passes
+        the gradient where w_min <= params <= w_max, inclusive), and the condition-order entries of `params_dict` are
+        torch ops on the boundary samples.  w_min / w_max as the call normalised with (after the expansion of
+        update_bounds=True), the times and the tokenizer state are constants; the boundary state the tokenizer keeps
+        for later reconstructs is detached.  Otherwise the call runs under no_grad, as before."""
+        if not (torch.is_grad_enabled() and isinstance(trajs, torch.Tensor) and trajs.requires_grad):
+            with torch.no_grad():
+                _, params = self._fit(trajs, want_tokens=False)
+                if update_bounds:
+                    self.update_weights_bounds_per_batch(params)
+                return self._normalize(params), self._params_dict(params)
+        plan = self._plan()
+        x = self._prep_trajs(trajs, plan.device)          # differentiable: .to() / slicing / .contiguous()
+
+        def fit(x):
+            _, params = self._fit(x, want_tokens=False)
+            if update_bounds:
+                self.update_weights_bounds_per_batch(params)
+            normalised = self._normalize(params)
+            # the bounds this call normalised with: a later update_weights_bounds* changes the buffers in place
+            lo, hi = self._bounds(plan.device)
+            return normalised, params, (lo.clone(), hi.clone())
+
+        normalised, params = _FitFn.apply(fit, plan, x)
+        st = self._boundary_state(x, plan) if self._has_conditions else None
+        return normalised, self._params_dict(params, st)
 
     def _normalize(self, params):
         plan = self._plan()

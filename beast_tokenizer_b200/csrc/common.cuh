@@ -37,7 +37,8 @@ struct Plan {
     // Band tables of the tiled kernels (csrc/spline_tiled.cu), pairs [lo, hi): the non-zero range of every projector
     // row (encode: samples t of basis k) and of every basis row (decode: basis k of sample t); the terms outside are
     // exact zeros, skipping them leaves the fp32 sums unchanged.  Layout: enc_joint[2*nb], enc_grip[2*nb],
-    // dec_joint[2*T], dec_grip[2*T].
+    // dec_joint[2*T], dec_grip[2*T], then the non-zero range over k of every projector column (the fit's adjoint,
+    // csrc/spline_fit_grad.cu): fit_joint[2*T], fit_grip[2*T].
     int* bands_d;
     // Work lists of the tiled kernels, token order (r = k*D + slot ascending), entries k | slot << 16 | gripper << 31:
     // enc_list = token positions whose projector row is not empty (every other coefficient is exactly 0 for every
@@ -48,6 +49,7 @@ struct Plan {
     int* dec_list_d;
     int n_enc, n_dec;
     int enc_band_max, dec_band_max;   // longest projector-row / basis-row band (terms per sum)
+    int fit_band_max;                 // longest projector-column band
     int num_sms;
     int max_smem_optin;
 };

@@ -162,9 +162,10 @@ extern "C" int beast_plan_create(const beast_plan_desc_t* d, beast_plan_t** out)
     e = cudaMemcpy(p->dev_block, host, total * sizeof(float), cudaMemcpyHostToDevice);
     free(host);
     if (e != cudaSuccess) { beast_plan_destroy((beast_plan_t*)p); return (int)e; }
-    {   // band tables: non-zero range of every projector row [k][t] and of every basis row [t][k]
+    {   // band tables: non-zero range of every projector row [k][t], of every basis row [t][k] and of every projector
+        // column
         const int T = p->T, nb = p->nb;
-        const size_t n_band = (size_t)4 * nb + (size_t)4 * T;
+        const size_t n_band = (size_t)4 * nb + (size_t)8 * T;
         int* bands = (int*)calloc(n_band, sizeof(int));
         if (!bands) { beast_plan_destroy((beast_plan_t*)p); return BEAST_E_NOMEM; }
         auto row_band = [](const float* row, int n, int stride, int* lo_hi) {
@@ -181,6 +182,12 @@ extern "C" int beast_plan_create(const beast_plan_desc_t* d, beast_plan_t** out)
         for (int t = 0; t < T; ++t) {
             if (p->nc == nb) row_band(p->phi_joint_h + (size_t)t * nb, nb, 1, bands + 4 * nb + 2 * t);
             if (has_grip) row_band(p->phi_grip_h + (size_t)t * nb, nb, 1, bands + 4 * nb + 2 * T + 2 * t);
+            int* fit = bands + 4 * nb + 4 * T;
+            row_band(p->proj_joint_h + t, nb, T, fit + 2 * t);
+            if (has_grip) row_band(p->proj_grip_h + t, nb, T, fit + 2 * T + 2 * t);
+            for (int s = 0; s < 2; ++s)
+                if (fit[2 * (s * T + t) + 1] - fit[2 * (s * T + t)] > p->fit_band_max)
+                    p->fit_band_max = fit[2 * (s * T + t) + 1] - fit[2 * (s * T + t)];
         }
         e = cudaMalloc((void**)&p->bands_d, n_band * sizeof(int));
         if (e == cudaSuccess) e = cudaMemcpy(p->bands_d, bands, n_band * sizeof(int), cudaMemcpyHostToDevice);

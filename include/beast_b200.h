@@ -228,6 +228,26 @@ int beast_decode_deriv_times_backward_f32(const beast_plan_t* plan, int64_t B, c
                                           const float* grad0, const float* grad1, const float* grad2,
                                           int32_t init_p_used, float* grad_params, float* grad_init_p, void* stream);
 
+/* ---- Adjoint of beast_encode_f32's coefficients (+ beast_normalize_f32) for encode_continuous backward:
+ *   g_w[b, slot, k] = grad_params[b, slot*nb + k]
+ *                   + (w_min[c] <= w <= w_max[c] ? (grad_norm[b, k*D + slot] * 2) / max(w_max[c] - w_min[c], 1e-8) : 0)
+ *   grad_traj[b, t, dof(slot)] = sum_k P_s[k, t] * g_w[b, slot, k]
+ * with c = slot*nb + k, w = params[b, c] the UNclamped forward coefficient, w_min / w_max [D*nb] the bounds the
+ * forward normalised with (inclusive: torch's clamp rule; each operation one fp32 rounding, in the order written) and
+ * P_s the fp32 projector K1 multiplies with (joint: proj_joint_h, which folds in the condition orders; gripper slots:
+ * the degree-0 proj_grip_h).  grad_norm [B, nb*D] '(t d)' and grad_params [B, D*nb] '(d t)' are nullable (NULL =
+ * zero, at least one is set); params, w_min and w_max are required with grad_norm.  grad_traj [B, seq_len, num_dof]
+ * fp32: every element is written (no accumulation, no memset needed).  Deterministic, no atomics: each element is
+ * one fp32 sum over k ascending (fmaf); terms with an exactly-zero projector entry may be skipped, which does not
+ * change the value for finite gradients, so the two kernels agree.  NaN inputs are not treated specially.
+ * Dispatch: a tiled kernel (persistent CTAs over tiles of trajectories, only the coefficients of non-empty projector
+ * rows loaded; the projector in shared memory when its column sums have more than two terms and it fits in 32 KB, else
+ * read through L1) whenever one trajectory's coefficients and the tables fit in shared memory; otherwise, and under
+ * beast_debug_disable_fast, a generic one-thread-per-element kernel. */
+int beast_fit_backward_f32(const beast_plan_t* plan, int64_t B, const float* grad_norm, const float* grad_params,
+                           const float* params, const float* w_min, const float* w_max, float* grad_traj,
+                           void* stream);
+
 /* ---- K2: bounds.
  * Column min/max of x [rows, cols] (update_weights_bounds :377-378; the reduction inside
  * update_weights_bounds_per_batch :382-383).  accumulate != 0 folds into the existing
