@@ -310,16 +310,17 @@ class BEASTBsplineBPETokenizer(BEASTBsplineTokenizer):
         return self._bpe_csr_to_discrete(flat, offsets)
 
     # ------------------------------------------------------------------ BEAST overridden
-    def encode(self, trajs: torch.Tensor, update_bounds: bool = False, *, return_mp_tokens: bool = False) -> tuple:
-        mp_tokens, params = super().encode(trajs, update_bounds=update_bounds, respect_llm_vocab_size=False)
+    def encode(self, trajs: torch.Tensor, update_bounds: bool = False, *, return_mp_tokens: bool = False,
+               times: Optional[torch.Tensor] = None) -> tuple:
+        mp_tokens, params = super().encode(trajs, update_bounds=update_bounds, respect_llm_vocab_size=False, times=times)
         bpe_tokens = self._discrete_to_bpe(mp_tokens)
         if return_mp_tokens:
             return bpe_tokens, params, mp_tokens
         return bpe_tokens, params
 
-    def encode_csr(self, trajs: torch.Tensor, update_bounds: bool = False):
+    def encode_csr(self, trajs: torch.Tensor, update_bounds: bool = False, *, times: Optional[torch.Tensor] = None):
         """Device-resident variant of `encode`: (flat ids int32, offsets int64 [B+1], params_dict)."""
-        mp_tokens, params = super().encode(trajs, update_bounds=update_bounds, respect_llm_vocab_size=False)
+        mp_tokens, params = super().encode(trajs, update_bounds=update_bounds, respect_llm_vocab_size=False, times=times)
         flat, offsets = self._discrete_to_bpe_csr(mp_tokens)
         return flat, offsets, params
 
@@ -327,9 +328,11 @@ class BEASTBsplineBPETokenizer(BEASTBsplineTokenizer):
         discrete = self._bpe_to_discrete(tokens)
         return super().decode(discrete, respect_llm_vocab_size=respect_llm_vocab_size)
 
-    def encode_to_mp_tokens(self, trajs: torch.Tensor, update_bounds: bool = False) -> tuple:
-        """Expose the underlying MP-token encoding without BPE."""
-        return super().encode(trajs, update_bounds=update_bounds, respect_llm_vocab_size=False)
+    def encode_to_mp_tokens(self, trajs: torch.Tensor, update_bounds: bool = False, *,
+                            times: Optional[torch.Tensor] = None) -> tuple:
+        """Expose the underlying MP-token encoding without BPE.  `times` [B, T]: per-row timestamps, as in
+        BEASTBsplineTokenizer.encode."""
+        return super().encode(trajs, update_bounds=update_bounds, respect_llm_vocab_size=False, times=times)
 
     def bpe_to_mp_tokens(self, tokens: Iterable[TokenLike]) -> torch.Tensor:
         return self._bpe_to_discrete(tokens)

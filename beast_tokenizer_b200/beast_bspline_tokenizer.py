@@ -16,6 +16,8 @@ drop a NaN where torch.min / torch.clamp would propagate it.  Entry points:
     reconstruct_traj_continuous(_derivatives)
         backward (autograd)                       -> beast_decode_grid_backward_f32 / beast_decode_deriv_times_backward_f32
     encode_continuous backward (autograd)         -> beast_fit_backward_f32
+    the fits above with times=[B, T]              -> beast_fit_times_f32 (+ quantize / normalize / minmax);
+                                                     backward beast_fit_times_backward_f32
     update_weights_bounds(_per_batch)             -> beast_minmax_f32 + beast_bounds_expand_f32
     fit_parameters                                -> beast_encode_f32 + beast_colselect_f32
 
@@ -211,6 +213,48 @@ class _FitFn(torch.autograd.Function):
         return None, None, grad_traj
 
 
+class _FitTimesFn(torch.autograd.Function):
+    """encode_continuous(times=[B, T])'s fit and normalisation as an autograd node: forward = `fit(x, bc, bias)` (the
+    beast_fit_times_f32 launch, the optional bounds expansion and beast_normalize_f32) -> (normalised, params, (w_min,
+    w_max) snapshot), backward = one beast_fit_times_backward_f32 launch -> gradients of x, of the pinned points bc and
+    of bias (both torch ops on x's boundary samples, so their gradients chain back to x).  times and the bounds are
+    constants; an output the loss does not use arrives as None and is passed to the kernel as NULL."""
+
+    @staticmethod
+    def forward(ctx, fit, plan, times, x, bc, bias):
+        ctx.set_materialize_grads(False)
+        normalised, params, bounds = fit(x, bc, bias)
+        ctx.plan, ctx.times, ctx.bounds = plan, times, bounds
+        ctx.has_bc, ctx.has_bias = bc is not None, bias is not None
+        ctx.save_for_backward(params)
+        return normalised, params
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_norm, grad_params):
+        if grad_norm is None and grad_params is None:
+            return None, None, None, None, None, None
+        plan, times = ctx.plan, ctx.times
+        (params,), (lo, hi) = ctx.saved_tensors, ctx.bounds
+        dev = plan.device
+        c = plan.consts
+        grad_norm, grad_params = (None if g is None else g.to(dev, torch.float32).contiguous()
+                                  for g in (grad_norm, grad_params))
+        B, T = times.shape
+        n_joint = len(c.joint_indices)
+        nbc = c.init_order + c.end_order
+        grad_traj = torch.empty((B, T, c.num_dof), device=dev, dtype=torch.float32)
+        grad_bc = torch.empty((B, n_joint, nbc), device=dev, dtype=torch.float32) if ctx.has_bc else None
+        grad_bias = torch.empty((B, n_joint), device=dev, dtype=torch.float32) if ctx.has_bias else None
+        if B > 0:                       # empty tensors carry no data pointer
+            with torch.cuda.device(dev):
+                _lib.check(plan._lib.beast_fit_times_backward_f32(
+                    plan.handle, B, T, _lib.ptr(times), _lib.ptr(grad_norm), _lib.ptr(grad_params), _lib.ptr(params),
+                    _lib.ptr(lo), _lib.ptr(hi), _lib.ptr(grad_traj), _lib.ptr(grad_bc), _lib.ptr(grad_bias),
+                    _lib.stream_ptr(dev)), "beast_fit_times_backward_f32")
+        return None, None, None, grad_traj, grad_bc, grad_bias
+
+
 class BEASTBsplineTokenizer(TokenizerBase):
 
     def __init__(self, num_dof=1, num_basis=10, duration=2 * torch.pi, seq_len=50, vocab_size=256,
@@ -327,13 +371,16 @@ class BEASTBsplineTokenizer(TokenizerBase):
     def _bounds(self, dev):
         return (self.w_min.to(dev, torch.float32).contiguous(), self.w_max.to(dev, torch.float32).contiguous())
 
-    def _prep_trajs(self, trajs, dev):
+    def _prep_trajs(self, trajs, dev, n_times=None):
         # pinned host batches are uploaded asynchronously on the current stream (stream-ordered before
         # the kernel), so callers can overlap the copy of one chunk with the compute of another
         trajs = trajs.to(dev, dtype=torch.float32, non_blocking=bool(trajs.device.type == "cpu" and trajs.is_pinned()))
         if trajs.dim() != 3:
             raise AssertionError(f"expected trajectories [batch, time, dof], got {tuple(trajs.shape)}")
-        if trajs.shape[1] != self.times.numel():
+        if n_times is not None:                    # per-row times [B, n_times]
+            if trajs.shape[1] != n_times:
+                raise AssertionError(f"trajectory has {trajs.shape[1]} samples, times has {n_times}")
+        elif trajs.shape[1] != self.times.numel():
             raise AssertionError(f"trajectory has {trajs.shape[1]} samples, tokenizer times has {self.times.numel()}")
         if trajs.shape[2] < self.num_dof:
             raise IndexError(f"trajectory has {trajs.shape[2]} DoF, tokenizer expects {self.num_dof}")
@@ -341,8 +388,11 @@ class BEASTBsplineTokenizer(TokenizerBase):
             trajs = trajs[..., :self.num_dof]
         return trajs.contiguous()
 
-    def _fit(self, trajs, want_tokens, offset=0, bounds=None):
-        """One K1 launch: (tokens | None, unclamped params)."""
+    def _fit(self, trajs, want_tokens, offset=0, bounds=None, times=None):
+        """One K1 launch: (tokens | None, unclamped params).  With per-row times [B, T]: beast_fit_times_f32, then
+        beast_quantize_f32 for the tokens."""
+        if times is not None:
+            return self._fit_times(trajs, times, want_tokens, offset, bounds)
         plan = self._plan()
         dev = plan.device
         x = self._prep_trajs(trajs, dev)
@@ -358,6 +408,40 @@ class BEASTBsplineTokenizer(TokenizerBase):
         self._remember_boundary(x, plan)
         return tokens, params
 
+    def _prep_times(self, trajs, times, dev):
+        """(x [B, T, num_dof], times [B, T]) on `dev` for a fit on per-row times: T may differ from seq_len but is the
+        same for every row; T >= 2 with condition orders (the boundary state reads y[1] and y[-2])."""
+        t = self._check_times(times, dev, trajs.shape[0] if trajs.dim() >= 1 else -1)
+        x = self._prep_trajs(trajs, dev, t.shape[1])
+        if t.shape[1] < 1:
+            raise AssertionError("times must hold at least one sample per row")
+        if self._has_conditions and t.shape[1] < 2:
+            raise AssertionError("init_cond_order / end_cond_order != 0: a fit needs at least 2 samples per row")
+        return x, t
+
+    def _fit_times_launch(self, plan, x, t, bc, bias):
+        """One beast_fit_times_f32 launch: unclamped params [B, D*nb]."""
+        dev = plan.device
+        B, T = t.shape
+        params = torch.empty((B, self.num_dof * self.num_basis), device=dev, dtype=torch.float32)
+        if B > 0:                       # empty tensors carry no data pointer
+            with torch.cuda.device(dev):
+                _lib.check(plan._lib.beast_fit_times_f32(plan.handle, _lib.ptr(x), B, T, _lib.ptr(t), _lib.ptr(bc),
+                                                         _lib.ptr(bias), _lib.ptr(params), _lib.stream_ptr(dev)),
+                           "beast_fit_times_f32")
+        return params
+
+    def _fit_times(self, trajs, times, want_tokens, offset=0, bounds=None):
+        plan = self._plan()
+        dev = plan.device
+        x, t = self._prep_times(trajs, times, dev)
+        st = self._boundary_state(x, plan, t) if self._has_conditions else None
+        if st is not None:
+            self._boundary = st
+        params = self._fit_times_launch(plan, x, t, *((st["bc"], st["bias"]) if st is not None else (None, None)))
+        tokens = self._quantize(params, offset, bounds) if want_tokens else None
+        return tokens, params
+
     @property
     def _has_conditions(self) -> bool:
         return (self.init_cond_order != 0 or self.end_cond_order != 0) and self.joint_dof > 0
@@ -370,13 +454,17 @@ class BEASTBsplineTokenizer(TokenizerBase):
             return
         self._boundary = self._boundary_state(x, plan)
 
-    def _boundary_state(self, x, plan):
-        """The boundary state of `x` (torch ops: attached to the graph of `x` under grad mode)."""
+    def _boundary_state(self, x, plan, times=None):
+        """The boundary state of `x` (torch ops: attached to the graph of `x` under grad mode).  `times` [B, T]: each
+        row's own step dt_b = times[b, 1] - times[b, 0]; None: the tokenizer's times."""
         io, eo, p = self.init_cond_order, self.end_cond_order, self.degree_p
         c = plan.consts
         nc = self.num_basis + io + eo
-        t = c.times
-        inv_dt = float(torch.tensor(1.0) / (t[1] - t[0]))
+        if times is None:
+            t = c.times
+            inv_dt = float(torch.tensor(1.0) / (t[1] - t[0]))
+        else:
+            inv_dt = (1.0 / (times[:, 1] - times[:, 0])).unsqueeze(1)
         tau = c.tau
         ji = torch.as_tensor(self.joint_indices, device=x.device)
         y0, y1, ym2, ym1 = (x[:, i, :].index_select(1, ji) for i in (0, 1, -2, -1))
@@ -623,19 +711,23 @@ class BEASTBsplineTokenizer(TokenizerBase):
 
     # ------------------------------------------------------------------ utils
     @torch.no_grad()
-    def compute_weights(self, demos):
-        """Unclamped spline coefficients [B, D*nb] '(d t)', joints first (reference :344-360)."""
-        return self._fit(demos, want_tokens=False)[1]
+    def compute_weights(self, demos, *, times=None):
+        """Unclamped spline coefficients [B, D*nb] '(d t)', joints first (reference :344-360).  `times` [B, T]: fit
+        each row on its own timestamps (T may differ from seq_len; see encode)."""
+        return self._fit(demos, want_tokens=False, times=times)[1]
 
     @torch.no_grad()
-    def update_weights_bounds(self, demos, process_group=None):
+    def update_weights_bounds(self, demos, process_group=None, *, times=None):
         """Global per-column min / max of the coefficients (reference :362-378): one fused launch,
         the coefficients are reduced in registers and never written.  Sharded (set_process_group, or
-        process_group= here; every rank passes its shard): one MIN and one MAX all-reduce of the D*nb vectors."""
+        process_group= here; every rank passes its shard): one MIN and one MAX all-reduce of the D*nb vectors.
+        `times` [B, T]: the coefficients of the per-row fit (see encode), then beast_minmax_f32."""
         plan = self._plan()
         dev = plan.device
-        x = self._prep_trajs(demos, dev)
         n = self.num_dof * self.num_basis
+        if times is not None:
+            return self._update_weights_bounds_times(plan, demos, times, n, process_group)
+        x = self._prep_trajs(demos, dev)
         # one launch, results written straight into the w_min / w_max buffers when they live on this device
         direct = (self.w_min.device == dev and self.w_max.device == dev and self.w_min.dtype == torch.float32
                   and self.w_max.dtype == torch.float32 and self.w_min.is_contiguous() and self.w_max.is_contiguous())
@@ -647,6 +739,21 @@ class BEASTBsplineTokenizer(TokenizerBase):
                                                          _lib.ptr(ws), ws.numel() * 4, _lib.stream_ptr(dev)),
                        "beast_fit_minmax_ws_f32")
         self._remember_boundary(x, plan)
+        _dist.allreduce_minmax(lo, hi, self._group(process_group), implicit=False)
+        if not direct:
+            self.w_min.copy_(lo.to(self.w_min.device))
+            self.w_max.copy_(hi.to(self.w_max.device))
+
+    def _update_weights_bounds_times(self, plan, demos, times, n, process_group):
+        dev = plan.device
+        _, params = self._fit_times(demos, times, want_tokens=False)
+        direct = (self.w_min.device == dev and self.w_max.device == dev and self.w_min.dtype == torch.float32
+                  and self.w_max.dtype == torch.float32 and self.w_min.is_contiguous() and self.w_max.is_contiguous())
+        lo = self.w_min if direct else torch.empty(n, device=dev, dtype=torch.float32)
+        hi = self.w_max if direct else torch.empty(n, device=dev, dtype=torch.float32)
+        with torch.cuda.device(dev):
+            _lib.check(plan._lib.beast_minmax_f32(_lib.ptr(params), params.shape[0], n, _lib.ptr(lo), _lib.ptr(hi), 0,
+                                                  _lib.stream_ptr(dev)), "beast_minmax_f32")
         _dist.allreduce_minmax(lo, hi, self._group(process_group), implicit=False)
         if not direct:
             self.w_min.copy_(lo.to(self.w_min.device))
@@ -690,25 +797,32 @@ class BEASTBsplineTokenizer(TokenizerBase):
 
     # ------------------------------------------------------------------ encoding
     @torch.no_grad()
-    def encode(self, trajs, update_bounds=False, *, respect_llm_vocab_size=True):
-        """trajs [B, T, D] -> (tokens int64 [B, nb*D] '(t d)', params_dict) — reference :399-428."""
+    def encode(self, trajs, update_bounds=False, *, respect_llm_vocab_size=True, times=None):
+        """trajs [B, T, D] -> (tokens int64 [B, nb*D] '(t d)', params_dict) — reference :399-428.
+
+        `times` [B, T] (any device, converted to fp32): fit every row on its own timestamps, the reference's
+        learn_mp_params_from_trajs(times=[B, T]) — one ridge system per row on the basis at times[b] (phase clip(t /
+        tau, 0, 1), as reconstruct_traj(times=...) evaluates it).  T may differ from seq_len (same for every row; >= 2
+        with condition orders, whose boundary velocity uses each row's dt_b = times[b, 1] - times[b, 0]); times need
+        not be sorted and are clamped to [0, duration].  NaN and dt_b = 0 are not treated specially.  A basis function
+        with no sample in its support gets coefficient 0.  None: the tokenizer's own times (the shared projector)."""
         offset = 0
         if respect_llm_vocab_size and self.llm_vocab_size is not None:
             offset = self._llm_vocab_offset()
         if not update_bounds:
-            tokens, params = self._fit(trajs, want_tokens=True, offset=offset)
+            tokens, params = self._fit(trajs, want_tokens=True, offset=offset, times=times)
             return tokens, self._params_dict(params)
         # bounds move before quantisation: fit, expand, then the exact quantiser on the coefficients
-        _, params = self._fit(trajs, want_tokens=False)
+        _, params = self._fit(trajs, want_tokens=False, times=times)
         self.update_weights_bounds_per_batch(params)
         tokens = self._quantize(params, offset)
         return tokens, self._params_dict(params)
 
-    def _quantize(self, params, offset=0):
+    def _quantize(self, params, offset=0, bounds=None):
         plan = self._plan()
         dev = plan.device
         params = params.to(dev, torch.float32).contiguous()
-        lo, hi = self._bounds(dev)
+        lo, hi = self._bounds(dev) if bounds is None else bounds
         tokens = torch.empty(params.shape, device=dev, dtype=torch.int64)
         with torch.cuda.device(dev):
             _lib.check(plan._lib.beast_quantize_f32(plan.handle, _lib.ptr(params), params.shape[0], _lib.ptr(lo),
@@ -716,7 +830,7 @@ class BEASTBsplineTokenizer(TokenizerBase):
                                                     _lib.stream_ptr(dev)), "beast_quantize_f32")
         return tokens
 
-    def encode_continuous(self, trajs, update_bounds=False):
+    def encode_continuous(self, trajs, update_bounds=False, *, times=None):
         """Normalised [-1, 1] coefficients in '(t d)' order (reference :430-450).
 
         Differentiable with respect to `trajs` when `trajs` requires grad under grad mode: the backward of `normalised`
@@ -724,13 +838,18 @@ class BEASTBsplineTokenizer(TokenizerBase):
         the gradient where w_min <= params <= w_max, inclusive), and the condition-order entries of `params_dict` are
         torch ops on the boundary samples.  w_min / w_max as the call normalised with (after the expansion of
         update_bounds=True), the times and the tokenizer state are constants; the boundary state the tokenizer keeps
-        for later reconstructs is detached.  Otherwise the call runs under no_grad, as before."""
+        for later reconstructs is detached.  Otherwise the call runs under no_grad, as before.
+
+        `times` [B, T]: the per-row fit of encode(times=...); its backward is beast_fit_times_backward_f32, with the
+        gradients of the pinned boundary points and of the bias chained back to the trajectories."""
         if not (torch.is_grad_enabled() and isinstance(trajs, torch.Tensor) and trajs.requires_grad):
             with torch.no_grad():
-                _, params = self._fit(trajs, want_tokens=False)
+                _, params = self._fit(trajs, want_tokens=False, times=times)
                 if update_bounds:
                     self.update_weights_bounds_per_batch(params)
                 return self._normalize(params), self._params_dict(params)
+        if times is not None:
+            return self._encode_continuous_times(trajs, times, update_bounds)
         plan = self._plan()
         x = self._prep_trajs(trajs, plan.device)          # differentiable: .to() / slicing / .contiguous()
 
@@ -745,6 +864,26 @@ class BEASTBsplineTokenizer(TokenizerBase):
 
         normalised, params = _FitFn.apply(fit, plan, x)
         st = self._boundary_state(x, plan) if self._has_conditions else None
+        return normalised, self._params_dict(params, st)
+
+    def _encode_continuous_times(self, trajs, times, update_bounds):
+        plan = self._plan()
+        dev = plan.device
+        x, t = self._prep_times(trajs, times, dev)         # differentiable: .to() / slicing / .contiguous()
+        st = self._boundary_state(x, plan, t) if self._has_conditions else None
+        bc, bias = (st["bc"], st["bias"]) if st is not None else (None, None)
+
+        def fit(x, bc, bias):
+            if st is not None:                              # kept for later reconstructs, detached
+                self._boundary = {k: None if v is None else v.detach() for k, v in st.items()}
+            params = self._fit_times_launch(plan, x, t, bc, bias)
+            if update_bounds:
+                self.update_weights_bounds_per_batch(params)
+            normalised = self._normalize(params)
+            lo, hi = self._bounds(dev)
+            return normalised, params, (lo.clone(), hi.clone())
+
+        normalised, params = _FitTimesFn.apply(fit, plan, t, x, bc, bias)
         return normalised, self._params_dict(params, st)
 
     def _normalize(self, params):

@@ -202,6 +202,30 @@ __device__ __forceinline__ float dequantize_fast(long long tok, float w_min, flo
     return clampf(c, w_min, w_max);
 }
 
+// ---------------------------------------------------------------- adjoint of the fit's normalisation
+// g_w of one coefficient from its loaded inputs: torch's rules for utils.normalize_tensor (the clamp passes the gradient
+// where w_min <= w <= w_max inclusively, then * 2 and / scale, each one fp32 rounding), plus the gradient of the raw
+// coefficient.  Shared by the fit adjoints on the tokenizer's own times (spline_fit_grad.cu) and on per-row times
+// (spline_fit_times.cu).
+__device__ __forceinline__ float fit_grad_weight(bool has_n, float gn, float w, float lo, float hi, bool has_p, float gp) {
+    float g = 0.0f;
+    if (has_n) g = (lo <= w && w <= hi) ? __fdiv_rn(__fmul_rn(gn, 2.0f), quant_scale(lo, hi)) : 0.0f;
+    if (has_p) g = has_n ? __fadd_rn(gp, g) : gp;
+    return g;
+}
+// Same, loaded from the callers' layouts: grad_norm [B, nb*D] '(t d)', grad_params / params [B, D*nb] '(d t)', bounds
+// [D*nb]; row0 = b * D * nb.  grad_norm / grad_params NULL = zero; params and the bounds are read with grad_norm only.
+__device__ __forceinline__ float fit_grad_coeff(const float* grad_norm, const float* grad_params, const float* params,
+                                                const float* w_min, const float* w_max, long long row0, int D, int nb,
+                                                int slot, int k) {
+    const bool has_n = grad_norm != nullptr, has_p = grad_params != nullptr;
+    const long long r = row0 + (long long)k * D + slot, c = row0 + (long long)slot * nb + k;
+    const float gn = has_n ? grad_norm[r] : 0.0f, w = has_n ? params[c] : 0.0f;
+    const float lo = has_n ? w_min[slot * nb + k] : 0.0f, hi = has_n ? w_max[slot * nb + k] : 0.0f;
+    const float gp = has_p ? grad_params[c] : 0.0f;
+    return fit_grad_weight(has_n, gn, w, lo, hi, has_p, gp);
+}
+
 // ---------------------------------------------------------------- packed fp32 FMA (Blackwell FFMA2)
 // fma.rn.f32x2: two IEEE fp32 FMAs per instruction (SASS FFMA2, which takes a uniform-register pair
 // and a broadcast scalar directly).  Bit-identical to two fmaf calls; halves the issue slots of the

@@ -32,14 +32,6 @@ constexpr int kFitGradThreads = 512;
 constexpr int kFitGradCtasPerSm = 2;
 constexpr int kFitGradGridPerSm = 4;
 
-// g_w of one coefficient from its loaded inputs (see the top of the file); the operations of both kernels.
-__device__ __forceinline__ float fit_grad_weight(bool has_n, float gn, float w, float lo, float hi, bool has_p, float gp) {
-    float g = 0.0f;
-    if (has_n) g = (lo <= w && w <= hi) ? __fdiv_rn(__fmul_rn(gn, 2.0f), quant_scale(lo, hi)) : 0.0f;
-    if (has_p) g = has_n ? __fadd_rn(gp, g) : gp;
-    return g;
-}
-
 struct FitGradArgs {
     const float* grad_norm;        // [B, nb*D] '(t d)' (nullable)
     const float* grad_params;      // [B, D*nb] '(d t)' (nullable)
@@ -167,7 +159,6 @@ fit_grad_tiled_kernel(const __grid_constant__ FitGradArgs a) {
 __global__ void fit_grad_generic_kernel(const __grid_constant__ FitGradArgs a) {
     const int T = a.T, D = a.D, nb = a.nb;
     const long long row_in = (long long)D * nb, row_out = (long long)T * D, n = a.B * row_out;
-    const bool has_n = a.grad_norm != nullptr, has_p = a.grad_params != nullptr;
     for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < n;
          idx += (long long)gridDim.x * blockDim.x) {
         const long long b = idx / row_out;
@@ -180,11 +171,8 @@ __global__ void fit_grad_generic_kernel(const __grid_constant__ FitGradArgs a) {
         for (int k = 0; k < nb; ++k) {
             const float pv = P[(size_t)k * T + t];
             if (pv == 0.0f) continue;
-            const long long r = b * row_in + k * D + slot, c = b * row_in + slot * nb + k;
-            const float gn = has_n ? a.grad_norm[r] : 0.0f, w = has_n ? a.params[c] : 0.0f;
-            const float lo = has_n ? a.w_min[slot * nb + k] : 0.0f, hi = has_n ? a.w_max[slot * nb + k] : 0.0f;
-            const float gp = has_p ? a.grad_params[c] : 0.0f;
-            acc = fmaf(pv, fit_grad_weight(has_n, gn, w, lo, hi, has_p, gp), acc);
+            acc = fmaf(pv, fit_grad_coeff(a.grad_norm, a.grad_params, a.params, a.w_min, a.w_max, b * row_in, D, nb,
+                                          slot, k), acc);
         }
         a.grad_traj[idx] = acc;
     }

@@ -248,6 +248,27 @@ int beast_fit_backward_f32(const beast_plan_t* plan, int64_t B, const float* gra
                            const float* params, const float* w_min, const float* w_max, float* grad_traj,
                            void* stream);
 
+/* ---- Fit on per-row times (encode / encode_continuous / compute_weights with times [B, T]).
+ * Row b solves its own ridge system on Phi_b = the basis at times[b] (phase clip(t / tau, 0, 1), the rows the per-row
+ * decode evaluates): joint slots w = (Phi_f^T Phi_f + 1e-9 I)^-1 Phi_f^T (y - bias - Phi_pin bc) on the nb free
+ * columns, gripper slots the same on the degree-0 basis.  traj [B, T, num_dof] and times [B, T] fp32, T >= 1 (>= 2
+ * when the plan pins control points) and independent of seq_len; times need not be sorted and are clamped to
+ * [0, tau] like the decode's; NaN and repeated first times (dt = 0 upstream) are not treated specially.  bc
+ * [B, n_joint, init_cond_order + end_cond_order] (required when the plan pins points, else ignored) and bias
+ * [B, n_joint] (nullable) as beast_reconstruct_bc_f32 takes them.  params_out [B, D*nb] '(d t)' unclamped.  Gram
+ * matrix, right-hand sides, band Cholesky and solves in fp64, one fp32 rounding per output; a coefficient whose basis
+ * function holds no sample is exactly 0.  Each element depends only on its row (no atomics, fixed summation order).
+ * BEAST_E_UNSUPPORTED when num_ctrlp + degree_p + 1 > 320 (as the per-row decode).  Tokens: beast_quantize_f32. */
+int beast_fit_times_f32(const beast_plan_t* plan, const float* traj, int64_t B, int32_t T, const float* times,
+                        const float* bc, const float* bias, float* params_out, void* stream);
+/* Its adjoint: g_w exactly as beast_fit_backward_f32 forms it (same arguments and nullability), v = G_b^-1 g_w and
+ * u = Phi_f v per row; grad_traj [B, T, num_dof] = u, grad_bc = -Phi_pin^T u (required when the plan pins points) and
+ * grad_bias [B, n_joint] = -sum_t u (nullable).  Every element of the given outputs is written; no atomics. */
+int beast_fit_times_backward_f32(const beast_plan_t* plan, int64_t B, int32_t T, const float* times,
+                                 const float* grad_norm, const float* grad_params, const float* params,
+                                 const float* w_min, const float* w_max, float* grad_traj, float* grad_bc,
+                                 float* grad_bias, void* stream);
+
 /* ---- K2: bounds.
  * Column min/max of x [rows, cols] (update_weights_bounds :377-378; the reduction inside
  * update_weights_bounds_per_batch :382-383).  accumulate != 0 folds into the existing
