@@ -15,23 +15,30 @@ __global__ void minmax_init_kernel(float* mn, float* mx, int n) {
     if (i < n) { mn[i] = __int_as_float(0x7f800000); mx[i] = __int_as_float(0xff800000); }
 }
 
-// Every thread owns one column group (VEC adjacent columns) for its whole life: the grid-wide
-// thread count is a multiple of the number of groups, so a flat grid-stride walk over the
-// row-major matrix never changes a thread's columns and consecutive threads read consecutive
-// 16-byte words.  Partials meet in shared memory; one warp per column finishes with shuffles.
+// The columns are cut into chunks of `chunk_groups` column groups (VEC adjacent columns each; at most
+// 1024 groups, so a chunk fits one block); the last chunk may be shorter.  Block b works on chunk
+// b / row_blocks and on rows (b % row_blocks) * rows_per_block + ..., stepping by row_blocks *
+// rows_per_block.  Every thread owns one column group of its chunk for its whole life, and
+// consecutive threads read consecutive 16-byte words.  Partials meet in shared memory; one warp per
+// column finishes with shuffles.
 template <int VEC>
 __global__ void __launch_bounds__(1024)
-minmax_kernel(const float* __restrict__ x, long long rows, int cols, int groups, int rows_per_block,
-              float* __restrict__ mn_out, float* __restrict__ mx_out) {
-    extern __shared__ float sm[];                 // [2][rows_per_block][cols]
+minmax_kernel(const float* __restrict__ x, long long rows, int cols, int chunk_groups, int rows_per_block,
+              int row_blocks, float* __restrict__ mn_out, float* __restrict__ mx_out) {
+    extern __shared__ float sm[];                 // [2][rows_per_block][chunk_groups * VEC]
+    const int chunk = blockIdx.x / row_blocks, rb = blockIdx.x - chunk * row_blocks;
+    const int ccols = chunk_groups * VEC;         // columns of a full chunk
+    const int c0 = chunk * ccols;
+    const int ncols = min(ccols, cols - c0);      // columns of this chunk (VEC divides it)
     const int tid = threadIdx.x;
-    const int g = tid % groups, rl = tid / groups;
+    const int g = tid % chunk_groups, rl = tid / chunk_groups;
     float mn[VEC], mx[VEC];
 #pragma unroll
     for (int v = 0; v < VEC; ++v) { mn[v] = __int_as_float(0x7f800000); mx[v] = __int_as_float(0xff800000); }
-    const long long row_stride = (long long)gridDim.x * rows_per_block;
-    for (long long r = (long long)blockIdx.x * rows_per_block + rl; r < rows; r += row_stride) {
-        const float* p = x + r * cols + g * VEC;
+    const long long row_stride = (long long)row_blocks * rows_per_block;
+    const long long row_end = g * VEC < ncols ? rows : 0;      // a group past the end of a short last chunk reads nothing
+    for (long long r = (long long)rb * rows_per_block + rl; r < row_end; r += row_stride) {
+        const float* p = x + r * cols + c0 + g * VEC;
         if (VEC == 4) {
             const float4 q = __ldg((const float4*)p);
             mn[0] = fminf(mn[0], q.x); mx[0] = fmaxf(mx[0], q.x);
@@ -44,23 +51,26 @@ minmax_kernel(const float* __restrict__ x, long long rows, int cols, int groups,
         }
     }
     float* smn = sm;
-    float* smx = sm + (size_t)rows_per_block * cols;
+    float* smx = sm + (size_t)rows_per_block * ccols;
 #pragma unroll
     for (int v = 0; v < VEC; ++v) {
-        smn[rl * cols + g * VEC + v] = mn[v];
-        smx[rl * cols + g * VEC + v] = mx[v];
+        smn[rl * ccols + g * VEC + v] = mn[v];
+        smx[rl * ccols + g * VEC + v] = mx[v];
     }
     __syncthreads();
+    // full warps only (the block need not be a multiple of 32, and the shuffles name all 32 lanes); a block has
+    // at least 257 threads, so 8 full warps or more
     const int warp = tid >> 5, lane = tid & 31, nwarps = blockDim.x >> 5;
-    for (int c = warp; c < cols; c += nwarps) {
+    if (warp >= nwarps) return;
+    for (int c = warp; c < ncols; c += nwarps) {
         float a = __int_as_float(0x7f800000), b = __int_as_float(0xff800000);
         for (int r = lane; r < rows_per_block; r += 32) {
-            a = fminf(a, smn[r * cols + c]);
-            b = fmaxf(b, smx[r * cols + c]);
+            a = fminf(a, smn[r * ccols + c]);
+            b = fmaxf(b, smx[r * ccols + c]);
         }
         a = warp_min(a);
         b = warp_max(b);
-        if (lane == 0) { atomic_min_f32(mn_out + c, a); atomic_max_f32(mx_out + c, b); }
+        if (lane == 0) { atomic_min_f32(mn_out + c0 + c, a); atomic_max_f32(mx_out + c0 + c, b); }
     }
 }
 
@@ -166,19 +176,26 @@ extern "C" int beast_minmax_f32(const float* x, int64_t rows, int32_t cols, floa
     const bool vec4 = (cols % 4 == 0) && (((uintptr_t)x & 15u) == 0);
     const int vec = vec4 ? 4 : 1;
     const int groups = cols / vec;
-    if (groups > 1024) return BEAST_E_UNSUPPORTED;
-    int rpb = 512 / groups;
+    // up to 1024 groups: one chunk, the whole row in one block; wider: the fewest chunks of <= 1024 groups, as even
+    // as possible, sharing the same 4 * SMs block budget
+    const int chunks = (groups + 1023) / 1024;
+    const int chunk_groups = (groups + chunks - 1) / chunks;
+    int rpb = 512 / chunk_groups;
     if (rpb < 1) rpb = 1;
-    const int block = groups * rpb;
-    const size_t smem = 2 * (size_t)rpb * cols * sizeof(float);
-    if (smem > 48 * 1024) return BEAST_E_UNSUPPORTED;
+    const int block = chunk_groups * rpb;
+    const size_t smem = 2 * (size_t)rpb * chunk_groups * vec * sizeof(float);     // <= 32 KB
     int dev = 0, sms = 148;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    long long grid = (rows + rpb - 1) / rpb;
-    if (grid > (long long)sms * 4) grid = (long long)sms * 4;
-    if (vec4) minmax_kernel<4><<<(int)grid, block, smem, st>>>(x, rows, cols, groups, rpb, min_out, max_out);
-    else minmax_kernel<1><<<(int)grid, block, smem, st>>>(x, rows, cols, groups, rpb, min_out, max_out);
+    long long row_blocks = (rows + rpb - 1) / rpb;
+    long long cap = (long long)sms * 4 / chunks;
+    if (cap < 1) cap = 1;
+    if (row_blocks > cap) row_blocks = cap;
+    const long long grid = row_blocks * chunks;
+    if (vec4) minmax_kernel<4><<<(unsigned)grid, block, smem, st>>>(x, rows, cols, chunk_groups, rpb, (int)row_blocks,
+                                                                   min_out, max_out);
+    else minmax_kernel<1><<<(unsigned)grid, block, smem, st>>>(x, rows, cols, chunk_groups, rpb, (int)row_blocks,
+                                                              min_out, max_out);
     count_launch();
     BEAST_CHECK_LAUNCH();
     return BEAST_OK;

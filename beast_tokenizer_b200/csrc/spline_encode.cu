@@ -56,7 +56,8 @@ struct EncArgs {
     const float* w_max;
     float* bmin;           // optional [D*NB]: column min / max of the coefficients
     float* bmax;
-    float* mm_ws;          // workspace of the single-launch reduction: [grid][2][D*NB] per-CTA partials + ticket; NULL = atomics
+    float* mm_ws;          // workspace of the single-launch reduction: ticket (4 floats), then [grid][2][D*NB] per-CTA
+                           // partials; NULL = atomics
     int mm_accumulate;     // fold the existing contents of bmin / bmax into the result
     int wait_first;        // 0 = may stream while the previous launch drains (disjoint buffers, common.cuh)
     long long offset;
@@ -247,8 +248,11 @@ encode_fast_kernel(const __grid_constant__ EncTables<T, NB> tab, const __grid_co
             // single-launch reduction: every CTA stores its partials, the LAST one to arrive (ticket) combines
             // them and writes the result with plain stores — no initialisation pass, no float atomics, and the
             // caller can pass the tokenizer's own w_min / w_max as the destination
-            float* part = a.mm_ws + (size_t)blockIdx.x * 2 * n_col;
-            unsigned int* ticket = (unsigned int*)(a.mm_ws + (size_t)gridDim.x * 2 * n_col);
+            // the ticket sits at a fixed place ahead of the partials: launches of different grid sizes share one
+            // workspace, and a larger grid's partials must never land where a smaller grid looks for its ticket
+            unsigned int* ticket = (unsigned int*)a.mm_ws;
+            float* parts = a.mm_ws + 4;
+            float* part = parts + (size_t)blockIdx.x * 2 * n_col;
             for (int c = tid; c < n_col; c += kComputeThreads) { part[c] = s_mn[c]; part[n_col + c] = s_mx[c]; }
             __threadfence();
             asm volatile("bar.sync %0, %1;" ::"r"(kEncGroups + 1), "r"(kComputeThreads) : "memory");
@@ -261,7 +265,7 @@ encode_fast_kernel(const __grid_constant__ EncTables<T, NB> tab, const __grid_co
                     float mn = a.mm_accumulate ? a.bmin[c] : __int_as_float(0x7f800000);
                     float mx = a.mm_accumulate ? a.bmax[c] : __int_as_float(0xff800000);
                     for (unsigned int bk = 0; bk < gridDim.x; ++bk) {
-                        const float* q = a.mm_ws + (size_t)bk * 2 * n_col;
+                        const float* q = parts + (size_t)bk * 2 * n_col;
                         mn = fminf(mn, __ldcg(q + c));
                         mx = fmaxf(mx, __ldcg(q + n_col + c));
                     }

@@ -272,7 +272,10 @@ int beast_fit_times_backward_f32(const beast_plan_t* plan, int64_t B, int32_t T,
 /* ---- K2: bounds.
  * Column min/max of x [rows, cols] (update_weights_bounds :377-378; the reduction inside
  * update_weights_bounds_per_batch :382-383).  accumulate != 0 folds into the existing
- * contents of min_out / max_out (used when the rows arrive in several batches or shards). */
+ * contents of min_out / max_out (used when the rows arrive in several batches or shards);
+ * accumulate == 0 with rows == 0 leaves min_out = +inf, max_out = -inf.  Any column count
+ * cols >= 1 and any 4-byte-aligned x are accepted.  The sign of a zero result is not kept
+ * (-0 comes back as +0). */
 int beast_minmax_f32(const float* x, int64_t rows, int32_t cols,
                      float* min_out, float* max_out, int32_t accumulate, void* stream);
 
@@ -281,7 +284,8 @@ int beast_minmax_f32(const float* x, int64_t rows, int32_t cols,
 int beast_fit_minmax_f32(const beast_plan_t* plan, const float* traj, int64_t B, float* min_out,
                          float* max_out, int32_t accumulate, void* stream);
 /* Same in ONE launch: with a zero-initialised workspace of beast_fit_minmax_workspace_bytes(plan) bytes (per-CTA
- * partials + a ticket that the kernel resets itself; one workspace per concurrent stream) the last CTA to finish
+ * partials + a ticket that the kernel resets itself; one workspace per concurrent stream, shared by calls of any batch
+ * size) the last CTA to finish
  * combines the partials and writes min_out / max_out with plain stores — no initialisation pass, no float atomics; the
  * destination may be the tokenizer's own w_min / w_max buffers.  workspace == NULL behaves as beast_fit_minmax_f32. */
 int64_t beast_fit_minmax_workspace_bytes(const beast_plan_t* plan);
