@@ -79,9 +79,12 @@ def token_char_entry(tb: bytes):
     the sequential UTF-8 state machine of A.6 does with this token's bytes, precomputed.  Returns 4 x uint32:
     x, y, z = six 16-bit slots with the token's characters in order (the last one = the partial accumulator, already
     shifted by the missing continuation bytes, when the token ends inside a character); w = characters started | bytes still needed << 3 | leading continuation bytes << 5
-    | slow << 7 | payload of the leading continuation bytes << 8.  slow = the token cannot be described this way (more
-    than 6 characters or 3 leading continuation bytes, an invalid or 4-byte lead, a stray continuation byte): sequences
-    holding it decode on the byte-level path, which also reports the reference's errors."""
+    | slow << 7 | payload of the leading continuation bytes << 8 | ends in a bare E0 lead << 26 | ends in a bare ED
+    lead << 27.  slow = the token cannot be described this way (more than 6 characters or 3 leading continuation bytes,
+    an invalid or 4-byte lead, a stray continuation byte, an overlong or surrogate form): sequences holding it decode on
+    the byte-level path, which also reports the reference's errors.  So do sequences holding a token that ends in a bare
+    E0 / ED lead (bits 26 / 27): strict UTF-8 restricts the next byte (A0..BF / 80..9F), which lies in the next token.
+    The entry still describes such a token; only the kernel's choice of path reads the two bits."""
     SLOW = (0, 0, 0, 0x80)
     i, lead_cont, lead_bits = 0, 0, 0
     while i < len(tb) and (tb[i] & 0xC0) == 0x80:
@@ -90,21 +93,24 @@ def token_char_entry(tb: bytes):
         i += 1
     if lead_cont > 3:
         return SLOW
-    cps, pending, acc = [], 0, 0
+    cps, pending, acc, lo, hi, last = [], 0, 0, 0x80, 0xBF, 0
     for b in tb[i:]:
+        last = b
         if pending:
-            if (b & 0xC0) != 0x80:
+            if not lo <= b <= hi:
                 return SLOW
+            lo, hi = 0x80, 0xBF
             acc = (acc << 6) | (b & 0x3F)
             pending -= 1
             if pending == 0:
                 cps.append(acc)
         elif b < 0x80:
             cps.append(b)
-        elif (b & 0xE0) == 0xC0:
+        elif 0xC2 <= b < 0xE0:     # C0 / C1 only start overlong forms
             acc, pending = b & 0x1F, 1
-        elif (b & 0xF0) == 0xE0:
+        elif 0xE0 <= b < 0xF0:
             acc, pending = b & 0x0F, 2
+            lo, hi = (0xA0 if b == 0xE0 else 0x80), (0x9F if b == 0xED else 0xBF)
         else:                      # 4-byte leads decode above U+FFFF (never a shifted bin), 0xF8.. and stray
             return SLOW            # continuation bytes are invalid: the byte-level path reports them
     if pending:
@@ -112,7 +118,8 @@ def token_char_entry(tb: bytes):
     if len(cps) > 6 or any(c > 0xFFFF for c in cps):
         return SLOW
     slots = cps + [0] * (6 - len(cps))
-    meta = len(cps) | (pending << 3) | (lead_cont << 5) | (lead_bits << 8)
+    lead3 = (1 if last == 0xE0 else 2 if last == 0xED else 0) if pending == 2 else 0
+    meta = len(cps) | (pending << 3) | (lead_cont << 5) | (lead_bits << 8) | (lead3 << 26)
     return (slots[0] | (slots[1] << 16), slots[2] | (slots[3] << 16), slots[4] | (slots[5] << 16), meta)
 
 

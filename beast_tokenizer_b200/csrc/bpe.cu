@@ -1639,6 +1639,16 @@ bpe_compact_kernel(const uint16_t* __restrict__ padded, int stride, const int* _
 // ---------------------------------------------------------------- decode (K5b)
 // ids (CSR) -> token bytes -> UTF-8 -> codepoints + min_token.  status: 1 = id out of range,
 // 2 = invalid UTF-8, 3 = decoded length != L (the reference's ValueError, bpe_tokenizer.py:241-244).
+// UTF-8 is strict (RFC 3629, what Python's bytes.decode("utf-8") accepts): C0, C1 and F5..FF never start a character,
+// and the byte after a lead must lie in [utf8_second_lo, utf8_second_hi] — that rejects overlong forms (E0 80 80 -> 0),
+// surrogates (ED A0 80) and code points above U+10FFFF as soon as their second byte is seen.  Characters above U+FFFF
+// are valid UTF-8 but no shifted bin: status 2 as well.
+__device__ __forceinline__ int utf8_lead_len(int b) {
+    return b < 0x80 ? 1 : (b < 0xC2 ? 0 : (b < 0xE0 ? 2 : (b < 0xF0 ? 3 : (b < 0xF5 ? 4 : 0))));
+}
+__device__ __forceinline__ int utf8_second_lo(int lead) { return lead == 0xE0 ? 0xA0 : (lead == 0xF0 ? 0x90 : 0x80); }
+__device__ __forceinline__ int utf8_second_hi(int lead) { return lead == 0xED ? 0x9F : (lead == 0xF4 ? 0x8F : 0xBF); }
+
 __global__ void __launch_bounds__(kBpeBlock)
 bpe_decode_kernel(const int* __restrict__ flat, const long long* __restrict__ offsets, long long N, int L,
                   long long min_token, const int* __restrict__ tok_off, const uint8_t* __restrict__ tok_bytes,
@@ -1652,7 +1662,7 @@ bpe_decode_kernel(const int* __restrict__ flat, const long long* __restrict__ of
     int status = 0, cnt = 0;
     if (threadIdx.x < rows_per_block && seq < N) {
         uint16_t* cp = s_cp + threadIdx.x * LP;
-        int pending = 0, acc = 0;
+        int pending = 0, acc = 0, lo = 0x80, hi = 0xBF;
         for (long long p = offsets[seq]; p < offsets[seq + 1] && !status; ++p) {
             const int id = flat[p];
             if (id < 0 || id >= n_vocab) { status = 1; break; }
@@ -1660,13 +1670,16 @@ bpe_decode_kernel(const int* __restrict__ flat, const long long* __restrict__ of
                 const int bt = tok_bytes[q];
                 int out_c = -1;
                 if (pending) {
-                    if ((bt & 0xC0) != 0x80) { status = 2; break; }
+                    if (bt < lo || bt > hi) { status = 2; break; }
+                    lo = 0x80; hi = 0xBF;
                     acc = (acc << 6) | (bt & 0x3F);
                     if (--pending == 0) out_c = acc;
                 } else if (bt < 0x80) out_c = bt;
-                else if ((bt & 0xE0) == 0xC0) { acc = bt & 0x1F; pending = 1; }
-                else if ((bt & 0xF0) == 0xE0) { acc = bt & 0x0F; pending = 2; }
-                else if ((bt & 0xF8) == 0xF0) { acc = bt & 0x07; pending = 3; }
+                else if (utf8_lead_len(bt) >= 2) {
+                    pending = utf8_lead_len(bt) - 1;
+                    acc = bt & (0x3F >> pending);
+                    lo = utf8_second_lo(bt); hi = utf8_second_hi(bt);
+                }
                 else { status = 2; break; }
                 if (out_c >= 0) {
                     if (out_c > 0xFFFF) { status = 2; break; }   // not a shifted bin
@@ -1697,7 +1710,8 @@ bpe_decode_kernel(const int* __restrict__ flat, const long long* __restrict__ of
 // range, tokens of more than SLOTS characters — is flagged (status kDecodeNeedsBytes) and decoded by the byte-level
 // kernel below, which also decides WHICH of the reference's errors the sequence has.
 //   SLOTS = 2: 8-byte entries {c0 | c1 << 16, meta}; SLOTS = 6: 16-byte entries {c0|c1, c2|c3, c4|c5, meta};
-//   meta = characters started | bytes still needed << 3 | leading continuation bytes << 5 | slow << 7 | payload << 8.
+//   meta = characters started | bytes still needed << 3 | leading continuation bytes << 5 | slow << 7 | payload << 8
+//          | ends in a bare E0 lead << 26 | ends in a bare ED lead << 27.
 constexpr int kDecodeNeedsBytes = 0x100;
 template <int SLOTS>
 __global__ void __launch_bounds__(256, 8)
@@ -1735,7 +1749,9 @@ bpe_decode_token_kernel(const int* __restrict__ flat, const long long* __restric
             if (lane == 31) nmeta = nmeta0;
             const int nst = (int)(meta & 7u);
             const unsigned int need = (meta >> 3) & 3u;
-            if ((meta & 0x80u) || need != ((nmeta >> 5) & 3u)) bad = true;
+            // slow, or a bare E0 / ED lead ends the token (bits 26 / 27: strict UTF-8 restricts the next byte — no overlong
+            // form, no surrogate — which the byte-level kernel checks), or the boundary does not match
+            if ((meta & 0x0C000080u) || need != ((nmeta >> 5) & 3u)) bad = true;
             const unsigned int tail = need ? ((nmeta >> 8) & 0x3ffffu) : 0u;
             int at, total;
             if (SLOTS == 2) {                                   // counts of 0 / 1 / 2: two ballots
@@ -1791,10 +1807,6 @@ bpe_decode_token_kernel(const int* __restrict__ flat, const long long* __restric
 // sequential decoder's order: the byte stream ends at the first id out of range; an invalid byte before
 // that point gives status 2, else the bad id gives 1, else an unfinished character at the end gives 2,
 // else a character count != L gives 3 (the reference's length ValueError, bpe_tokenizer.py:241-244).
-__device__ __forceinline__ int utf8_lead_len(int b) {
-    return b < 0x80 ? 1 : ((b & 0xE0) == 0xC0 ? 2 : ((b & 0xF0) == 0xE0 ? 3 : ((b & 0xF8) == 0xF0 ? 4 : 0)));
-}
-
 __global__ void __launch_bounds__(256)
 bpe_decode_warp_kernel(const int* __restrict__ flat, const long long* __restrict__ offsets, long long N, int L,
                        long long min_token, const int* __restrict__ tok_off, const uint8_t* __restrict__ tok_bytes,
@@ -1835,7 +1847,7 @@ bpe_decode_warp_kernel(const int* __restrict__ flat, const long long* __restrict
             // more bytes than any valid sequence can have: the sequential state machine decides which error
             // comes first (rare; one lane, straight from global memory)
             if (lane == 0) {
-                int pending = 0, acc = 0;
+                int pending = 0, acc = 0, lo = 0x80, hi = 0xBF;
                 for (long long p = p0; p < p1 && !status; ++p) {
                     const int id = flat[p];
                     if (id < 0 || id >= n_vocab) { status = 1; break; }
@@ -1843,11 +1855,16 @@ bpe_decode_warp_kernel(const int* __restrict__ flat, const long long* __restrict
                         const int bt = tok_bytes[q];
                         int out_c = -1;
                         if (pending) {
-                            if ((bt & 0xC0) != 0x80) { status = 2; break; }
+                            if (bt < lo || bt > hi) { status = 2; break; }
+                            lo = 0x80; hi = 0xBF;
                             acc = (acc << 6) | (bt & 0x3F);
                             if (--pending == 0) out_c = acc;
                         } else if (bt < 0x80) out_c = bt;
-                        else if (utf8_lead_len(bt) >= 2) { pending = utf8_lead_len(bt) - 1; acc = bt & (0x3F >> pending); }
+                        else if (utf8_lead_len(bt) >= 2) {
+                            pending = utf8_lead_len(bt) - 1;
+                            acc = bt & (0x3F >> pending);
+                            lo = utf8_second_lo(bt); hi = utf8_second_hi(bt);
+                        }
                         else { status = 2; break; }
                         if (out_c >= 0) {
                             if (out_c > 0xFFFF) { status = 2; break; }
@@ -1873,14 +1890,15 @@ bpe_decode_warp_kernel(const int* __restrict__ flat, const long long* __restrict
                 int err = 0x7fffffff, cpv = -1;
                 if (start) {
                     const int n = utf8_lead_len(b);
-                    if (n == 0) err = i;                      // 0xF8..0xFF
+                    if (n == 0) err = i;                      // C0, C1, F5..FF
                     else {
                         int acc = n == 1 ? b : (b & (0x7F >> n));
                         bool complete = true;
                         for (int k = 1; k < n; ++k) {
                             if (i + k >= B) { pend_end = true; complete = false; break; }
                             const int c = s_b[i + k];
-                            if ((c & 0xC0) != 0x80) { err = i + k; complete = false; break; }
+                            const bool ok = k == 1 ? c >= utf8_second_lo(b) && c <= utf8_second_hi(b) : (c & 0xC0) == 0x80;
+                            if (!ok) { err = i + k; complete = false; break; }
                             acc = (acc << 6) | (c & 0x3F);
                         }
                         if (complete) {
@@ -1936,6 +1954,52 @@ static int stage_rows_per_block(int L, int cp_bytes = 2) {
 }
 static size_t stage_smem(int L, int rows, int cp_bytes = 2) {
     return (((size_t)rows * (L + 1) * cp_bytes + 3) & ~(size_t)3) + (size_t)rows * sizeof(int);
+}
+
+// Launch shape of the warp-per-sequence apply kernels: warps per CTA (0: a warp's arrays do not fit shared memory)
+// and the CTA cap of the grid.  Every warp strides over the sequences, so one pass covers warps * max_ctas of them.
+struct ApplyShape { int warps; long long max_ctas; size_t warp_bytes, key2_off; };
+
+static int device_sms() {
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    return sms;
+}
+// CTAs per SM: as many as shared memory and the 2048 threads of an SM allow
+static long long ctas_per_sm(int warps, size_t smem) {
+    long long per_sm = (long long)(220 * 1024) / (long long)(smem + 1024);
+    if (per_sm > 2048 / (warps * 32)) per_sm = 2048 / (warps * 32);
+    return per_sm < 1 ? 1 : per_sm;
+}
+// bpe_encode_warp_kernel; per warp: key u32[M], sym / wid u16[M], cp u16[L rounded to even], wbeg u16[L+2], key2 u32[M]
+static ApplyShape encode_warp_shape(int L, int M, int sms) {
+    ApplyShape s{};
+    s.key2_off = ((size_t)8 * M + 2 * (size_t)((L + 1) & ~1) + 2 * (size_t)(L + 2) + 3) & ~(size_t)3;
+    s.warp_bytes = (s.key2_off + (size_t)4 * M + 15) & ~(size_t)15;
+    s.warps = (int)((200 * 1024) / s.warp_bytes);
+    if (s.warps > 8) s.warps = 8;
+    if (s.warps >= 1) s.max_ctas = sms * ctas_per_sm(s.warps, s.warp_bytes * s.warps);
+    return s;
+}
+// bpe_decode_token_kernel (8 warps of 256 threads, up to 8 CTAs per SM); per warp: u16[L rounded up to 8].  Rows
+// longer than 8192 bins are left to the byte-level kernel.
+static ApplyShape decode_token_shape(int L, int sms) {
+    ApplyShape s{};
+    s.warps = L <= 8192 ? 8 : 0;
+    s.warp_bytes = (((size_t)L + 7) & ~(size_t)7) * 2;
+    s.max_ctas = (long long)sms * 8;
+    return s;
+}
+// bpe_decode_warp_kernel; per warp: the token bytes (cap = 4 L + 64: a valid sequence has at most 3 L) + u16[L]
+static ApplyShape decode_warp_shape(int L, int sms) {
+    ApplyShape s{};
+    const int cap = 4 * L + 64;
+    s.warp_bytes = (((size_t)cap + 15) & ~(size_t)15) + (((size_t)L * 2 + 15) & ~(size_t)15);
+    s.warps = (int)((200 * 1024) / s.warp_bytes);
+    if (s.warps > 8) s.warps = 8;
+    if (s.warps >= 1) s.max_ctas = sms * ctas_per_sm(s.warps, s.warp_bytes * s.warps);
+    return s;
 }
 
 }  // namespace beast
@@ -2274,27 +2338,19 @@ extern "C" int bpe_encode(const int64_t* bins, int64_t N, int32_t L, int64_t min
     if (M > 65535) return BEAST_E_SHAPE;
     // one warp per sequence, working arrays in shared memory; sequences too long for that (or
     // BEAST_B200_BPE_THREAD_ENCODE=1) take the one-thread-per-sequence kernel
-    const size_t key2_off = ((size_t)8 * M + 2 * (size_t)((L + 1) & ~1) + 2 * (size_t)(L + 2) + 3) & ~(size_t)3;
-    const size_t warp_bytes = (key2_off + (size_t)4 * M + 15) & ~(size_t)15;
-    int warps = (int)((200 * 1024) / warp_bytes);
-    if (warps > 8) warps = 8;
+    const ApplyShape sh = encode_warp_shape(L, M, device_sms());
     // test hook, re-read per call (the tests toggle it): one getenv is noise next to a launch
     const char* env = getenv("BEAST_B200_BPE_THREAD_ENCODE");
-    if (warps >= 1 && !(env && env[0] == '1')) {
-        const size_t smem = warp_bytes * warps;
+    if (sh.warps >= 1 && !(env && env[0] == '1')) {
+        const int warps = sh.warps;
+        const size_t smem = sh.warp_bytes * warps;
         static size_t granted[kMaxDevices] = {};
         if (int rc = opt_in_smem(bpe_encode_warp_kernel, smem, granted)) return rc;
-        int dev = 0, sms = 148;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        long long per_sm = (long long)(220 * 1024) / (long long)(smem + 1024);
-        if (per_sm > 2048 / (warps * 32)) per_sm = 2048 / (warps * 32);
-        if (per_sm < 1) per_sm = 1;
         long long grid = (N + warps - 1) / warps;
-        if (grid > sms * per_sm) grid = sms * per_sm;
+        if (grid > sh.max_ctas) grid = sh.max_ctas;
         bpe_encode_warp_kernel<<<(unsigned)grid, warps * 32, smem, (cudaStream_t)stream>>>(
             (const long long*)bins, N, L, min_token, max_shift, byte_to_id, cls_tab, rank_tab, V, ids_padded, out_stride,
-            len_out, status_out, M, (int)warp_bytes, (int)key2_off, hash_bits);
+            len_out, status_out, M, (int)sh.warp_bytes, (int)sh.key2_off, hash_bits);
         count_launch();
         BEAST_CHECK_LAUNCH();
         return BEAST_OK;
@@ -2310,6 +2366,18 @@ extern "C" int bpe_encode(const int64_t* bins, int64_t N, int32_t L, int64_t min
         len_out, status_out, rows, hash_bits);
     count_launch();
     BEAST_CHECK_LAUNCH();
+    return BEAST_OK;
+}
+
+extern "C" int bpe_apply_shape(int32_t kernel, int32_t L, int64_t max_shift, int32_t* warps, int64_t* max_ctas) {
+    if (!warps || !max_ctas) return BEAST_E_NULL;
+    if (L < 1 || kernel < 0 || kernel > 2) return BEAST_E_SHAPE;
+    const int mult = max_shift < 0x80 ? 1 : (max_shift < 0x800 ? 2 : 3);
+    const int sms = device_sms();
+    const ApplyShape s = kernel == 0 ? encode_warp_shape(L, mult * L, sms)
+                                     : (kernel == 1 ? decode_token_shape(L, sms) : decode_warp_shape(L, sms));
+    *warps = s.warps;
+    *max_ctas = s.warps ? s.max_ctas : 0;
     return BEAST_OK;
 }
 
@@ -2333,22 +2401,21 @@ extern "C" int bpe_decode(const int32_t* flat, const int64_t* offsets, int64_t N
     if (tok_tab && tok_tab_slots != 2 && tok_tab_slots != 6) return BEAST_E_SHAPE;
     if ((uintptr_t)tok_tab & 15u) return BEAST_E_ALIGN;
     cudaStream_t st = (cudaStream_t)stream;
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const int sms = device_sms();
     // test hook, re-read per call (the tests toggle it between calls): one getenv is noise next to a launch
     const char* env_thread = getenv("BEAST_B200_BPE_THREAD_DECODE");
     const int force_thread = (env_thread && env_thread[0] == '1') ? 1 : 0;
     int only_flagged = 0;
-    if (tok_tab && !force_thread && L <= 8192) {
+    const ApplyShape tsh = decode_token_shape(L, sms);
+    if (tok_tab && !force_thread && tsh.warps) {
         // fast path: one lane per token from the per-token character table; sequences it cannot describe are flagged
-        const size_t smem = (size_t)8 * (((size_t)L + 7) & ~(size_t)7) * 2;
+        const size_t smem = tsh.warp_bytes * tsh.warps;
         static size_t granted2[kMaxDevices] = {}, granted6[kMaxDevices] = {};
         int rc = tok_tab_slots == 2 ? opt_in_smem(bpe_decode_token_kernel<2>, smem, granted2)
                                     : opt_in_smem(bpe_decode_token_kernel<6>, smem, granted6);
         if (rc) return rc;
         long long grid = (N + 7) / 8;
-        if (grid > (long long)sms * 8) grid = (long long)sms * 8;
+        if (grid > tsh.max_ctas) grid = tsh.max_ctas;
         if (tok_tab_slots == 2)
             bpe_decode_token_kernel<2><<<(unsigned)grid, 256, smem, st>>>(flat, (const long long*)offsets, N, L, min_token, tok_tab,
                                                                          n_vocab, (long long*)bins_out, status_out, declen_out);
@@ -2361,22 +2428,17 @@ extern "C" int bpe_decode(const int32_t* flat, const int64_t* offsets, int64_t N
     }
     {   // byte-level path, one warp per sequence (all sequences, or only the ones the fast kernel flagged);
         // BEAST_B200_BPE_THREAD_DECODE=1 (or rows too long for shared memory) takes the one-thread-per-sequence kernel
-        const int cap = 4 * L + 64;                          // a valid sequence has at most 3 L bytes
-        const size_t warp_bytes = (((size_t)cap + 15) & ~(size_t)15) + (((size_t)L * 2 + 15) & ~(size_t)15);
-        int warps = (int)((200 * 1024) / warp_bytes);
-        if (warps > 8) warps = 8;
-        if (warps >= 1 && !force_thread) {
-            const size_t smem = warp_bytes * warps;
+        const ApplyShape sh = decode_warp_shape(L, sms);
+        if (sh.warps >= 1 && !force_thread) {
+            const int warps = sh.warps;
+            const size_t smem = sh.warp_bytes * warps;
             static size_t granted_w[kMaxDevices] = {};
             if (int rc = opt_in_smem(bpe_decode_warp_kernel, smem, granted_w)) return rc;
-            long long per_sm = (long long)(220 * 1024) / (long long)(smem + 1024);
-            if (per_sm > 2048 / (warps * 32)) per_sm = 2048 / (warps * 32);
-            if (per_sm < 1) per_sm = 1;
             long long grid = (N + warps - 1) / warps;
-            if (grid > sms * per_sm) grid = sms * per_sm;
+            if (grid > sh.max_ctas) grid = sh.max_ctas;
             bpe_decode_warp_kernel<<<(unsigned)grid, warps * 32, smem, st>>>(
                 flat, (const long long*)offsets, N, L, min_token, tok_off, tok_bytes, n_vocab, (long long*)bins_out,
-                status_out, declen_out, cap, (int)warp_bytes, only_flagged);
+                status_out, declen_out, 4 * L + 64, (int)sh.warp_bytes, only_flagged);
             count_launch();
             BEAST_CHECK_LAUNCH();
             return BEAST_OK;

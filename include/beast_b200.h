@@ -455,6 +455,10 @@ int bpe_encode(const int64_t* bins, int64_t N, int32_t L, int64_t min_token, int
                const int16_t* byte_to_id, const uint8_t* cls_tab, const uint32_t* rank_tab, int32_t V,
                int32_t hash_bits, uint16_t* ids_padded, int32_t out_stride, int32_t* len_out, int32_t* status_out,
                void* stream);
+/* Launch shape of a warp-per-sequence apply kernel on the current device (kernel 0 = bpe_encode's, 1 = bpe_decode's
+ * per-token fast path, 2 = bpe_decode's byte-level kernel) for rows of L bins: warps per CTA (0 = the kernel is not
+ * used at this L) and the CTA cap of its grid.  Each warp strides over the rows, warps * max_ctas of them per pass. */
+int bpe_apply_shape(int32_t kernel, int32_t L, int64_t max_shift, int32_t* warps, int64_t* max_ctas);
 int bpe_compact(const uint16_t* ids_padded, int32_t stride, const int32_t* len, const int64_t* offsets,
                 int64_t N, int32_t* flat, void* stream);
 int bpe_decode(const int32_t* flat, const int64_t* offsets, int64_t N, int32_t L, int64_t min_token,

@@ -407,6 +407,22 @@ int bpe_oracle_encode(const void* p, const int64_t* shifted, int n, int32_t* ids
     return out;
 }
 
+/* Encode n_seq rows of L shifted bins: the ids of row s land at ids_out[off_out[s] .. off_out[s + 1]).  ids_out holds
+ * ids_cap entries (3 * n_seq * L always suffice).  Returns the total id count, or -1 if ids_cap is too small. */
+int64_t bpe_oracle_encode_batch(const void* p, const int64_t* shifted, int64_t n_seq, int L, int32_t* ids_out,
+                                int64_t ids_cap, int64_t* off_out) {
+    int32_t* row = (int32_t*)malloc(sizeof(int32_t) * ((size_t)3 * L + 3));
+    off_out[0] = 0;
+    for (int64_t s = 0; s < n_seq; ++s) {
+        const int n = bpe_oracle_encode(p, shifted + s * L, L, row);
+        if (off_out[s] + n > ids_cap) { free(row); return -1; }
+        memcpy(ids_out + off_out[s], row, sizeof(int32_t) * (size_t)n);
+        off_out[s + 1] = off_out[s] + n;
+    }
+    free(row);
+    return off_out[n_seq];
+}
+
 /* Decode ids -> codepoints (before adding min_token).  Returns the count, or -1 on an unknown id /
  * a byte-level character outside the 256-entry map, -2 on invalid UTF-8, -3 if out_cap is too small. */
 int bpe_oracle_decode(const void* p, const int32_t* ids, int n, int64_t* out, int out_cap) {

@@ -27,6 +27,9 @@ def lib():
         _lib.bpe_oracle_model_free.argtypes = [C.c_void_p]
         _lib.bpe_oracle_encode.restype = C.c_int
         _lib.bpe_oracle_encode.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
+        _lib.bpe_oracle_encode_batch.restype = C.c_int64
+        _lib.bpe_oracle_encode_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_int64,
+                                                 C.c_void_p]
         _lib.bpe_oracle_decode.restype = C.c_int
         _lib.bpe_oracle_decode.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int]
         _lib.bpe_oracle_pretokenize.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
@@ -165,6 +168,19 @@ class OracleBPE:
         out = np.zeros(3 * len(shifted) + 3, dtype=np.int32)
         n = lib().bpe_oracle_encode(self._m(), shifted.ctypes.data, len(shifted), out.ctypes.data)
         return out[:n].tolist()
+
+    def encode_batch(self, shifted):
+        """Rows [N, L] of shifted bins -> (ids int32, offsets int64 [N + 1]): encode() of every row in one call."""
+        shifted = np.ascontiguousarray(shifted, dtype=np.int64)
+        n, L = shifted.shape
+        width = 1 if n == 0 or shifted.max() < 0x80 else 2 if shifted.max() < 0x800 else 3   # ids <= UTF-8 bytes
+        ids = np.zeros(max(width * n * L, 1), dtype=np.int32)
+        off = np.zeros(n + 1, dtype=np.int64)
+        total = lib().bpe_oracle_encode_batch(self._m(), shifted.ctypes.data, n, L, ids.ctypes.data, ids.size,
+                                              off.ctypes.data)
+        if total < 0:
+            raise RuntimeError("bpe_oracle_encode_batch: id buffer too small")
+        return ids[:total], off
 
     def decode(self, ids, cap=4096):
         ids = np.ascontiguousarray(ids, dtype=np.int32)

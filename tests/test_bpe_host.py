@@ -305,21 +305,37 @@ def test_match_resolution_by_function_composition():
 def test_parallel_utf8_decode_rules_match_the_state_machine():
     """The warp-per-sequence BPE decode (csrc/bpe.cu: bpe_decode_warp_kernel) classifies every byte on its own:
     a non-continuation byte starts a character (index = number of such bytes before it), a continuation byte
-    must lie inside the span of the lead before it.  Restated here and compared with the sequential decoder
-    (status 2 = invalid UTF-8, 3 = wrong length, character count) on random byte streams."""
+    must lie inside the span of the lead before it.  Restated here and compared with the sequential decoder and with
+    Python's strict decoder (status 2 = invalid UTF-8 — overlong and surrogate forms included — or a character above
+    U+FFFF, 3 = wrong length, character count) on random byte streams."""
     rng = np.random.default_rng(9)
 
-    def lead_len(b):
-        return 1 if b < 0x80 else 2 if (b & 0xE0) == 0xC0 else 3 if (b & 0xF0) == 0xE0 else 4 if (b & 0xF8) == 0xF0 else 0
+    def lead_len(b):                                    # strict UTF-8: C0, C1 and F5..FF start nothing
+        return 1 if b < 0x80 else 0 if b < 0xC2 else 2 if b < 0xE0 else 3 if b < 0xF0 else 4 if b < 0xF5 else 0
+
+    def second_ok(lead, c):                             # overlong, surrogate and > U+10FFFF forms fail here
+        lo = 0xA0 if lead == 0xE0 else 0x90 if lead == 0xF0 else 0x80
+        hi = 0x9F if lead == 0xED else 0x8F if lead == 0xF4 else 0xBF
+        return lo <= c <= hi
+
+    def python_strict(bs, L):                           # Python's strict decoder + the kernels' status order
+        try:
+            cps = [ord(c) for c in bytes(bs).decode("utf-8")]
+        except UnicodeDecodeError:
+            return 2, None, None
+        if any(c > 0xFFFF for c in cps):                # valid UTF-8, but no shifted bin
+            return 2, None, None
+        return (3 if len(cps) != L else 0), len(cps), cps[:L]
 
     def sequential(bs, L):
-        status = cnt = pending = acc = 0
+        status = cnt = pending = acc = lead = 0
         out = []
         for bt in bs:
             c = -1
             if pending:
-                if (bt & 0xC0) != 0x80:
+                if not (second_ok(lead, bt) if lead else (bt & 0xC0) == 0x80):
                     return 2, cnt, out
+                lead = 0
                 acc = (acc << 6) | (bt & 0x3F)
                 pending -= 1
                 if pending == 0:
@@ -329,6 +345,7 @@ def test_parallel_utf8_decode_rules_match_the_state_machine():
             elif lead_len(bt) >= 2:
                 pending = lead_len(bt) - 1
                 acc = bt & (0x3F >> pending)
+                lead = bt
             else:
                 return 2, cnt, out
             if c >= 0:
@@ -359,7 +376,7 @@ def test_parallel_utf8_decode_rules_match_the_state_machine():
                             pend_end, complete = True, False
                             break
                         c = bs[i + k]
-                        if (c & 0xC0) != 0x80:
+                        if not (second_ok(b, c) if k == 1 else (c & 0xC0) == 0x80):
                             err, complete = i + k, False
                             break
                         acc = (acc << 6) | (c & 0x3F)
@@ -387,7 +404,16 @@ def test_parallel_utf8_decode_rules_match_the_state_machine():
             return 2, None, None
         return (3 if cnt != L else 0), cnt, [out[i] for i in range(min(cnt, L))]
 
-    pool = [0x41, 0x7A, 0xC3, 0xA9, 0x80, 0xBF, 0xE2, 0x82, 0xAC, 0xF0, 0x9F, 0x98, 0xF8, 0xFF, 0xC2]
+    pool = [0x41, 0x7A, 0xC3, 0xA9, 0x80, 0xBF, 0xE2, 0x82, 0xAC, 0xF0, 0x9F, 0x98, 0xF8, 0xFF, 0xC2,
+            0xE0, 0xED, 0xA0, 0x90, 0x8F, 0xC0, 0xC1, 0xF4, 0xF5]
+    fixed = [[0xE0, 0x80, 0x80], [0xED, 0xA0, 0x80], [0xC0, 0x80], [0xC1, 0xBF], [0xF0, 0x80, 0x80, 0x80],
+             [0xF4, 0x90, 0x80, 0x80], [0xF5, 0x80], [0xE0, 0xA0, 0x80], [0xED, 0x9F, 0xBF], [0xEE, 0x80, 0x80],
+             [0xF0, 0x90, 0x80, 0x80], [0x41, 0xE0], [0x41, 0xE0, 0x9F], [0x41, 0xED, 0xA0]]
+    for bs in fixed:                                    # overlong / surrogate / out-of-range forms and their neighbours
+        for L in range(4):
+            want = python_strict(bs, L)
+            for got in (sequential(bs, L), parallel(bs, L)):
+                assert got[0] == want[0] and (want[0] == 2 or got[1:] == want[1:]), (bs, L, got, want)
     for trial in range(3000):
         if trial % 3 == 0:                              # valid text with a few mutations
             text = "".join(chr(int(v)) for v in rng.integers(1, 0x2FFF, int(rng.integers(0, 12))))
@@ -399,9 +425,10 @@ def test_parallel_utf8_decode_rules_match_the_state_machine():
         L = int(rng.integers(0, 8))
         s1, c1, o1 = sequential(bs, L)
         s2, c2, o2 = parallel(bs, L)
-        assert s1 == s2, (bs, L, s1, s2)
+        s3, c3, o3 = python_strict(bs, L)
+        assert s1 == s2 == s3, (bs, L, s1, s2, s3)
         if s1 in (0, 3):
-            assert c1 == c2 and o1 == o2, (bs, L)
+            assert c1 == c2 == c3 and o1 == o2 == o3, (bs, L)
 
 
 def test_token_character_table_matches_the_state_machine():
@@ -414,36 +441,19 @@ def test_token_character_table_matches_the_state_machine():
     from beast_tokenizer_b200.bpe_model import token_char_entry
     rng = np.random.default_rng(13)
 
-    def sequential(bs):
-        out, pending, acc = [], 0, 0
-        for bt in bs:
-            if pending:
-                if (bt & 0xC0) != 0x80:
-                    return None
-                acc = (acc << 6) | (bt & 0x3F)
-                pending -= 1
-                if pending == 0:
-                    if acc > 0xFFFF:
-                        return None
-                    out.append(acc)
-            elif bt < 0x80:
-                out.append(bt)
-            elif (bt & 0xE0) == 0xC0:
-                acc, pending = bt & 0x1F, 1
-            elif (bt & 0xF0) == 0xE0:
-                acc, pending = bt & 0x0F, 2
-            elif (bt & 0xF8) == 0xF0:
-                acc, pending = bt & 0x07, 3
-            else:
-                return None
-        return None if pending else out
+    def sequential(bs):                 # Python's strict decoder; characters above U+FFFF are no shifted bin
+        try:
+            out = [ord(c) for c in bytes(bs).decode("utf-8")]
+        except UnicodeDecodeError:
+            return None
+        return None if any(c > 0xFFFF for c in out) else out
 
     def fast(tokens):
         ent = [token_char_entry(t) for t in tokens]
         if not ent:
             return []
         meta = [e[3] for e in ent]
-        if any(m & 0x80 for m in meta) or (meta[0] >> 5) & 3:
+        if any(m & 0x0C000080 for m in meta) or (meta[0] >> 5) & 3:     # slow, or a bare E0 / ED lead ends a token
             return None
         out = []
         for i, e in enumerate(ent):
@@ -476,17 +486,27 @@ def test_token_character_table_matches_the_state_machine():
             # and the character needs more
             chained = any(all((b & 0xC0) == 0x80 for b in t) and i + 1 < len(toks) and (toks[i + 1][0] & 0xC0) == 0x80
                           for i, t in enumerate(toks))
-            if short and not chained:
+            # a token ending in a bare E0 / ED lead sends the sequence to the byte-level path (its next byte is restricted)
+            bare_lead = any(t[-1] in (0xE0, 0xED) for t in toks[:-1])
+            if short and not chained and not bare_lead:
                 assert got == want, (toks, got, want)
                 accepted += 1
         else:                   # garbage bytes: the fast path may refuse, but must never disagree
-            pool = [0x41, 0x7A, 0xC3, 0xA9, 0x80, 0xBF, 0xE2, 0x82, 0xAC, 0xF0, 0x9F, 0x98, 0xF8, 0xFF, 0xC2]
+            pool = [0x41, 0x7A, 0xC3, 0xA9, 0x80, 0xBF, 0xE2, 0x82, 0xAC, 0xF0, 0x9F, 0x98, 0xF8, 0xFF, 0xC2,
+                    0xE0, 0xED, 0xA0, 0x90, 0x8F, 0xC0, 0xC1, 0xF4, 0xF5]
             toks = [bytes(int(v) for v in rng.choice(pool, int(rng.integers(1, 5)))) for _ in range(int(rng.integers(1, 12)))]
             want = sequential(b"".join(toks))
             got = fast(toks)
             if got is not None:
                 assert want == got, (toks, got, want)
     assert accepted > 1000
+    # overlong and surrogate forms, whole or split after their lead: never accepted
+    for toks in ([b"\xe0\x80\x80"], [b"\xe0", b"\x80\x80"], [b"\xe0\x80", b"\x80"], [b"\xed\xa0\x80"], [b"A\xed", b"\xa0\x80"],
+                 [b"\xed", b"\xbf\xbf"], [b"\xc0\x80"], [b"\xc1", b"\xbf"]):
+        assert fast(toks) is None, toks
+    # the nearest valid forms are, unless split after their lead
+    assert fast([b"\xed\x9f", b"\xbf"]) == [0xD7FF] and fast([b"\xe0\xa0", b"\x80A"]) == [0x800, 0x41]
+    assert fast([b"\xed", b"\x9f\xbf"]) is None and fast([b"\xe0", b"\xa0\x80A"]) is None
 
 
 def test_rank_order_batch_merging_equals_one_merge_at_a_time():
