@@ -79,7 +79,7 @@ class GpuBpeEngine:
 
     DEDUP_SAMPLE = 65536          # "auto": distinct-word statistics are taken on this many sequences first
     DEDUP_KEEP = 0.7              # ... and the corpus is de-duplicated when distinct symbols / symbols is below this
-    DEDUP_PACK = int(__import__("os").environ.get("BEAST_B200_DEDUP_PACK", "64"))   # symbols per pseudo-sequence of packed distinct words (plus one straddling word)
+    DEDUP_PACK = 64               # symbols per pseudo-sequence of packed distinct words (plus one straddling word)
 
     def __init__(self, bins: torch.Tensor, min_token: int, byte_to_id: np.ndarray, V: int, max_shift: int = 255,
                  row_len: Optional[torch.Tensor] = None, dedup="auto", seen_bytes: Optional[np.ndarray] = None):

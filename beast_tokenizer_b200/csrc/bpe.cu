@@ -24,7 +24,6 @@
 // walks 32 sequences reads / writes chunk c of all of them as 512 contiguous bytes, one 128-bit access
 // per lane.
 #include <cstring>
-#include <cooperative_groups.h>
 #include "bpe_common.cuh"
 
 namespace beast {
@@ -770,30 +769,16 @@ __device__ __forceinline__ void rewrite_sequence_warp(uint16_t* __restrict__ sym
     __syncwarp();
 }
 
-// A "virtual block": the scan and rewrite phases are written for blocks of 256 threads.  As stand-alone kernels a
-// virtual block is a CUDA block (barrier 0); inside the persistent loop kernel a 1024-thread block hosts four of them
-// (named barriers 1..4, private shared-memory regions), so that the same code runs in both.
-struct VBlock {
-    int tid, bid, nblocks, nthreads, bar;
-};
-__device__ __forceinline__ void vb_sync(const VBlock& vb) {
-    asm volatile("bar.sync %0, %1;" ::"r"(vb.bar), "r"(vb.nthreads) : "memory");
-}
-__device__ __forceinline__ VBlock real_block() {
-    VBlock vb;
-    vb.tid = (int)threadIdx.x; vb.bid = (int)blockIdx.x; vb.nblocks = (int)gridDim.x; vb.nthreads = (int)blockDim.x; vb.bar = 0;
-    return vb;
-}
-
 // Block-private 4 x V delta counters in (dynamic, 16-byte aligned) shared memory: zero / flush with
-// 128-bit accesses; only non-zero counters reach the global delta block.
-__device__ __forceinline__ void zero_delta_block(const VBlock& vb, int* s_delta, int V) {
+// 128-bit accesses; only non-zero counters reach the global delta block.  The strides of these loops (and of the
+// pick + scan kernel's) are signed: `i += blockDim.x` may wrap, which keeps the compiler from unrolling them.
+__device__ __forceinline__ void zero_delta_block(int* s_delta, int V) {
     int4* p = (int4*)s_delta;
-    for (int i = vb.tid; i < V; i += vb.nthreads) p[i] = make_int4(0, 0, 0, 0);      // 4 V ints = V int4
+    for (int i = threadIdx.x; i < V; i += (int)blockDim.x) p[i] = make_int4(0, 0, 0, 0);      // 4 V ints = V int4
 }
-__device__ __forceinline__ void flush_delta_block(const VBlock& vb, const int* s_delta, int* __restrict__ delta, int V) {
+__device__ __forceinline__ void flush_delta_block(const int* s_delta, int* __restrict__ delta, int V) {
     const int4* p = (const int4*)s_delta;
-    for (int i = vb.tid; i < V; i += vb.nthreads) {
+    for (int i = threadIdx.x; i < V; i += (int)blockDim.x) {
         const int4 d = p[i];
         if (d.x | d.y | d.z | d.w) {
             if (d.x) atomicAdd(&delta[4 * i], d.x);
@@ -805,36 +790,42 @@ __device__ __forceinline__ void flush_delta_block(const VBlock& vb, const int* s
 }
 
 constexpr int kRewriteOut = 32 * kChunk + kChunk;            // staging of one warp-rewritten sequence (symbols)
-__device__ __forceinline__ void
-rewrite_body(const VBlock& vb, int* s_delta, uint16_t (*s_out)[kRewriteOut],
-             uint16_t* __restrict__ sym, int* __restrict__ len, long long n_stride, int a, int b, int c, int V,
-             const BpeCtl* __restrict__ ctl, const int* __restrict__ work_count,
-             const int* __restrict__ work_seq, const int* __restrict__ work_q0, int* __restrict__ delta,
-             unsigned int* __restrict__ sig, const int* __restrict__ weight) {
+__global__ void __launch_bounds__(256)
+bpe_rewrite_kernel(uint16_t* __restrict__ sym, int* __restrict__ len, long long n_stride, int a, int b, int c, int V,
+                   const BpeCtl* __restrict__ ctl, const int* __restrict__ work_count,
+                   const int* __restrict__ work_seq, const int* __restrict__ work_q0, int* __restrict__ delta,
+                   unsigned int* __restrict__ sig, const int* __restrict__ weight) {
+    extern __shared__ int s_dyn[];
+    __shared__ uint16_t s_out[8][kRewriteOut];
+    // V < 0: launched without the 16 |V|-byte dynamic shared memory (vocabularies above 12 800 entries)
+    int* const s_delta = V > 0 ? s_dyn : nullptr;
+    V = V > 0 ? V : -V;
     if (ctl) {                                                // the state the scan kernel's pick wrote
+        pdl_wait();
+        pdl_launch();
         if (ctl->done) return;
         a = ctl->a; b = ctl->b; c = ctl->c;
         delta += ((ctl->n_merges - 1) & 1) * 4 * V;           // double-buffered by merge parity (peers may still read the other half)
     }
     const int n_work = *work_count;
-    if (n_work > kDirectDeltaWork && (long long)vb.bid * vb.nthreads >= n_work) return;       // nothing for this block
+    if (n_work > kDirectDeltaWork && (long long)blockIdx.x * blockDim.x >= n_work) return;       // nothing for this block
     if (n_work <= kDirectDeltaWork) {
         // short work list (the steady state after the first ~100 merges): the few count changes go straight
         // to the global delta block as fire-and-forget reductions, no 4 x V block-private counters to zero and
         // flush; one WARP per sequence (entries with more than 32 chunks left take the one-thread state machine)
-        const int lane = vb.tid & 31, warp = vb.tid >> 5, nw = vb.nthreads >> 5;
+        const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
         // a warp's entries are e0 + k * stride: the lanes fetch the (sequence, position, length) triples of up to
         // 32 of them at once, so that dependent-load chain is paid once per batch; the chunks of entry k + 1 are
         // pulled towards L1 while entry k is rewritten
-        const long long stride = (long long)vb.nblocks * nw;
+        const long long stride = (long long)gridDim.x * nw;
         const uint4* sym4 = (const uint4*)sym;
         const bool use_smem = n_work > kGlobalDeltaWork && s_delta != nullptr;   // nullptr: 4 x V counters do not fit shared memory
         if (use_smem) {
-            if ((long long)vb.bid * nw >= n_work) return;        // no entry for this block
-            zero_delta_block(vb, s_delta, V);
-            vb_sync(vb);
+            if ((long long)blockIdx.x * nw >= n_work) return;    // no entry for this block
+            zero_delta_block(s_delta, V);
+            __syncthreads();
         }
-        for (long long e0 = (long long)vb.bid * nw + warp; e0 < n_work; e0 += 32 * stride) {
+        for (long long e0 = (long long)blockIdx.x * nw + warp; e0 < n_work; e0 += 32 * stride) {
             const long long my_e = e0 + lane * stride;
             const bool have = my_e < n_work;
             const int my_seq = have ? work_seq[my_e] : 0, my_q0 = have ? work_q0[my_e] : 0;
@@ -863,42 +854,23 @@ rewrite_body(const VBlock& vb, int* s_delta, uint16_t (*s_out)[kRewriteOut],
             }
         }
         if (use_smem) {
-            vb_sync(vb);
-            flush_delta_block(vb, s_delta, delta, V);
+            __syncthreads();
+            flush_delta_block(s_delta, delta, V);
         }
         return;
     }
     if (s_delta != nullptr) {
-        zero_delta_block(vb, s_delta, V);
-        vb_sync(vb);
+        zero_delta_block(s_delta, V);
+        __syncthreads();
     }
     int* target = s_delta != nullptr ? s_delta : delta;         // very large vocabularies: straight to the global block
-    for (long long i = (long long)vb.bid * vb.nthreads + vb.tid; i < n_work;
-         i += (long long)vb.nblocks * vb.nthreads)
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n_work; i += (long long)gridDim.x * blockDim.x)
         rewrite_sequence(sym, len, work_seq[i], work_q0[i], n_stride, a, b, c, V, target, sig,
                          weight ? weight[work_seq[i]] : 1);
     if (s_delta != nullptr) {
-        vb_sync(vb);
-        flush_delta_block(vb, s_delta, delta, V);
+        __syncthreads();
+        flush_delta_block(s_delta, delta, V);
     }
-}
-
-__global__ void __launch_bounds__(256)
-bpe_rewrite_kernel(uint16_t* __restrict__ sym, int* __restrict__ len, long long n_stride, int a, int b, int c, int V,
-                   const BpeCtl* __restrict__ ctl, const int* __restrict__ work_count,
-                   const int* __restrict__ work_seq, const int* __restrict__ work_q0, int* __restrict__ delta,
-                   unsigned int* __restrict__ sig, const int* __restrict__ weight) {
-    extern __shared__ int s_delta[];
-    __shared__ uint16_t s_out[8][kRewriteOut];
-    if (ctl) {
-        pdl_wait();
-        pdl_launch();
-    }
-    // V < 0: launched without the 16 |V|-byte dynamic shared memory (vocabularies above 12 800 entries)
-    const bool has_smem = V > 0;
-    V = V > 0 ? V : -V;
-    rewrite_body(real_block(), has_smem ? s_delta : nullptr, s_out, sym, len, n_stride, a, b, c, V, ctl, work_count, work_seq, work_q0,
-                 delta, sig, weight);
 }
 
 // Iteration head of the sync-free loop: arg-max of the histogram, folding the delta block of the previous merge
@@ -910,10 +882,13 @@ bpe_rewrite_kernel(uint16_t* __restrict__ sym, int* __restrict__ len, long long 
 // flags and the fold pass sums the ranks' delta blocks with peer loads.  The histogram replicas stay identical, so
 // every rank picks the same merge without a broadcast.
 // (One block of 1024 threads per SM writes its maximum to partial[block]; every block of the scan kernel reduces them.)
-__device__ __forceinline__ void
-iterate_body(int* __restrict__ hist, int V, BpeCtl* __restrict__ ctl, int* __restrict__ delta,
-             unsigned long long* __restrict__ partial, int* __restrict__ work_count, const BpePeersDev& peers,
-             unsigned long long* s_best) {
+__global__ void __launch_bounds__(1024)
+bpe_iterate_kernel(int* __restrict__ hist, int V, BpeCtl* __restrict__ ctl, int* __restrict__ delta,
+                   unsigned long long* __restrict__ partial, int* __restrict__ work_count,
+                   const __grid_constant__ BpePeersDev peers) {
+    __shared__ unsigned long long s_best[32];
+    pdl_wait();
+    pdl_launch();
     if (ctl->done) return;
     const int n_active = ctl->n_tokens;
     const bool fold = ctl->has_delta != 0;
@@ -1044,16 +1019,6 @@ iterate_body(int* __restrict__ hist, int V, BpeCtl* __restrict__ ctl, int* __res
     }
 }
 
-__global__ void __launch_bounds__(1024)
-bpe_iterate_kernel(int* __restrict__ hist, int V, BpeCtl* __restrict__ ctl, int* __restrict__ delta,
-                   unsigned long long* __restrict__ partial, int* __restrict__ work_count,
-                   const __grid_constant__ BpePeersDev peers) {
-    __shared__ unsigned long long s_best[32];
-    pdl_wait();
-    pdl_launch();
-    iterate_body(hist, V, ctl, delta, partial, work_count, peers, s_best);
-}
-
 // Second kernel of an iteration: pick + scan.
 //   pick   EVERY block reduces the per-block maxima of the iteration head and applies BpeTrainer's stop rules
 //          (vocabulary full, count < min_frequency) itself — the state is read from ctl_in and the new state written
@@ -1064,42 +1029,37 @@ bpe_iterate_kernel(int* __restrict__ hist, int V, BpeCtl* __restrict__ ctl, int*
 //          those (lane per sequence, lock step) for the first hit; hits go to the global work list by
 //          warp-aggregated atomics — the rewrite kernel deals them evenly over all warps of the GPU (a fused
 //          scan + rewrite was measured 25 % slower: the hits of one warp's 32 survivors then serialise in that warp).
-struct ScanSmem {
-    int list[kScanTile];
-    unsigned long long best[8];
-    int pick[4];
-    int n;
-};
 template <bool DEEP>
-__device__ __forceinline__ void
-pick_scan_body(const VBlock& vb, ScanSmem& sm,
-               const uint16_t* __restrict__ sym, const int* __restrict__ len, long long N, long long n_stride, int V,
-               const BpeCtl* __restrict__ ctl_in, BpeCtl* __restrict__ ctl_out,
-               const unsigned long long* __restrict__ partial, int n_partial, int* __restrict__ log,
-               int vocab_size, int min_frequency, int max_merges, int* __restrict__ work_count,
-               int* __restrict__ work_seq, int* __restrict__ work_q0, const unsigned int* __restrict__ sig,
-               int tile_size) {
-    int* s_list = sm.list;
-    int& s_n = sm.n;
-    unsigned long long* s_best = sm.best;
-    int* s_pick = sm.pick;
-    const int lane = vb.tid & 31, warp = vb.tid >> 5;
+__global__ void __launch_bounds__(256)
+bpe_pick_scan_kernel(const uint16_t* __restrict__ sym, const int* __restrict__ len, long long N, long long n_stride, int V,
+                     const BpeCtl* __restrict__ ctl_in, BpeCtl* __restrict__ ctl_out,
+                     const unsigned long long* __restrict__ partial, int n_partial, int* __restrict__ log,
+                     int vocab_size, int min_frequency, int max_merges, int* __restrict__ work_count,
+                     int* __restrict__ work_seq, int* __restrict__ work_q0, const unsigned int* __restrict__ sig,
+                     int tile_size) {
+    __shared__ int s_list[kScanTile];
+    __shared__ unsigned long long s_best[8];
+    __shared__ int s_pick[4];
+    __shared__ int s_n;
+    pdl_wait();
+    pdl_launch();
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     // ---------------- pick
     const BpeCtl cur = *ctl_in;
     if (cur.done) {
-        if (vb.bid == 0 && vb.tid == 0) *ctl_out = cur;
+        if (blockIdx.x == 0 && threadIdx.x == 0) *ctl_out = cur;
         return;
     }
     unsigned long long best = 0;
-    for (int i = vb.tid; i < n_partial; i += vb.nthreads) best = partial[i] > best ? partial[i] : best;
+    for (int i = threadIdx.x; i < n_partial; i += (int)blockDim.x) best = partial[i] > best ? partial[i] : best;
     for (int o = 16; o > 0; o >>= 1) {
         const unsigned long long other = __shfl_xor_sync(0xffffffffu, best, o);
         best = other > best ? other : best;
     }
     if (lane == 0) s_best[warp] = best;
-    vb_sync(vb);
-    if (vb.tid == 0) {
-        for (int w = 1; w < (int)(vb.nthreads >> 5); ++w) best = s_best[w] > best ? s_best[w] : best;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        for (int w = 1; w < (int)(blockDim.x >> 5); ++w) best = s_best[w] > best ? s_best[w] : best;
         const int count = (int)(best >> 32);
         const bool stop = best == 0 || count < 1 || count < min_frequency || cur.n_tokens >= vocab_size ||
                           cur.n_merges >= max_merges || cur.err;
@@ -1117,7 +1077,7 @@ pick_scan_body(const VBlock& vb, ScanSmem& sm,
             next.has_delta = 1;
         }
         s_pick[0] = next.a; s_pick[1] = next.b; s_pick[3] = stop ? 1 : 0;
-        if (vb.bid == 0) {
+        if (blockIdx.x == 0) {
             *ctl_out = next;
             if (!stop) {
                 int* e = log + 4 * cur.n_merges;
@@ -1125,7 +1085,7 @@ pick_scan_body(const VBlock& vb, ScanSmem& sm,
             }
         }
     }
-    vb_sync(vb);
+    __syncthreads();
     if (s_pick[3]) return;
     const int a = s_pick[0], b = s_pick[1];
     // ---------------- scan
@@ -1145,8 +1105,8 @@ pick_scan_body(const VBlock& vb, ScanSmem& sm,
         }
     };
     if (!sig) {
-        for (long long base = (long long)vb.bid * vb.nthreads + (vb.tid & ~31); base < N;
-             base += (long long)vb.nblocks * vb.nthreads)
+        for (long long base = (long long)blockIdx.x * blockDim.x + (threadIdx.x & ~31u); base < N;
+             base += (long long)gridDim.x * blockDim.x)
             scan_warp(base + lane, base + lane < N, false);
         return;
     }
@@ -1155,20 +1115,20 @@ pick_scan_body(const VBlock& vb, ScanSmem& sm,
     const unsigned int* sig_col = sig + (long long)(sh >> 5) * n_stride;
     const unsigned int* sig_col2 = sig + (long long)(sh2 >> 5) * n_stride;
     const unsigned int sig_bit = 1u << (sh & 31u), sig_bit2 = 1u << (sh2 & 31u);
-    for (long long tile = (long long)vb.bid * tile_size; tile < N; tile += (long long)vb.nblocks * tile_size) {
-        if (vb.tid == 0) s_n = 0;
-        vb_sync(vb);
+    for (long long tile = (long long)blockIdx.x * tile_size; tile < N; tile += (long long)gridDim.x * tile_size) {
+        if (threadIdx.x == 0) s_n = 0;
+        __syncthreads();
         // all signature words of the tile first (up to 16 loads in flight per thread), then the ballots
         unsigned int pass_bits = 0;
 #pragma unroll
         for (int r = 0; r < kScanTile / 256; ++r) {
-            const int k = vb.tid + r * 256;
+            const int k = threadIdx.x + r * 256;
             const long long seq = tile + k;
             if (k < tile_size && seq < N && (__ldg(sig_col + seq) & sig_bit) && (__ldg(sig_col2 + seq) & sig_bit2))
                 pass_bits |= 1u << r;
         }
         for (int r = 0; r * 256 < tile_size; ++r) {
-            const int k = vb.tid + r * 256;
+            const int k = threadIdx.x + r * 256;
             const bool pass = (pass_bits >> r) & 1u;
             const unsigned int m = __ballot_sync(0xffffffffu, pass);
             if (m) {
@@ -1178,73 +1138,14 @@ pick_scan_body(const VBlock& vb, ScanSmem& sm,
                 if (pass) s_list[base + __popc(m & ((1u << lane) - 1u))] = k;
             }
         }
-        vb_sync(vb);
+        __syncthreads();
         const int n_pass = s_n;
-        for (int i0 = vb.tid & ~31; i0 < n_pass; i0 += vb.nthreads) {
+        for (int i0 = threadIdx.x & ~31u; i0 < n_pass; i0 += (int)blockDim.x) {
             const int i = i0 + lane;
             const bool valid = i < n_pass;
             scan_warp(valid ? tile + s_list[i] : 0, valid, DEEP);
         }
-        vb_sync(vb);
-    }
-}
-
-template <bool DEEP>
-__global__ void __launch_bounds__(256)
-bpe_pick_scan_kernel(const uint16_t* __restrict__ sym, const int* __restrict__ len, long long N, long long n_stride, int V,
-                     const BpeCtl* __restrict__ ctl_in, BpeCtl* __restrict__ ctl_out,
-                     const unsigned long long* __restrict__ partial, int n_partial, int* __restrict__ log,
-                     int vocab_size, int min_frequency, int max_merges, int* __restrict__ work_count,
-                     int* __restrict__ work_seq, int* __restrict__ work_q0, const unsigned int* __restrict__ sig,
-                     int tile_size) {
-    __shared__ ScanSmem sm;
-    pdl_wait();
-    pdl_launch();
-    pick_scan_body<DEEP>(real_block(), sm, sym, len, N, n_stride, V, ctl_in, ctl_out, partial, n_partial, log, vocab_size,
-                         min_frequency, max_merges, work_count, work_seq, work_q0, sig, tile_size);
-}
-
-// The whole merge loop in ONE cooperative kernel (opt-in, BEAST_B200_BPE_LOOP=persistent): the three phases of an
-// iteration are separated by grid barriers instead of kernel boundaries, and the host enqueues one launch per block of
-// up to 256 merges.  Slower than the PDL-chained launches on every size measured (see bpe_train_step).  One 1024-thread block per SM; the scan and rewrite phases
-// run as four 256-thread virtual blocks per block (VBlock), the code is the stand-alone kernels' code.
-struct LoopArgs {
-    uint16_t* sym; int* len; long long N, n_stride; int V;
-    int* hist; int* delta; BpeCtl* ctl; int* log; unsigned long long* partial;
-    int* work_count; int* work_seq; int* work_q0;
-    int vocab_size, min_frequency, max_merges;
-    unsigned int* sig; const int* weight; int tile_size, first_iter, iters;
-};
-template <bool DEEP>
-__global__ void __launch_bounds__(1024, 1)
-bpe_loop_kernel(const __grid_constant__ LoopArgs a, const __grid_constant__ BpePeersDev peers) {
-    extern __shared__ __align__(16) int s_dyn[];              // four private 4 x V delta blocks, then the rewrite staging
-    __shared__ unsigned long long s_best[32];
-    __shared__ ScanSmem s_scan[4];
-    uint16_t (*s_out)[8][kRewriteOut] = (uint16_t (*)[8][kRewriteOut])(s_dyn + (size_t)16 * a.V);
-    cooperative_groups::grid_group grid = cooperative_groups::this_grid();
-    const int sub = (int)(threadIdx.x >> 8);
-    VBlock vb;
-    vb.tid = (int)(threadIdx.x & 255); vb.bid = (int)blockIdx.x * 4 + sub; vb.nblocks = (int)gridDim.x * 4; vb.nthreads = 256;
-    vb.bar = 1 + sub;
-    int* s_delta = s_dyn + (size_t)sub * 4 * a.V;
-    for (int it = 0; it < a.iters; ++it) {
-        const int i = a.first_iter + it;
-        BpeCtl* cin = a.ctl + (i & 1);
-        BpeCtl* cout = a.ctl + ((i + 1) & 1);
-        iterate_body(a.hist, a.V, cin, a.delta, a.partial, a.work_count, peers, s_best);
-        grid.sync();
-        pick_scan_body<DEEP>(vb, s_scan[sub], a.sym, a.len, a.N, a.n_stride, a.V, cin, cout, a.partial, (int)gridDim.x, a.log,
-                             a.vocab_size, a.min_frequency, a.max_merges, a.work_count, a.work_seq, a.work_q0, a.sig, a.tile_size);
-        grid.sync();
-        if (cout->done) {                                     // uniform: every block reads the state block 0 wrote before the barrier
-            if (blockIdx.x == 0 && threadIdx.x == 0) *cin = *cout;       // both control blocks hold the final state
-            break;
-        }
-        if (a.N > 0)
-            rewrite_body(vb, s_delta, s_out[sub], a.sym, a.len, a.n_stride, 0, 0, 0, a.V, cout, a.work_count, a.work_seq, a.work_q0,
-                         a.delta, a.sig, a.weight);
-        grid.sync();
+        __syncthreads();
     }
 }
 
@@ -2201,8 +2102,7 @@ extern "C" int bpe_train_step(uint16_t* sym, int32_t* len, int64_t N, int64_t n_
     // ones are better off with two (measured: 65 k sequences 0.056 -> 0.053 s, 1.6 M sequences 0.214 -> 0.228 s)
     const bool deep_walk = N <= (1 << 19);
     BpeCtl* ctl2 = (BpeCtl*)ctl;
-    static int use_pdl = -1;
-    if (use_pdl < 0) { const char* e = getenv("BEAST_B200_BPE_NO_PDL"); use_pdl = (e && e[0] == '1') ? 0 : 1; }
+    // three PDL-chained launches per merge: one cooperative kernel with grid barriers was measured slower (DESIGN §9)
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
@@ -2210,41 +2110,9 @@ extern "C" int bpe_train_step(uint16_t* sym, int32_t* len, int64_t N, int64_t n_
         cudaLaunchConfig_t c;
         memset(&c, 0, sizeof(c));
         c.gridDim = dim3(g); c.blockDim = dim3(b); c.dynamicSmemBytes = sm; c.stream = st;
-        c.attrs = attr; c.numAttrs = use_pdl ? 1 : 0;
+        c.attrs = attr; c.numAttrs = 1;
         return c;
     };
-    // BEAST_B200_BPE_LOOP=persistent: the whole block of iterations in ONE cooperative kernel, grid barriers instead of
-    // kernel boundaries.  Measured SLOWER than the PDL-chained launches (200 k-sequence shard 62.6 vs 40.2 ms, 12 000
-    // pseudo-sequences 54.3 vs 31.3 ms: three grid barriers of a 148 x 1024-thread grid cost more than three
-    // programmatic launch boundaries), so it is opt-in; kept because it is the same device code and is tested.
-    const char* loop_env = getenv("BEAST_B200_BPE_LOOP");      // re-read per call: the tests run both forms in one process
-    const int loop_mode = (loop_env && loop_env[0] == 'p') ? 1 : 0;
-    const size_t loop_smem = (size_t)64 * V + (size_t)4 * 8 * kRewriteOut * sizeof(uint16_t);
-    if (loop_mode == 1 && loop_smem <= 176 * 1024) {
-        static size_t granted_ld[kMaxDevices] = {}, granted_lf[kMaxDevices] = {};
-        int rc2 = deep_walk ? opt_in_smem(bpe_loop_kernel<true>, loop_smem, granted_ld) : opt_in_smem(bpe_loop_kernel<false>, loop_smem, granted_lf);
-        int per_sm = 0, coop = 0, dev = 0;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, dev);
-        if (rc2 == BEAST_OK) {
-            if (deep_walk) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, bpe_loop_kernel<true>, 1024, loop_smem);
-            else cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, bpe_loop_kernel<false>, 1024, loop_smem);
-        }
-        if (rc2 == BEAST_OK && coop && per_sm >= 1) {
-            LoopArgs la;
-            la.sym = sym; la.len = len; la.N = N; la.n_stride = n_stride; la.V = V;
-            la.hist = hist; la.delta = delta; la.ctl = ctl2; la.log = log; la.partial = (unsigned long long*)result;
-            la.work_count = work_count; la.work_seq = work_seq; la.work_q0 = work_q0;
-            la.vocab_size = vocab_size; la.min_frequency = min_frequency; la.max_merges = max_merges;
-            la.sig = sig; la.weight = weight; la.tile_size = (int)tile; la.first_iter = first_iter; la.iters = iters < 1 ? 1 : iters;
-            void* args[2] = {&la, &peers};
-            const void* fn = deep_walk ? (const void*)bpe_loop_kernel<true> : (const void*)bpe_loop_kernel<false>;
-            cudaError_t e = cudaLaunchCooperativeKernel(fn, dim3((unsigned)n_part), dim3(1024), args, loop_smem, st);
-            if (e != cudaSuccess) return (int)e;
-            count_launch();
-            return BEAST_OK;
-        }
-    }
     const unsigned long long* partial = (const unsigned long long*)result;
     const uint16_t* csym = sym;
     const int32_t* clen = len;

@@ -488,10 +488,9 @@ def test_word_dedup_gives_the_same_table(kind):
 
 
 @pytest.mark.parametrize("kind", ["normal", "repetitive", "bins1000"])
-def test_persistent_loop_kernel_equals_the_launch_chain(kind, monkeypatch):
-    """The merge loop has two forms: three launches per merge chained with programmatic dependent launch, and ONE
-    cooperative kernel per block of merges with grid barriers between the phases (small corpora).  Same device code
-    (virtual blocks); both must log exactly the same merges, with and without word de-duplication."""
+def test_launch_chain_logs_the_oracle_merges(kind):
+    """The merge loop runs three launches per merge chained with programmatic dependent launch, and never syncs with
+    the host.  It must log exactly the oracle's merges, with and without word de-duplication."""
     from beast_tokenizer_b200 import FIGBPE
     rng = np.random.default_rng(41)
     if kind == "normal":
@@ -503,11 +502,9 @@ def test_persistent_loop_kernel_equals_the_launch_chain(kind, monkeypatch):
         bins, vocab = np.clip(rng.normal(500, 120, (5000, 100)).round(), 0, 999).astype(np.int64), 2200
     dev_bins = torch.from_numpy(bins).cuda()
     out = {}
-    for mode in ("launches", "persistent"):
-        monkeypatch.setenv("BEAST_B200_BPE_LOOP", mode)
-        for dedup in (True, False):
-            st = FIGBPE(vocab_size=vocab, show_progress=False, dedup=dedup).fit_from_bins(dev_bins)
-            out[(mode, dedup)] = (st.tokenizer.merges_txt(), st.tokenizer.vocab_json())
+    for dedup in (True, False):
+        st = FIGBPE(vocab_size=vocab, show_progress=False, dedup=dedup).fit_from_bins(dev_bins)
+        out[dedup] = (st.tokenizer.merges_txt(), st.tokenizer.vocab_json())
     o = OracleBPE.train(bins, vocab)
     for key, val in out.items():
         assert val == (o.merges_txt(), o.vocab_json()), key
