@@ -87,6 +87,11 @@ _SIGNATURES = {
                                       C.c_void_p]),
     "beast_fit_times_backward_f32": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, c_f32p, c_f32p, c_f32p, c_f32p,
                                                c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, C.c_void_p]),
+    "beast_fit_masked_f32": (C.c_int, [C.c_void_p, c_f32p, C.c_int64, C.c_int32, c_f32p, C.c_int64, C.c_void_p,
+                                       C.c_int32, c_f32p, c_f32p, c_f32p, C.c_void_p]),
+    "beast_fit_masked_backward_f32": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, c_f32p, C.c_int64, C.c_void_p,
+                                                C.c_int32, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p,
+                                                c_f32p, C.c_void_p]),
     "beast_fit_minmax_f32":(C.c_int, [C.c_void_p, c_f32p, C.c_int64, c_f32p, c_f32p, C.c_int32, C.c_void_p]),
     "beast_fit_minmax_workspace_bytes": (C.c_int64, [C.c_void_p]),
     "beast_fit_minmax_ws_f32": (C.c_int, [C.c_void_p, c_f32p, C.c_int64, c_f32p, c_f32p, C.c_int32, C.c_void_p, C.c_int64,

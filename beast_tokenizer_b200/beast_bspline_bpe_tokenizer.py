@@ -311,16 +311,19 @@ class BEASTBsplineBPETokenizer(BEASTBsplineTokenizer):
 
     # ------------------------------------------------------------------ BEAST overridden
     def encode(self, trajs: torch.Tensor, update_bounds: bool = False, *, return_mp_tokens: bool = False,
-               times: Optional[torch.Tensor] = None) -> tuple:
-        mp_tokens, params = super().encode(trajs, update_bounds=update_bounds, respect_llm_vocab_size=False, times=times)
+               times: Optional[torch.Tensor] = None, mask: Optional[torch.Tensor] = None) -> tuple:
+        mp_tokens, params = super().encode(trajs, update_bounds=update_bounds, respect_llm_vocab_size=False, times=times,
+                                           mask=mask)
         bpe_tokens = self._discrete_to_bpe(mp_tokens)
         if return_mp_tokens:
             return bpe_tokens, params, mp_tokens
         return bpe_tokens, params
 
-    def encode_csr(self, trajs: torch.Tensor, update_bounds: bool = False, *, times: Optional[torch.Tensor] = None):
+    def encode_csr(self, trajs: torch.Tensor, update_bounds: bool = False, *, times: Optional[torch.Tensor] = None,
+                   mask: Optional[torch.Tensor] = None):
         """Device-resident variant of `encode`: (flat ids int32, offsets int64 [B+1], params_dict)."""
-        mp_tokens, params = super().encode(trajs, update_bounds=update_bounds, respect_llm_vocab_size=False, times=times)
+        mp_tokens, params = super().encode(trajs, update_bounds=update_bounds, respect_llm_vocab_size=False, times=times,
+                                           mask=mask)
         flat, offsets = self._discrete_to_bpe_csr(mp_tokens)
         return flat, offsets, params
 
@@ -329,10 +332,10 @@ class BEASTBsplineBPETokenizer(BEASTBsplineTokenizer):
         return super().decode(discrete, respect_llm_vocab_size=respect_llm_vocab_size)
 
     def encode_to_mp_tokens(self, trajs: torch.Tensor, update_bounds: bool = False, *,
-                            times: Optional[torch.Tensor] = None) -> tuple:
-        """Expose the underlying MP-token encoding without BPE.  `times` [B, T]: per-row timestamps, as in
-        BEASTBsplineTokenizer.encode."""
-        return super().encode(trajs, update_bounds=update_bounds, respect_llm_vocab_size=False, times=times)
+                            times: Optional[torch.Tensor] = None, mask: Optional[torch.Tensor] = None) -> tuple:
+        """Expose the underlying MP-token encoding without BPE.  `times` [B, T]: per-row timestamps, `mask` [B, T]:
+        the samples to fit (True = fitted, i.e. LeRobot's ~action_is_pad), as in BEASTBsplineTokenizer.encode."""
+        return super().encode(trajs, update_bounds=update_bounds, respect_llm_vocab_size=False, times=times, mask=mask)
 
     def bpe_to_mp_tokens(self, tokens: Iterable[TokenLike]) -> torch.Tensor:
         return self._bpe_to_discrete(tokens)

@@ -18,6 +18,8 @@ drop a NaN where torch.min / torch.clamp would propagate it.  Entry points:
     encode_continuous backward (autograd)         -> beast_fit_backward_f32
     the fits above with times=[B, T]              -> beast_fit_times_f32 (+ quantize / normalize / minmax);
                                                      backward beast_fit_times_backward_f32
+    the fits above with mask=[B, T]               -> beast_fit_masked_f32 (times None: after K1, partial rows only);
+                                                     backward beast_fit_masked_backward_f32
     update_weights_bounds(_per_batch)             -> beast_minmax_f32 + beast_bounds_expand_f32
     fit_parameters                                -> beast_encode_f32 + beast_colselect_f32
 
@@ -53,6 +55,8 @@ class _Plan:
 
         self._keep = [consts.proj_joint, consts.proj_grip, consts.phi_joint, consts.phi_grip,
                       consts.knots_joint, consts.knots_grip]
+        self._times_dev = None
+        self._joint_dev = None
         slots = (C.c_int32 * consts.num_dof)(*consts.slot_to_dof)
         desc = _lib.PlanDesc(
             seq_len=consts.seq_len, num_dof=consts.num_dof, num_basis=consts.num_basis,
@@ -68,6 +72,19 @@ class _Plan:
         self.handle = handle
         self._lib = lib
         self._workspaces = {}
+
+    def device_times(self) -> torch.Tensor:
+        """The plan's times [T] on its device (the masked fit's shared grid), copied once."""
+        if self._times_dev is None:
+            self._times_dev = self.consts.times.to(self.device, torch.float32).contiguous()
+        return self._times_dev
+
+    def joint_index(self) -> torch.Tensor:
+        """The joint DoF indices as int64 [n_joint] on the plan's device, copied once (a host copy per call could not be
+        captured in a CUDA graph)."""
+        if self._joint_dev is None:
+            self._joint_dev = torch.as_tensor(self.consts.joint_indices, dtype=torch.int64, device=self.device)
+        return self._joint_dev
 
     def minmax_workspace(self) -> torch.Tensor:
         """Zero-initialised scratch of beast_fit_minmax_ws_f32, one per (plan, stream)."""
@@ -214,17 +231,23 @@ class _FitFn(torch.autograd.Function):
 
 
 class _FitTimesFn(torch.autograd.Function):
-    """encode_continuous(times=[B, T])'s fit and normalisation as an autograd node: forward = `fit(x, bc, bias)` (the
-    beast_fit_times_f32 launch, the optional bounds expansion and beast_normalize_f32) -> (normalised, params, (w_min,
-    w_max) snapshot), backward = one beast_fit_times_backward_f32 launch -> gradients of x, of the pinned points bc and
-    of bias (both torch ops on x's boundary samples, so their gradients chain back to x).  times and the bounds are
-    constants; an output the loss does not use arrives as None and is passed to the kernel as NULL."""
+    """encode_continuous(times=[B, T] and / or mask=[B, T])'s fit and normalisation as an autograd node: forward =
+    `fit(x, bc, bias)` (the fit launches, the optional bounds expansion and beast_normalize_f32) -> (normalised, params,
+    (w_min, w_max) snapshot), backward -> gradients of x, of the pinned points bc and of bias (both torch ops on x's
+    boundary samples, so their gradients chain back to x):
+      times, no mask:  one beast_fit_times_backward_f32 launch;
+      times and mask:  one beast_fit_masked_backward_f32 launch;
+      mask, no times:  beast_fit_backward_f32 over every row, then beast_fit_masked_backward_f32 over the rows with a
+                       masked sample (partial_only); grad_bc / grad_bias are 0 on the other rows, whose boundary
+                       dependence the shared projector already holds.
+    times, mask (uint8 [B, T]) and the bounds are constants; an output the loss does not use arrives as None and is
+    passed to the kernel as NULL."""
 
     @staticmethod
-    def forward(ctx, fit, plan, times, x, bc, bias):
+    def forward(ctx, fit, plan, times, mask, x, bc, bias):
         ctx.set_materialize_grads(False)
         normalised, params, bounds = fit(x, bc, bias)
-        ctx.plan, ctx.times, ctx.bounds = plan, times, bounds
+        ctx.plan, ctx.times, ctx.mask, ctx.bounds = plan, times, mask, bounds
         ctx.has_bc, ctx.has_bias = bc is not None, bias is not None
         ctx.save_for_backward(params)
         return normalised, params
@@ -233,26 +256,51 @@ class _FitTimesFn(torch.autograd.Function):
     @once_differentiable
     def backward(ctx, grad_norm, grad_params):
         if grad_norm is None and grad_params is None:
-            return None, None, None, None, None, None
-        plan, times = ctx.plan, ctx.times
+            return None, None, None, None, None, None, None
+        plan, times, mask = ctx.plan, ctx.times, ctx.mask
         (params,), (lo, hi) = ctx.saved_tensors, ctx.bounds
         dev = plan.device
         c = plan.consts
         grad_norm, grad_params = (None if g is None else g.to(dev, torch.float32).contiguous()
                                   for g in (grad_norm, grad_params))
-        B, T = times.shape
+        B, T = times.shape if times is not None else mask.shape
         n_joint = len(c.joint_indices)
         nbc = c.init_order + c.end_order
+        shared = times is None          # mask on the tokenizer's times: full rows keep the shared-projector adjoint
+        alloc = torch.zeros if shared else torch.empty
         grad_traj = torch.empty((B, T, c.num_dof), device=dev, dtype=torch.float32)
-        grad_bc = torch.empty((B, n_joint, nbc), device=dev, dtype=torch.float32) if ctx.has_bc else None
-        grad_bias = torch.empty((B, n_joint), device=dev, dtype=torch.float32) if ctx.has_bias else None
+        grad_bc = alloc((B, n_joint, nbc), device=dev, dtype=torch.float32) if ctx.has_bc else None
+        grad_bias = alloc((B, n_joint), device=dev, dtype=torch.float32) if ctx.has_bias else None
         if B > 0:                       # empty tensors carry no data pointer
+            g = (_lib.ptr(grad_norm), _lib.ptr(grad_params), _lib.ptr(params), _lib.ptr(lo), _lib.ptr(hi),
+                 _lib.ptr(grad_traj))
             with torch.cuda.device(dev):
-                _lib.check(plan._lib.beast_fit_times_backward_f32(
-                    plan.handle, B, T, _lib.ptr(times), _lib.ptr(grad_norm), _lib.ptr(grad_params), _lib.ptr(params),
-                    _lib.ptr(lo), _lib.ptr(hi), _lib.ptr(grad_traj), _lib.ptr(grad_bc), _lib.ptr(grad_bias),
-                    _lib.stream_ptr(dev)), "beast_fit_times_backward_f32")
-        return None, None, None, grad_traj, grad_bc, grad_bias
+                if mask is None:
+                    _lib.check(plan._lib.beast_fit_times_backward_f32(
+                        plan.handle, B, T, _lib.ptr(times), *g, _lib.ptr(grad_bc), _lib.ptr(grad_bias),
+                        _lib.stream_ptr(dev)), "beast_fit_times_backward_f32")
+                else:
+                    if shared:
+                        _lib.check(plan._lib.beast_fit_backward_f32(plan.handle, B, *g, _lib.stream_ptr(dev)),
+                                   "beast_fit_backward_f32")
+                    t = plan.device_times() if shared else times
+                    _lib.check(plan._lib.beast_fit_masked_backward_f32(
+                        plan.handle, B, T, _lib.ptr(t), 0 if shared else T, _lib.ptr(mask), int(shared), *g,
+                        _lib.ptr(grad_bc), _lib.ptr(grad_bias), _lib.stream_ptr(dev)), "beast_fit_masked_backward_f32")
+        return None, None, None, None, grad_traj, grad_bc, grad_bias
+
+
+def boundary_sample_indices(mask: torch.Tensor):
+    """(i0, i1, im2, im1), each int64 [B]: the first, second, second-to-last and last valid sample of every row of the
+    bool mask [B, T] — the samples the condition orders read on the compacted row.  Torch ops only (no host
+    synchronisation).  A row with fewer than two valid samples gets indices of no meaning, still clamped to [0, T)."""
+    B, T = mask.shape
+    ar = torch.arange(T, device=mask.device).expand(B, T)
+    i0 = torch.where(mask, ar, T).amin(1, keepdim=True)
+    i1 = torch.where(mask & (ar > i0), ar, T).amin(1, keepdim=True)
+    im1 = torch.where(mask, ar, -1).amax(1, keepdim=True)
+    im2 = torch.where(mask & (ar < im1), ar, -1).amax(1, keepdim=True)
+    return tuple(i.squeeze(1).clamp(0, T - 1) for i in (i0, i1, im2, im1))
 
 
 class BEASTBsplineTokenizer(TokenizerBase):
@@ -388,11 +436,13 @@ class BEASTBsplineTokenizer(TokenizerBase):
             trajs = trajs[..., :self.num_dof]
         return trajs.contiguous()
 
-    def _fit(self, trajs, want_tokens, offset=0, bounds=None, times=None):
+    def _fit(self, trajs, want_tokens, offset=0, bounds=None, times=None, mask=None):
         """One K1 launch: (tokens | None, unclamped params).  With per-row times [B, T]: beast_fit_times_f32, then
-        beast_quantize_f32 for the tokens."""
+        beast_quantize_f32 for the tokens.  With a mask [B, T]: see _fit_times / _fit_masked."""
         if times is not None:
-            return self._fit_times(trajs, times, want_tokens, offset, bounds)
+            return self._fit_times(trajs, times, want_tokens, offset, bounds, mask)
+        if mask is not None:
+            return self._fit_masked(trajs, mask, want_tokens, offset, bounds)
         plan = self._plan()
         dev = plan.device
         x = self._prep_trajs(trajs, dev)
@@ -419,26 +469,73 @@ class BEASTBsplineTokenizer(TokenizerBase):
             raise AssertionError("init_cond_order / end_cond_order != 0: a fit needs at least 2 samples per row")
         return x, t
 
-    def _fit_times_launch(self, plan, x, t, bc, bias):
-        """One beast_fit_times_f32 launch: unclamped params [B, D*nb]."""
+    def _prep_mask(self, mask, dev, B, T):
+        """mask [B, T] (bool, or integer 0 / 1; any device) -> contiguous bool [B, T] on `dev`, True = fitted.  No host
+        synchronisation: the values are not inspected (a non-zero integer counts as True)."""
+        m = torch.as_tensor(mask)
+        if m.dtype != torch.bool and (m.dtype.is_floating_point or m.dtype.is_complex):
+            raise TypeError(f"mask must be bool or integer, got {m.dtype}")
+        if m.dim() != 2 or tuple(m.shape) != (B, T):
+            raise AssertionError(f"mask must be [batch, T] = [{B}, {T}], got {tuple(m.shape)}")
+        m = m.to(dev)
+        return (m if m.dtype == torch.bool else m != 0).contiguous()
+
+    def _fit_times_launch(self, plan, x, t, bc, bias, mask=None):
+        """One beast_fit_times_f32 (beast_fit_masked_f32 with a mask) launch: unclamped params [B, D*nb]."""
         dev = plan.device
         B, T = t.shape
         params = torch.empty((B, self.num_dof * self.num_basis), device=dev, dtype=torch.float32)
         if B > 0:                       # empty tensors carry no data pointer
             with torch.cuda.device(dev):
-                _lib.check(plan._lib.beast_fit_times_f32(plan.handle, _lib.ptr(x), B, T, _lib.ptr(t), _lib.ptr(bc),
-                                                         _lib.ptr(bias), _lib.ptr(params), _lib.stream_ptr(dev)),
-                           "beast_fit_times_f32")
+                if mask is None:
+                    _lib.check(plan._lib.beast_fit_times_f32(plan.handle, _lib.ptr(x), B, T, _lib.ptr(t), _lib.ptr(bc),
+                                                             _lib.ptr(bias), _lib.ptr(params), _lib.stream_ptr(dev)),
+                               "beast_fit_times_f32")
+                else:
+                    _lib.check(plan._lib.beast_fit_masked_f32(plan.handle, _lib.ptr(x), B, T, _lib.ptr(t), T,
+                                                              _lib.ptr(mask), 0, _lib.ptr(bc), _lib.ptr(bias),
+                                                              _lib.ptr(params), _lib.stream_ptr(dev)),
+                               "beast_fit_masked_f32")
         return params
 
-    def _fit_times(self, trajs, times, want_tokens, offset=0, bounds=None):
+    def _fit_shared_masked(self, plan, x, mask, bc, bias):
+        """The masked fit on the tokenizer's times: K1 over every row (params only), then beast_fit_masked_f32 with
+        partial_only over the same buffer, which refits the rows holding a masked sample and leaves the others as K1
+        wrote them.  Unclamped params [B, D*nb]."""
+        dev = plan.device
+        B, T = mask.shape
+        params = torch.empty((B, self.num_dof * self.num_basis), device=dev, dtype=torch.float32)
+        if B > 0:
+            with torch.cuda.device(dev):
+                _lib.check(plan._lib.beast_encode_f32(plan.handle, _lib.ptr(x), B, None, None, 0, _lib.ptr(params),
+                                                      None, _lib.stream_ptr(dev)), "beast_encode_f32")
+                _lib.check(plan._lib.beast_fit_masked_f32(plan.handle, _lib.ptr(x), B, T,
+                                                          _lib.ptr(plan.device_times()), 0, _lib.ptr(mask), 1,
+                                                          _lib.ptr(bc), _lib.ptr(bias), _lib.ptr(params),
+                                                          _lib.stream_ptr(dev)), "beast_fit_masked_f32")
+        return params
+
+    def _fit_times(self, trajs, times, want_tokens, offset=0, bounds=None, mask=None):
         plan = self._plan()
         dev = plan.device
         x, t = self._prep_times(trajs, times, dev)
-        st = self._boundary_state(x, plan, t) if self._has_conditions else None
+        m = None if mask is None else self._prep_mask(mask, dev, *t.shape)
+        st = self._boundary_state(x, plan, t, m) if self._has_conditions else None
         if st is not None:
             self._boundary = st
-        params = self._fit_times_launch(plan, x, t, *((st["bc"], st["bias"]) if st is not None else (None, None)))
+        params = self._fit_times_launch(plan, x, t, *((st["bc"], st["bias"]) if st is not None else (None, None)), m)
+        tokens = self._quantize(params, offset, bounds) if want_tokens else None
+        return tokens, params
+
+    def _fit_masked(self, trajs, mask, want_tokens, offset=0, bounds=None):
+        plan = self._plan()
+        dev = plan.device
+        x = self._prep_trajs(trajs, dev)
+        m = self._prep_mask(mask, dev, x.shape[0], x.shape[1])
+        st = self._boundary_state(x, plan, None, m) if self._has_conditions else None
+        if st is not None:
+            self._boundary = st
+        params = self._fit_shared_masked(plan, x, m, *((st["bc"], st["bias"]) if st is not None else (None, None)))
         tokens = self._quantize(params, offset, bounds) if want_tokens else None
         return tokens, params
 
@@ -454,20 +551,29 @@ class BEASTBsplineTokenizer(TokenizerBase):
             return
         self._boundary = self._boundary_state(x, plan)
 
-    def _boundary_state(self, x, plan, times=None):
+    def _boundary_state(self, x, plan, times=None, mask=None):
         """The boundary state of `x` (torch ops: attached to the graph of `x` under grad mode).  `times` [B, T]: each
-        row's own step dt_b = times[b, 1] - times[b, 0]; None: the tokenizer's times."""
+        row's own step dt_b = times[b, 1] - times[b, 0]; None: the tokenizer's times.  `mask` [B, T] (bool): the state
+        of the compacted rows — samples i0, i1, im2, im1 of boundary_sample_indices and dt_b = t[i1] - t[i0] — gathered
+        with torch ops (no host synchronisation)."""
         io, eo, p = self.init_cond_order, self.end_cond_order, self.degree_p
         c = plan.consts
         nc = self.num_basis + io + eo
-        if times is None:
-            t = c.times
-            inv_dt = float(torch.tensor(1.0) / (t[1] - t[0]))
+        ji = plan.joint_index()
+        if mask is not None:
+            idx = torch.stack(boundary_sample_indices(mask), dim=1)                    # [B, 4]
+            sel = torch.gather(x, 1, idx.unsqueeze(2).expand(-1, -1, x.shape[2]))       # [B, 4, D]
+            y0, y1, ym2, ym1 = (sel[:, k, :].index_select(1, ji) for k in range(4))
+            t01 = (torch.gather(times, 1, idx[:, :2]) if times is not None else plan.device_times()[idx[:, :2]])
+            inv_dt = (1.0 / (t01[:, 1] - t01[:, 0])).unsqueeze(1)
         else:
-            inv_dt = (1.0 / (times[:, 1] - times[:, 0])).unsqueeze(1)
+            if times is None:
+                t = c.times
+                inv_dt = float(torch.tensor(1.0) / (t[1] - t[0]))
+            else:
+                inv_dt = (1.0 / (times[:, 1] - times[:, 0])).unsqueeze(1)
+            y0, y1, ym2, ym1 = (x[:, i, :].index_select(1, ji) for i in (0, 1, -2, -1))
         tau = c.tau
-        ji = torch.as_tensor(self.joint_indices, device=x.device)
-        y0, y1, ym2, ym1 = (x[:, i, :].index_select(1, ji) for i in (0, 1, -2, -1))
         st = {"init_pos": None, "init_vel": None, "end_pos": None, "end_vel": None}
         parts = []
         if io != 0:
@@ -711,22 +817,24 @@ class BEASTBsplineTokenizer(TokenizerBase):
 
     # ------------------------------------------------------------------ utils
     @torch.no_grad()
-    def compute_weights(self, demos, *, times=None):
+    def compute_weights(self, demos, *, times=None, mask=None):
         """Unclamped spline coefficients [B, D*nb] '(d t)', joints first (reference :344-360).  `times` [B, T]: fit
-        each row on its own timestamps (T may differ from seq_len; see encode)."""
-        return self._fit(demos, want_tokens=False, times=times)[1]
+        each row on its own timestamps (T may differ from seq_len; see encode).  `mask` [B, T]: fit only the samples
+        where it is True (see encode)."""
+        return self._fit(demos, want_tokens=False, times=times, mask=mask)[1]
 
     @torch.no_grad()
-    def update_weights_bounds(self, demos, process_group=None, *, times=None):
+    def update_weights_bounds(self, demos, process_group=None, *, times=None, mask=None):
         """Global per-column min / max of the coefficients (reference :362-378): one fused launch,
         the coefficients are reduced in registers and never written.  Sharded (set_process_group, or
         process_group= here; every rank passes its shard): one MIN and one MAX all-reduce of the D*nb vectors.
-        `times` [B, T]: the coefficients of the per-row fit (see encode), then beast_minmax_f32."""
+        `times` [B, T] and / or `mask` [B, T]: the coefficients of that fit (see encode), written, then
+        beast_minmax_f32."""
         plan = self._plan()
         dev = plan.device
         n = self.num_dof * self.num_basis
-        if times is not None:
-            return self._update_weights_bounds_times(plan, demos, times, n, process_group)
+        if times is not None or mask is not None:
+            return self._update_weights_bounds_fitted(plan, demos, times, mask, n, process_group)
         x = self._prep_trajs(demos, dev)
         # one launch, results written straight into the w_min / w_max buffers when they live on this device
         direct = (self.w_min.device == dev and self.w_max.device == dev and self.w_min.dtype == torch.float32
@@ -744,9 +852,9 @@ class BEASTBsplineTokenizer(TokenizerBase):
             self.w_min.copy_(lo.to(self.w_min.device))
             self.w_max.copy_(hi.to(self.w_max.device))
 
-    def _update_weights_bounds_times(self, plan, demos, times, n, process_group):
+    def _update_weights_bounds_fitted(self, plan, demos, times, mask, n, process_group):
         dev = plan.device
-        _, params = self._fit_times(demos, times, want_tokens=False)
+        _, params = self._fit(demos, want_tokens=False, times=times, mask=mask)
         direct = (self.w_min.device == dev and self.w_max.device == dev and self.w_min.dtype == torch.float32
                   and self.w_max.dtype == torch.float32 and self.w_min.is_contiguous() and self.w_max.is_contiguous())
         lo = self.w_min if direct else torch.empty(n, device=dev, dtype=torch.float32)
@@ -797,7 +905,7 @@ class BEASTBsplineTokenizer(TokenizerBase):
 
     # ------------------------------------------------------------------ encoding
     @torch.no_grad()
-    def encode(self, trajs, update_bounds=False, *, respect_llm_vocab_size=True, times=None):
+    def encode(self, trajs, update_bounds=False, *, respect_llm_vocab_size=True, times=None, mask=None):
         """trajs [B, T, D] -> (tokens int64 [B, nb*D] '(t d)', params_dict) — reference :399-428.
 
         `times` [B, T] (any device, converted to fp32): fit every row on its own timestamps, the reference's
@@ -805,15 +913,25 @@ class BEASTBsplineTokenizer(TokenizerBase):
         tau, 0, 1), as reconstruct_traj(times=...) evaluates it).  T may differ from seq_len (same for every row; >= 2
         with condition orders, whose boundary velocity uses each row's dt_b = times[b, 1] - times[b, 0]); times need
         not be sorted and are clamped to [0, duration].  NaN and dt_b = 0 are not treated specially.  A basis function
-        with no sample in its support gets coefficient 0.  None: the tokenizer's own times (the shared projector)."""
+        with no sample in its support gets coefficient 0.  None: the tokenizer's own times (the shared projector).
+
+        `mask` [B, T] (bool or integer 0 / 1, any device; T = seq_len, or times.shape[1]): fit only the samples where
+        it is True, e.g. padded chunk ends or dropped frames — LeRobot's `action_is_pad` is `~mask`.  Row b is fitted
+        exactly as the per-row fit fits y[b, mask[b]] on times[b, mask[b]] (the tokenizer's times when `times` is
+        None); masked samples are never read, so NaN or inf padding cannot reach any output.  Condition orders use the
+        first, second, second-to-last and last valid samples, dt_b from the first two.  A row whose mask is all True
+        is bit-identical to the call without a mask; a row without a valid sample gets coefficients 0 (no condition
+        orders); with condition orders a row with fewer than 2 valid samples is not treated specially.  With `times`
+        None the shared projector (K1) fits every row and the rows with a masked sample are then refitted; no host
+        synchronisation either way."""
         offset = 0
         if respect_llm_vocab_size and self.llm_vocab_size is not None:
             offset = self._llm_vocab_offset()
         if not update_bounds:
-            tokens, params = self._fit(trajs, want_tokens=True, offset=offset, times=times)
+            tokens, params = self._fit(trajs, want_tokens=True, offset=offset, times=times, mask=mask)
             return tokens, self._params_dict(params)
         # bounds move before quantisation: fit, expand, then the exact quantiser on the coefficients
-        _, params = self._fit(trajs, want_tokens=False, times=times)
+        _, params = self._fit(trajs, want_tokens=False, times=times, mask=mask)
         self.update_weights_bounds_per_batch(params)
         tokens = self._quantize(params, offset)
         return tokens, self._params_dict(params)
@@ -830,7 +948,7 @@ class BEASTBsplineTokenizer(TokenizerBase):
                                                     _lib.stream_ptr(dev)), "beast_quantize_f32")
         return tokens
 
-    def encode_continuous(self, trajs, update_bounds=False, *, times=None):
+    def encode_continuous(self, trajs, update_bounds=False, *, times=None, mask=None):
         """Normalised [-1, 1] coefficients in '(t d)' order (reference :430-450).
 
         Differentiable with respect to `trajs` when `trajs` requires grad under grad mode: the backward of `normalised`
@@ -841,15 +959,19 @@ class BEASTBsplineTokenizer(TokenizerBase):
         for later reconstructs is detached.  Otherwise the call runs under no_grad, as before.
 
         `times` [B, T]: the per-row fit of encode(times=...); its backward is beast_fit_times_backward_f32, with the
-        gradients of the pinned boundary points and of the bias chained back to the trajectories."""
+        gradients of the pinned boundary points and of the bias chained back to the trajectories.
+
+        `mask` [B, T]: the masked fit of encode(mask=...); its backward is beast_fit_masked_backward_f32 (after
+        beast_fit_backward_f32 over every row when `times` is None).  Masked samples get a gradient of exactly 0; the
+        mask is a constant.  Rows whose mask is all True get the gradients of the call without a mask."""
         if not (torch.is_grad_enabled() and isinstance(trajs, torch.Tensor) and trajs.requires_grad):
             with torch.no_grad():
-                _, params = self._fit(trajs, want_tokens=False, times=times)
+                _, params = self._fit(trajs, want_tokens=False, times=times, mask=mask)
                 if update_bounds:
                     self.update_weights_bounds_per_batch(params)
                 return self._normalize(params), self._params_dict(params)
-        if times is not None:
-            return self._encode_continuous_times(trajs, times, update_bounds)
+        if times is not None or mask is not None:
+            return self._encode_continuous_times(trajs, times, mask, update_bounds)
         plan = self._plan()
         x = self._prep_trajs(trajs, plan.device)          # differentiable: .to() / slicing / .contiguous()
 
@@ -866,24 +988,31 @@ class BEASTBsplineTokenizer(TokenizerBase):
         st = self._boundary_state(x, plan) if self._has_conditions else None
         return normalised, self._params_dict(params, st)
 
-    def _encode_continuous_times(self, trajs, times, update_bounds):
+    def _encode_continuous_times(self, trajs, times, mask, update_bounds):
         plan = self._plan()
         dev = plan.device
-        x, t = self._prep_times(trajs, times, dev)         # differentiable: .to() / slicing / .contiguous()
-        st = self._boundary_state(x, plan, t) if self._has_conditions else None
+        if times is not None:                               # differentiable: .to() / slicing / .contiguous()
+            x, t = self._prep_times(trajs, times, dev)
+        else:
+            x, t = self._prep_trajs(trajs, dev), None
+        m = None if mask is None else self._prep_mask(mask, dev, x.shape[0], x.shape[1])
+        st = self._boundary_state(x, plan, t, m) if self._has_conditions else None
         bc, bias = (st["bc"], st["bias"]) if st is not None else (None, None)
 
         def fit(x, bc, bias):
             if st is not None:                              # kept for later reconstructs, detached
                 self._boundary = {k: None if v is None else v.detach() for k, v in st.items()}
-            params = self._fit_times_launch(plan, x, t, bc, bias)
+            if t is None:
+                params = self._fit_shared_masked(plan, x, m, bc, bias)
+            else:
+                params = self._fit_times_launch(plan, x, t, bc, bias, m)
             if update_bounds:
                 self.update_weights_bounds_per_batch(params)
             normalised = self._normalize(params)
             lo, hi = self._bounds(dev)
             return normalised, params, (lo.clone(), hi.clone())
 
-        normalised, params = _FitTimesFn.apply(fit, plan, t, x, bc, bias)
+        normalised, params = _FitTimesFn.apply(fit, plan, t, None if m is None else m.view(torch.uint8), x, bc, bias)
         return normalised, self._params_dict(params, st)
 
     def _normalize(self, params):

@@ -15,6 +15,14 @@
 // side has one owner lane that adds the chunk's terms in t ascending order, so a row's result depends on nothing but
 // the row.  Gram, rhs, factorisation and solves are fp64 (products of fp32 values are exact); each output is rounded
 // once to fp32.  No atomics.
+//
+// Masked fit (beast_fit_masked_f32 / _backward_f32, the kMasked instantiations): a byte mask [B, T] marks the samples
+// that are fitted.  Each chunk of 32 raw samples stages only its valid samples, compacted in t order (a ballot and a
+// prefix popcount), so the owners see exactly the samples, values and order the unmasked kernel sees on the compacted
+// row y[b, mask[b]] on times[b, mask[b]]: the results are bit-identical to it.  A masked sample's time and trajectory
+// value are never loaded, it adds no term anywhere, and its grad_traj is written as 0.  The times may be one grid [T]
+// for every row (row stride 0).  partial_only: a warp first reads its row's mask and leaves a row whose samples are all
+// valid untouched (its outputs stay what another launch wrote there).
 #include <climits>
 #include <initializer_list>
 #include "common.cuh"
@@ -34,7 +42,7 @@ struct FitTimesArgs {
     const float* knots_j;        // [nc + p + 1]
     const float* knots_g;        // [nb + 1] or nullptr
     const int* slot_to_dof;
-    const float* times;          // [B, T]
+    const float* times;          // [B, T] (row stride times_stride: T, or 0 for one grid [T])
     // forward
     const float* traj;           // [B, T, D]
     const float* bc;             // [B, n_joint, ico + eco] (pinned points only)
@@ -50,6 +58,10 @@ struct FitTimesArgs {
     float* grad_bc;              // [B, n_joint, ico + eco] (pinned points only)
     float* grad_bias;            // [B, n_joint] or nullptr
     size_t warp_bytes;           // shared memory per warp
+    // masked kernels only
+    const uint8_t* mask;         // [B, T] non-zero = fitted
+    long long times_stride;
+    int partial_only;            // skip rows whose mask is all non-zero
 };
 
 // Per-warp shared memory: fp64 arrays first (8-byte aligned), then fp32 / int.
@@ -63,15 +75,16 @@ struct FitTimesWarp {
     float* v;        // [chunk][p+2] non-zero joint basis values of each sample (+ a zero sentinel)
     int* f;          // [chunk] first joint column (of nc) of each sample's values
     int* g;          // [chunk] gripper interval of each sample
+    int* r;          // [chunk] raw index of each staged sample (masked kernels only)
 };
 
 static size_t fit_times_doubles(int D, int nb, int p, int n_joint, int nbc) {
     return (size_t)nb * (p + 1) + 2 * (size_t)nb + (size_t)D * nb + (size_t)kFitTimesChunk * D +
            (size_t)n_joint * (nbc + 1);
 }
-static size_t fit_times_warp_bytes(int D, int nb, int p, int n_joint, int nbc) {
+static size_t fit_times_warp_bytes(int D, int nb, int p, int n_joint, int nbc, bool masked) {
     const size_t b = fit_times_doubles(D, nb, p, n_joint, nbc) * 8 + (size_t)kFitTimesChunk * (p + 2) * 4 +
-                     2 * (size_t)kFitTimesChunk * 4;
+                     (masked ? 3 : 2) * (size_t)kFitTimesChunk * 4;
     return (b + 15) & ~(size_t)15;
 }
 
@@ -88,6 +101,7 @@ __device__ __forceinline__ FitTimesWarp fit_times_warp(const FitTimesArgs& a, ch
     w.v = (float*)d;
     w.f = (int*)(w.v + kFitTimesChunk * (a.p + 2));
     w.g = w.f + kFitTimesChunk;
+    w.r = w.g + kFitTimesChunk;
     return w;
 }
 
@@ -101,13 +115,11 @@ __device__ __forceinline__ int knot_span(const float* kn, int lo, int hi, float 
     return lo;
 }
 
-// Lane `lane` < nt stages sample t0 + lane of row b: joint span values v[0..p] of columns f .. f+p (deboor_basis's
+// Stages one sample at time tv into slot `lane`: joint span values v[0..p] of columns f .. f+p (deboor_basis's
 // recursion restricted to the triangle of non-zero entries, same operations in the same order) and the gripper interval.
-__device__ __forceinline__ void fit_times_stage(const FitTimesArgs& a, const FitTimesWarp& w, const float* kj,
-                                                const float* kg, long long b, int t0, int nt, int lane) {
-    if (lane >= nt) return;
+__device__ __forceinline__ void fit_times_stage_one(const FitTimesArgs& a, const FitTimesWarp& w, const float* kj,
+                                                    const float* kg, float tv, int lane) {
     const int p = a.p;
-    const float tv = a.times[b * a.T + t0 + lane];
     const float u = clampf(__fdiv_rn(__fsub_rn(tv, 0.0f), a.tau), 0.0f, 1.0f);   // as decode_generic_kernel
     float* N = w.v + lane * (p + 2);                       // N[m] = basis j - p + m, N[p + 1] = 0 (basis j + 1)
     if (a.n_joint > 0) {
@@ -129,6 +141,42 @@ __device__ __forceinline__ void fit_times_stage(const FitTimesArgs& a, const Fit
         w.f[lane] = 0;
     }
     w.g[lane] = kg ? knot_span(kg, 0, a.nb - 1, u) : 0;
+}
+
+// Stages the n raw samples t0 .. t0+n-1 of row b and returns how many were staged (slots 0 .. nt-1, t ascending).
+// Unmasked: lane < n stages sample t0 + lane.  Masked: only the valid samples, each at slot = the number of valid samples
+// before it in the chunk, its raw index in w.r; *valid = the chunk's ballot (bit i: sample t0 + i is fitted).
+template <bool kMasked>
+__device__ __forceinline__ int fit_times_stage(const FitTimesArgs& a, const FitTimesWarp& w, const float* kj,
+                                               const float* kg, long long b, int t0, int n, int lane,
+                                               unsigned* valid = nullptr) {
+    if constexpr (!kMasked) {
+        if (lane < n) fit_times_stage_one(a, w, kj, kg, a.times[b * a.T + t0 + lane], lane);
+        return n;
+    } else {
+        const bool on = lane < n && a.mask[b * a.T + t0 + lane] != 0;
+        const unsigned bal = __ballot_sync(0xffffffffu, on);
+        if (on) {
+            const int slot = __popc(bal & ((1u << lane) - 1u));
+            fit_times_stage_one(a, w, kj, kg, a.times[b * a.times_stride + t0 + lane], slot);
+            w.r[slot] = t0 + lane;
+        }
+        if (valid) *valid = bal;
+        return __popc(bal);
+    }
+}
+
+// partial_only: true when every sample of row b is valid (the warp then leaves the row to the launch that wrote it)
+template <bool kMasked>
+__device__ __forceinline__ bool fit_times_skip_row(const FitTimesArgs& a, long long b, int lane) {
+    if constexpr (!kMasked) {
+        return false;
+    } else {
+        if (!a.partial_only) return false;
+        bool full = true;
+        for (int t = lane; t < a.T; t += 32) full &= a.mask[b * a.T + t] != 0;
+        return __all_sync(0xffffffffu, full);
+    }
 }
 
 // Owners of the Gram entries add the chunk's terms, t ascending.  Joint: entry (k, k-d) of the free columns; gripper:
@@ -229,6 +277,7 @@ __device__ __forceinline__ FitTimesWarp fit_times_setup(const FitTimesArgs& a, c
     return fit_times_warp(a, smem + head + (threadIdx.x >> 5) * a.warp_bytes);
 }
 
+template <bool kMasked>
 __global__ void __launch_bounds__(kFitTimesMaxWarps * 32, kFitTimesMinCtas)
 fit_times_kernel(const __grid_constant__ FitTimesArgs a) {
     extern __shared__ __align__(16) char smem_c[];
@@ -240,19 +289,22 @@ fit_times_kernel(const __grid_constant__ FitTimesArgs a) {
     const int T = a.T, D = a.D, nb = a.nb, p = a.p, pp = p + 2, nj = a.n_joint, nbc = a.ico + a.eco;
     const int n_g = nj > 0 ? nb * (p + 1) : 0;
     for (long long b = (long long)blockIdx.x * warps + (threadIdx.x >> 5); b < a.B; b += (long long)gridDim.x * warps) {
+        if (fit_times_skip_row<kMasked>(a, b, lane)) continue;
         for (int i = lane; i < n_g; i += 32) w.G[i] = 0.0;
         for (int i = lane; i < nb; i += 32) w.cnt[i] = 0.0;
         for (int i = lane; i < D * nb; i += 32) w.rhs[i] = 0.0;
         for (int t0 = 0; t0 < T; t0 += kFitTimesChunk) {
-            const int nt = T - t0 < kFitTimesChunk ? T - t0 : kFitTimesChunk;
+            const int n = T - t0 < kFitTimesChunk ? T - t0 : kFitTimesChunk;
             __syncwarp();                                  // previous chunk consumed, accumulators zeroed
-            fit_times_stage(a, w, kj, kg, b, t0, nt, lane);
+            const int nt = fit_times_stage<kMasked>(a, w, kj, kg, b, t0, n, lane);
             __syncwarp();
             // targets in slot order; joint slots minus bias and the pinned points' contribution
             const float* y = a.traj + (b * T + t0) * D;
             for (int i = lane; i < nt * D; i += 32) {
                 const int t = i / D, dof = i - t * D, s = dof_slot[dof];
-                double v = (double)__ldcs(y + i);
+                double v;
+                if constexpr (kMasked) v = (double)__ldcs(a.traj + (b * T + w.r[t]) * D + dof);
+                else v = (double)__ldcs(y + i);
                 if (s < nj && (nbc > 0 || a.bias)) {
                     if (a.bias) v -= (double)a.bias[b * nj + s];
                     const float* pin = a.bc + (b * nj + s) * nbc;
@@ -299,6 +351,7 @@ fit_times_kernel(const __grid_constant__ FitTimesArgs a) {
     }
 }
 
+template <bool kMasked>
 __global__ void __launch_bounds__(kFitTimesMaxWarps * 32, kFitTimesMinCtas)
 fit_times_backward_kernel(const __grid_constant__ FitTimesArgs a) {
     extern __shared__ __align__(16) char smem_c[];
@@ -311,14 +364,15 @@ fit_times_backward_kernel(const __grid_constant__ FitTimesArgs a) {
     const int n_g = nj > 0 ? nb * (p + 1) : 0;
     const int n_acc = a.grad_bc ? nj * (nbc + 1) : 0;
     for (long long b = (long long)blockIdx.x * warps + (threadIdx.x >> 5); b < a.B; b += (long long)gridDim.x * warps) {
+        if (fit_times_skip_row<kMasked>(a, b, lane)) continue;
         for (int i = lane; i < n_g; i += 32) w.G[i] = 0.0;
         for (int i = lane; i < nb; i += 32) w.cnt[i] = 0.0;
         for (int i = lane; i < n_acc; i += 32) w.acc[i] = 0.0;
         // pass 1: the row's Gram matrices, exactly as the forward builds them
         for (int t0 = 0; t0 < T; t0 += kFitTimesChunk) {
-            const int nt = T - t0 < kFitTimesChunk ? T - t0 : kFitTimesChunk;
+            const int n = T - t0 < kFitTimesChunk ? T - t0 : kFitTimesChunk;
             __syncwarp();
-            fit_times_stage(a, w, kj, kg, b, t0, nt, lane);
+            const int nt = fit_times_stage<kMasked>(a, w, kj, kg, b, t0, n, lane);
             __syncwarp();
             int fmin, fmax, gmin, gmax;
             warp_range(nt, lane, w, fmin, fmax, gmin, gmax);
@@ -336,11 +390,16 @@ fit_times_backward_kernel(const __grid_constant__ FitTimesArgs a) {
         fit_times_solve(a, w, lane);
         // pass 2: u = Phi v per sample (output order), then the pinned points' and the bias's sums, t ascending
         for (int t0 = 0; t0 < T; t0 += kFitTimesChunk) {
-            const int nt = T - t0 < kFitTimesChunk ? T - t0 : kFitTimesChunk;
+            const int n = T - t0 < kFitTimesChunk ? T - t0 : kFitTimesChunk;
             __syncwarp();
-            fit_times_stage(a, w, kj, kg, b, t0, nt, lane);
+            unsigned valid = 0;
+            const int nt = fit_times_stage<kMasked>(a, w, kj, kg, b, t0, n, lane, &valid);
             __syncwarp();
             float* gy = a.grad_traj + (b * T + t0) * D;
+            if constexpr (kMasked) {                       // masked samples: exactly 0
+                for (int i = lane; i < n * D; i += 32)
+                    if (!((valid >> (i / D)) & 1u)) __stcs(gy + i, 0.0f);
+            }
             for (int i = lane; i < nt * D; i += 32) {
                 const int t = i / D, dof = i - t * D, s = dof_slot[dof];
                 const double* v = w.rhs + (size_t)s * nb;
@@ -354,7 +413,8 @@ fit_times_backward_kernel(const __grid_constant__ FitTimesArgs a) {
                 } else {
                     u = v[w.g[t]];
                 }
-                __stcs(gy + i, __double2float_rn(u));
+                if constexpr (kMasked) __stcs(a.grad_traj + (b * T + w.r[t]) * D + dof, __double2float_rn(u));
+                else __stcs(gy + i, __double2float_rn(u));
                 w.yc[t * D + s] = u;
             }
             __syncwarp();
@@ -389,7 +449,7 @@ static int launch_fit_times(const Plan* p, FitTimesArgs& a, K kernel, cudaStream
     const int nbc = p->ico + p->eco;
     const size_t head = (((size_t)(p->nc + p->degree_p + 1 + (p->n_joint < p->D ? p->nb + 1 : 0) + p->D) * 4) + 15) &
                         ~(size_t)15;
-    a.warp_bytes = fit_times_warp_bytes(p->D, p->nb, p->degree_p, p->n_joint, nbc);
+    a.warp_bytes = fit_times_warp_bytes(p->D, p->nb, p->degree_p, p->n_joint, nbc, a.mask != nullptr);
     long long warps = ((long long)p->max_smem_optin - (long long)head) / (long long)a.warp_bytes;
     if (warps < 1) return BEAST_E_UNSUPPORTED;
     if (warps > kFitTimesMaxWarps) warps = kFitTimesMaxWarps;
@@ -414,6 +474,7 @@ static void fit_times_common(const Plan* p, FitTimesArgs& a, long long B, int T,
     a.knots_g = p->n_joint < p->D ? p->knots_grip_d : nullptr;
     a.slot_to_dof = p->slot_to_dof_d;
     a.times = times;
+    a.times_stride = T;
 }
 
 static bool misaligned4(std::initializer_list<const void*> ps) {
@@ -444,7 +505,7 @@ extern "C" int beast_fit_times_f32(const beast_plan_t* plan, const float* traj, 
     a.bias = pinned ? bias : nullptr;
     a.params_out = params_out;
     static size_t granted[kMaxDevices] = {};
-    return launch_fit_times(p, a, fit_times_kernel, (cudaStream_t)stream, granted);
+    return launch_fit_times(p, a, fit_times_kernel<false>, (cudaStream_t)stream, granted);
 }
 
 extern "C" int beast_fit_times_backward_f32(const beast_plan_t* plan, int64_t B, int32_t T, const float* times,
@@ -471,5 +532,63 @@ extern "C" int beast_fit_times_backward_f32(const beast_plan_t* plan, int64_t B,
     a.grad_bc = pinned ? grad_bc : nullptr;
     a.grad_bias = pinned ? grad_bias : nullptr;
     static size_t granted[kMaxDevices] = {};
-    return launch_fit_times(p, a, fit_times_backward_kernel, (cudaStream_t)stream, granted);
+    return launch_fit_times(p, a, fit_times_backward_kernel<false>, (cudaStream_t)stream, granted);
+}
+
+extern "C" int beast_fit_masked_f32(const beast_plan_t* plan, const float* traj, int64_t B, int32_t T,
+                                    const float* times, int64_t times_row_stride, const uint8_t* mask,
+                                    int32_t partial_only, const float* bc, const float* bias, float* params_out,
+                                    void* stream) {
+    const Plan* p = (const Plan*)plan;
+    if (!p) return BEAST_E_NULL;
+    const bool pinned = p->ico + p->eco > 0 && p->n_joint > 0;
+    if (B < 0 || T < 1 || (pinned && T < 2)) return BEAST_E_SHAPE;
+    if (times_row_stride != 0 && times_row_stride != T) return BEAST_E_SHAPE;
+    if (p->nc + p->degree_p + 1 > kMaxEvalKnots) return BEAST_E_UNSUPPORTED;
+    if (B > 0 && (!traj || !times || !mask || !params_out || (pinned && !bc))) return BEAST_E_NULL;
+    if (misaligned4({traj, times, bc, bias, params_out})) return BEAST_E_ALIGN;
+    if (B == 0) return BEAST_OK;
+    FitTimesArgs a = {};
+    fit_times_common(p, a, B, T, times);
+    a.times_stride = times_row_stride;
+    a.mask = mask;
+    a.partial_only = partial_only ? 1 : 0;
+    a.traj = traj;
+    a.bc = pinned ? bc : nullptr;
+    a.bias = pinned ? bias : nullptr;
+    a.params_out = params_out;
+    static size_t granted[kMaxDevices] = {};
+    return launch_fit_times(p, a, fit_times_kernel<true>, (cudaStream_t)stream, granted);
+}
+
+extern "C" int beast_fit_masked_backward_f32(const beast_plan_t* plan, int64_t B, int32_t T, const float* times,
+                                             int64_t times_row_stride, const uint8_t* mask, int32_t partial_only,
+                                             const float* grad_norm, const float* grad_params, const float* params,
+                                             const float* w_min, const float* w_max, float* grad_traj, float* grad_bc,
+                                             float* grad_bias, void* stream) {
+    const Plan* p = (const Plan*)plan;
+    if (!p) return BEAST_E_NULL;
+    const bool pinned = p->ico + p->eco > 0 && p->n_joint > 0;
+    if (B < 0 || T < 1 || (pinned && T < 2)) return BEAST_E_SHAPE;
+    if (times_row_stride != 0 && times_row_stride != T) return BEAST_E_SHAPE;
+    if (p->nc + p->degree_p + 1 > kMaxEvalKnots) return BEAST_E_UNSUPPORTED;
+    if (!grad_norm && !grad_params) return BEAST_E_NULL;
+    if (grad_norm && (!params || !w_min || !w_max)) return BEAST_E_NULL;
+    if (B > 0 && (!times || !mask || !grad_traj || (pinned && !grad_bc))) return BEAST_E_NULL;
+    if (misaligned4({times, grad_norm, grad_params, params, w_min, w_max, grad_traj, grad_bc, grad_bias}))
+        return BEAST_E_ALIGN;
+    if (B == 0) return BEAST_OK;
+    FitTimesArgs a = {};
+    fit_times_common(p, a, B, T, times);
+    a.times_stride = times_row_stride;
+    a.mask = mask;
+    a.partial_only = partial_only ? 1 : 0;
+    a.grad_norm = grad_norm; a.grad_params = grad_params;
+    a.params = grad_norm ? params : nullptr;
+    a.w_min = grad_norm ? w_min : nullptr; a.w_max = grad_norm ? w_max : nullptr;
+    a.grad_traj = grad_traj;
+    a.grad_bc = pinned ? grad_bc : nullptr;
+    a.grad_bias = pinned ? grad_bias : nullptr;
+    static size_t granted[kMaxDevices] = {};
+    return launch_fit_times(p, a, fit_times_backward_kernel<true>, (cudaStream_t)stream, granted);
 }

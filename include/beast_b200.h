@@ -269,6 +269,28 @@ int beast_fit_times_backward_f32(const beast_plan_t* plan, int64_t B, int32_t T,
                                  const float* w_min, const float* w_max, float* grad_traj, float* grad_bc,
                                  float* grad_bias, void* stream);
 
+/* ---- Masked fit (encode / encode_continuous / compute_weights / update_weights_bounds with mask [B, T]).
+ * mask [B, T] bytes, non-zero = the sample is fitted (LeRobot's action_is_pad is its negation).  Row b is fitted as
+ * beast_fit_times_f32 fits the compacted row y[b, mask[b]] on times[b, mask[b]], bit for bit: same fp64 Gram matrix,
+ * right-hand sides, band Cholesky, single fp32 rounding and t-ascending order.  A masked sample's time and trajectory
+ * value are never read and add no term anywhere.  times_row_stride is T (times [B, T]) or 0 (one grid [T] for every
+ * row); any other value is BEAST_E_SHAPE.  bc / bias are the row's boundary state computed from its valid samples.
+ * A row without valid samples gets exactly 0 (without pinned points); with pinned points a row with fewer than two
+ * valid samples is not treated specially.  partial_only != 0: a row whose mask is all non-zero is skipped and its
+ * outputs are left untouched (the shared-grid path lets K1 write those rows first).  NULL mask is BEAST_E_NULL;
+ * the other NULL, shape, alignment and support rules are beast_fit_times_f32's.  An ordinary launch. */
+int beast_fit_masked_f32(const beast_plan_t* plan, const float* traj, int64_t B, int32_t T, const float* times,
+                         int64_t times_row_stride, const uint8_t* mask, int32_t partial_only, const float* bc,
+                         const float* bias, float* params_out, void* stream);
+/* Its adjoint, as beast_fit_times_backward_f32 on the compacted row: masked samples get grad_traj exactly 0 and add
+ * nothing to grad_bc / grad_bias.  With partial_only, rows whose mask is all non-zero are left untouched in every
+ * output (grad_traj, grad_bc, grad_bias). */
+int beast_fit_masked_backward_f32(const beast_plan_t* plan, int64_t B, int32_t T, const float* times,
+                                  int64_t times_row_stride, const uint8_t* mask, int32_t partial_only,
+                                  const float* grad_norm, const float* grad_params, const float* params,
+                                  const float* w_min, const float* w_max, float* grad_traj, float* grad_bc,
+                                  float* grad_bias, void* stream);
+
 /* ---- K2: bounds.
  * Column min/max of x [rows, cols] (update_weights_bounds :377-378; the reduction inside
  * update_weights_bounds_per_batch :382-383).  accumulate != 0 folds into the existing
